@@ -2,7 +2,9 @@
 """bench.py — MCMC iterations/s of the SpamTrees hot path on N B200s (BASELINE.json metric), one process per GPU.
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
-  python bench.py --impl reference --gpus N ...            # the reference algorithm on the host cores (CPU oracle)
+  python bench.py --impl reference --gpus N ...            # the reference algorithm on the host cores (CPU oracle): --steps full
+                                                           # CPU iterations, about 1.3 s each at C4 on 16 cores
+  python bench.py --steps K --dump-outputs DIR             # + the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one MCMC iteration of the hot path (spamtree_fit.cpp:167-330 minus predict/save): GIBBS sweep over w + LLW +
 BUILD at a proposed theta + accept/swap + tausq + beta.  The workload is BASELINE config C4 (q=3, n=1M) at every N: at
@@ -96,6 +98,23 @@ def proposals(theta, k, seed):
     """a fixed sequence of small random-walk proposals around the parity-point theta (same for every arm)"""
     rng = np.random.default_rng(seed)
     return [theta * (1 + 0.002 * rng.standard_normal(theta.size)) for _ in range(k)]
+
+
+DUMP_ROWS = 1 << 21  # rows of w and XB written by --dump-outputs: 2 x 16 MB of float64 at most
+
+
+def dump_outputs(path, gm, last):
+    """what the last timed step computed, as a caller of bench_iteration receives it: its return values (log-density of the
+    proposal, of the previous current state, 1 if the proposal's BUILD was acceptable) and the state it leaves (w, beta,
+    1 / tausq, X beta).  Above DUMP_ROWS rows, w and XB are kept at a fixed, seeded sample of rows, written as rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    pr = gm.params()
+    out = {"loglik": last, "w": gm.w, "beta": pr["Bcoeff"], "tausq_inv": pr["tausq_inv"], "xb": pr["XB"]}
+    if gm.n_all > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(gm.n_all, DUMP_ROWS, replace=False))
+        out.update(w=out["w"][rows], xb=out["xb"][rows], rows=rows)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def measure_fp64_peak(torch, dev):
@@ -194,16 +213,16 @@ def run_reference(args, rank, world, emit):
             backend = b
         else:
             orc.use_blas(False)
-    t_warm = max(om.timed_iteration(props[i], do_swap=(i % 4 == 3)) for i in range(warm))
-    # exactly --steps iterations unless that would take more than ~2.5 minutes of CPU time (or --ref-steps says otherwise)
-    steps = max(1, min(args.steps, args.ref_steps if args.ref_steps > 0 else max(2, int(150.0 / max(t_warm, 1e-6)))))
+    for i in range(warm):
+        om.timed_iteration(props[i], do_swap=(i % 4 == 3))
+    steps = min(args.steps, args.ref_steps) if args.ref_steps > 0 else args.steps
     ts = [om.timed_iteration(props[warm + i], do_swap=(i % 4 == 3)) for i in range(steps)]
     v = steps / float(np.sum(ts))
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": 1e3 / v, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": config_of(args.workload, d, t, args.gpus),
             "note": "CPU arm: the reference algorithm (oracle port, OpenMP over the blocks of a level) on the host cores; --steps iterations, "
-                    "fewer only if they would not fit ~2.5 minutes",
+                    "fewer only where --ref-steps caps them",
             "cpu_baseline": {"value": v, "unit": UNIT, "cores": int(cores), "kind": "port", "backend": backend,
                              "sample": f"{steps} timed iteration(s) after {warm} warm-up on the full {args.workload} tree, lean-state oracle"},
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
@@ -213,11 +232,13 @@ def run_reference(args, rank, world, emit):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed iterations, in both arms; with --impl reference each is a full CPU iteration (about 1.3 s at C4 on 16 "
+                         "host cores), so the run takes about that many times longer (--ref-steps caps them)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C4", choices=["C1", "C2", "C3", "C4", "C5"])
-    ap.add_argument("--ref-steps", type=int, default=0, help="cap on the timed iterations of --impl reference (0: as many of --steps as fit ~2.5 min)")
+    ap.add_argument("--ref-steps", type=int, default=0, help="cap on the timed iterations of --impl reference (0: --steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-loops", action="store_true", help="CPU arm with the port's own loops instead of the host's OpenBLAS")
     ap.add_argument("--no-predict-leg", action="store_true", help="skip the extra end-to-end leg with prediction on a thin schedule")
@@ -225,7 +246,11 @@ def main():
     ap.add_argument("--e2e-sd", type=float, default=1e-8,
                     help="diagonal of mcmcsd in the end-to-end leg (the proposal covariance in logit space, spamtree_fit.cpp:95): small "
                          "enough that a share of the proposals is accepted at n = 1M, as in a tuned chain; the accepted count is reported")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64), to compare builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE JSON line: anything a library prints there (NCCL's version banner ...) goes to stderr
     real_stdout = os.dup(1)
     os.dup2(2, 1)
@@ -236,6 +261,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        ap.error("--dump-outputs writes the outputs of the CUDA path on one GPU")
     if args.impl == "reference":
         run_reference(args, rank, world, emit)
         return
@@ -284,13 +311,15 @@ def main():
     barrier()
     t0 = time.perf_counter()
     for i in range(args.steps):
-        _, ms = gm.bench_iteration(props[args.warmup + i], do_swap=(i % 4 == 3), seed=1000 + i)
+        last, ms = gm.bench_iteration(props[args.warmup + i], do_swap=(i % 4 == 3), seed=1000 + i)
         phase += ms
     gm.sync()
     barrier()
     elapsed = time.perf_counter() - t0
     c1 = gm.counters()
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, gm, last)
     # device time of the step: CUDA events around the whole iteration on the launching stream (the per-phase times do not
     # add up to it: the upper levels of BUILD run on a second stream underneath the Gibbs sweep)
     dev_ms = float(phase[4])

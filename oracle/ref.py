@@ -1,8 +1,9 @@
 """ctypes wrapper of oracle/_ref/libspamtree_ref.so — the reference's OWN model layer (spamtree_model.cpp,
-covariance_functions.cpp, tree_utils.cpp, tree_dep.cpp, mh_adapt.cpp), compiled unmodified from /root/reference/src
-against the Armadillo/Rcpp stand-in in oracle/refshim/.  TEST INFRASTRUCTURE ONLY: it pins the CPU oracle.
-The library is built by `make -C oracle ref` where /root/reference exists and travels prebuilt elsewhere."""
+covariance_functions.cpp, tree_utils.cpp, tree_dep.cpp, mh_adapt.cpp), compiled unmodified from the reference package's
+src/ directory against the Armadillo/Rcpp stand-in in oracle/refshim/.  TEST INFRASTRUCTURE ONLY: it pins the CPU oracle.
+The library is built by `make -C oracle ref` wherever that directory exists (ref_src())."""
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -14,10 +15,23 @@ _dp, _ip = C.POINTER(C.c_double), C.POINTER(C.c_int64)
 _lib = None
 
 
+def ref_src():
+    """the reference package's src/ directory: SPAMTREE_REF_SRC if set, else src/ under BASELINE.json's reference_path"""
+    src = os.environ.get("SPAMTREE_REF_SRC")
+    if not src:
+        with open(os.path.join(os.path.dirname(_HERE), "BASELINE.json")) as f:
+            src = os.path.join(json.load(f)["reference_path"], "src")
+    return src
+
+
+def build(stdout=subprocess.DEVNULL, stderr=None):
+    subprocess.check_call(["make", "-C", _HERE, "ref", "REFSRC=" + ref_src()], stdout=stdout, stderr=stderr)
+
+
 def available():
-    if not os.path.exists(LIB_PATH) and os.path.isdir("/root/reference/src"):
+    if not os.path.exists(LIB_PATH) and os.path.isdir(ref_src()):
         try:
-            subprocess.check_call(["make", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            build(stderr=subprocess.DEVNULL)
         except Exception:
             return False
     return os.path.exists(LIB_PATH)

@@ -1,10 +1,11 @@
 """Generates tests/golden/ref_*.npz by running THE REFERENCE'S OWN CODE: oracle/_ref/libspamtree_ref.so is the reference's
 model layer (spamtree_model.cpp, covariance_functions.cpp, tree_utils.cpp, tree_dep.cpp, mh_adapt.cpp) compiled
-unmodified from /root/reference/src against the Armadillo/Rcpp stand-in of oracle/refshim/ (`make -C oracle ref`).
-The reference exists only in the build container, so its outputs are committed here as fixtures; the CPU oracle and the
-CUDA path are both checked against them (tests/test_golden_reference.py).  The ref_chain_*.npz files are whole chains of the reference's own MCMC driver
+unmodified from the reference package's src/ directory against the Armadillo/Rcpp stand-in of oracle/refshim/
+(`make -C oracle ref`).  The reference's sources are not part of this repository, so its outputs are committed here as
+fixtures; the CPU oracle and the CUDA path are both checked against them (tests/test_golden_reference.py).  The ref_chain_*.npz files are whole chains of the reference's own MCMC driver
 (spamtree_fit.cpp, compiled unmodified as well).
-Run (where /root/reference exists):  python tests/golden/make_golden_from_reference.py"""
+Run (the reference's src/ is SPAMTREE_REF_SRC, else src/ under BASELINE.json's reference_path):
+    python tests/golden/make_golden_from_reference.py"""
 import os
 import sys
 
@@ -99,7 +100,7 @@ def chain(q, n, limited, sd, keep, burn, thin, adapting, predicts, seed=31):
 
 if __name__ == "__main__":
     if not ref.available():
-        raise SystemExit("oracle/_ref/libspamtree_ref.so is missing and /root/reference is not here to build it")
+        raise SystemExit("oracle/_ref/libspamtree_ref.so is missing and the reference sources are not at " + ref.ref_src())
     which = sys.argv[1] if len(sys.argv) > 1 else "all"
     if which in ("all", "model"):
         for q, n, limited in CASES:

@@ -44,6 +44,70 @@ def test_reference_arm_runs_on_rank_0_only():
 import pytest  # noqa: E402
 
 
+def test_dump_outputs_writes_float64_and_samples_large_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: every array as float64; above DUMP_ROWS rows, w and XB at a fixed sample of rows (the same every run)"""
+    sys.path.insert(0, ROOT)
+    import bench
+
+    class Model:
+        n_all = 50
+        w = np.arange(50.0)
+
+        def params(self):
+            return {"Bcoeff": np.ones((3, 2)), "tausq_inv": np.ones(2, dtype=np.float32), "XB": -np.arange(50.0)}
+
+    monkeypatch.setattr(bench, "DUMP_ROWS", 20)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), Model(), np.array([-1.5, -2.5, 1.0]))
+    got = {f.stem: np.load(f) for f in sorted((tmp_path / "a").glob("*.npy"))}
+    assert set(got) == {"loglik", "w", "beta", "tausq_inv", "xb", "rows"} and all(a.dtype == np.float64 for a in got.values())
+    rows = got["rows"].astype(int)
+    assert rows.size == 20 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(got["w"], rows) and np.array_equal(got["xb"], -rows)
+    assert all(np.array_equal(np.load(tmp_path / "b" / f"{k}.npy"), v) for k, v in got.items())
+
+
+def test_dump_outputs_is_refused_for_the_reference_arm(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, cwd=ROOT, timeout=600)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and not any(tmp_path.iterdir())
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_the_last_steps_outputs(tmp_path):
+    """--dump-outputs holds what the LAST timed step returned and left: bench.py's step sequence on C1 (same problem, same
+    proposals and seeds) replayed in this process must give every file exactly; --steps sets the timed steps"""
+    warmup, steps = 3, 5
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "C1", "--steps", str(steps), "--warmup", str(warmup),
+                        "--no-cpu-baseline", "--no-predict-leg", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, cwd=ROOT, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout)["steps"] == steps
+    got = {f.stem: np.load(f) for f in sorted(tmp_path.glob("*.npy"))}
+    assert set(got) == {"loglik", "w", "beta", "tausq_inv", "xb"} and all(v.dtype == np.float64 for v in got.values())
+    sys.path.insert(0, ROOT)
+    import bench
+    import spamtree_b200 as sb
+    d, t, csr, theta = bench.build_problem("C1", 2021)
+    gm = sb.SpamTreeMV(d["y"], d["X"], d["coords"], d["mv_id"], t["res_is_ref"], None, None, False, t["block_names"], t["block_groups"],
+                       None, np.zeros(3), theta, 0.1, csr=csr, keep_H=False, device=0)
+    gm.set_beta_index(False)
+    gm.get_loglik_comps_w(0)
+    gm.get_loglik_comps_w(1)
+    props = bench.proposals(theta, warmup + steps, 99)
+    for i in range(warmup):
+        gm.bench_iteration(props[i], do_swap=(i % 4 == 3), seed=i)
+    gm.get_loglik_w(0)  # bench.py's parity probe
+    outs = [gm.bench_iteration(props[warmup + i], do_swap=(i % 4 == 3), seed=1000 + i)[0] for i in range(steps)]
+    pr = gm.params()
+    want = {"loglik": outs[-1], "w": gm.w, "beta": pr["Bcoeff"], "tausq_inv": pr["tausq_inv"], "xb": pr["XB"]}
+    gm.close()
+    assert not np.array_equal(outs[-2], outs[-1])  # the last step is told apart from the one before it
+    assert want["w"].shape == (625,) and np.any(want["w"] != 0) and not np.array_equal(want["w"], want["xb"])
+    for k, v in want.items():
+        assert np.array_equal(got[k], v), k
+
+
 @pytest.mark.gpu
 def test_product_arm_prints_one_json_line_with_the_contract_keys():
     """the CUDA arm on the smallest config (C1): ONE JSON line on stdout with every key the measurement contract names"""

@@ -155,7 +155,7 @@ def test_device_chain_is_reproducible_and_seed_dependent():
     assert not np.array_equal(runs[0]["w_mcmc"], runs[2]["w_mcmc"])
 
 
-def test_device_chain_without_graph_matches_graph(monkeypatch):
+def test_device_chain_without_graph_matches_graph(monkeypatch, tmp_path):
     """ST_GRAPH=0 enqueues every iteration kernel by kernel; the CUDA-graph replay must give bit-identical chains"""
     import os, subprocess, sys
     code = ("import sys; sys.path.insert(0, 'tests'); import numpy as np, common; from spamtree_b200 import synth;"
@@ -164,7 +164,7 @@ def test_device_chain_without_graph_matches_graph(monkeypatch):
             "np.save(sys.argv[1], np.concatenate([r['theta_mcmc'].ravel(), r['w_mcmc'].ravel(), r['beta_mcmc'].ravel()]))")
     outs = []
     for g in ("1", "0"):
-        path = f"/tmp/_st_graph_{g}.npy"
+        path = str(tmp_path / f"graph_{g}.npy")
         env = dict(os.environ, ST_GRAPH=g)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env, cwd=common.ROOT)
         outs.append(np.load(path))

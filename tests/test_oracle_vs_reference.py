@@ -1,7 +1,9 @@
 """Pins the CPU oracle against the REFERENCE ITSELF: oracle/_ref/libspamtree_ref.so is the reference's own model layer
-(spamtree_model.cpp, covariance_functions.cpp, tree_utils.cpp, tree_dep.cpp, mh_adapt.cpp) compiled UNMODIFIED from
-/root/reference/src against the Armadillo/Rcpp stand-in of oracle/refshim/ (recipe: `make -C oracle ref`).  The library
-is built where /root/reference exists and travels prebuilt elsewhere; without it these tests are skipped."""
+(spamtree_model.cpp, covariance_functions.cpp, tree_utils.cpp, tree_dep.cpp, mh_adapt.cpp) compiled UNMODIFIED from the
+reference package's src/ directory against the Armadillo/Rcpp stand-in of oracle/refshim/ (recipe: `make -C oracle ref`).
+The library is built wherever that directory exists (SPAMTREE_REF_SRC, else src/ under BASELINE.json's reference_path);
+without it these tests are skipped (the reference's outputs on fixed problems are stored in tests/golden/ref_*.npz and
+checked by tests/test_golden_reference.py)."""
 import numpy as np
 import pytest
 
@@ -9,7 +11,7 @@ import common
 from common import orc, relerr
 from oracle import ref
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libspamtree_ref.so not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libspamtree_ref.so not built (the reference sources are not at ref.ref_src())")
 
 
 def _pair(q, n, missing=.1, limited=False, cell_size=25, proportions=None):

@@ -11,7 +11,7 @@ from oracle import ref
 import spamtree_b200 as sb
 from spamtree_b200 import synth
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libspamtree_ref.so not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libspamtree_ref.so not built (the reference sources are not at ref.ref_src())")
 
 
 def _same_lists(a, b):
