@@ -167,6 +167,53 @@ typedef struct {                 /* caller-allocated; NULL pointers are skipped 
 } st_mcmc_out;
 int st_mcmc_run(st_handle* h, const st_mcmc_opts* opts, st_mcmc_out* out);
 
+/* ---- prediction at new locations from saved samples (no reference counterpart; the math is predict_std,
+ * spamtree_model.cpp:1234-1358, and the yhat of spamtree_fit.cpp:384, per saved sample s):
+ *   w_new,i = K_{i,pa} K_pa^-1 w_pa,s + sqrt(K_ii - K_{i,pa} K_pa^-1 K_{pa,i}) z_i     (covariance at theta_s; sd 0 when
+ *                                                                                      the Schur complement is not positive)
+ *   y_new,i = x_i' beta_s[:, mv_i] + w_new,i + sqrt(tausq_s[mv_i]) eps_i
+ * pa = the parent list of the row's group (st_tree_attach).  The handle's fitted state is not changed: the current slot,
+ * w, beta, tausq and the chain state stay as they are; the alter slot is used as scratch for the BUILD of each distinct
+ * theta_s: until st_get_loglik_comps_w(h, 1, ...) or st_mcmc_run rebuilds it, st_accept_make_change and
+ * st_get_loglik_w(h, 1, ...) return ST_ERR_INVALID.  Samples that repeat the previous theta bit for bit skip that BUILD.
+ * ST_ERR_NOT_SPD: the covariance at some sample's theta is not positive definite on a reference block (a chain never saves
+ * such a theta); the outputs are then not draws of the model.  Single-GPU handles only (ST_ERR_UNSUPPORTED otherwise). */
+typedef struct {
+  int64_t n_new;
+  const double* coords;        /* n_new x 2 */
+  const int64_t* mv_id;        /* n_new, 1-based */
+  const double* X;             /* n_new x p, or NULL: no covariates (x' beta = 0) */
+  int64_t n_groups;
+  const int64_t* group;        /* n_new: 0-based group of each row */
+  const int64_t* parents_ptr;  /* n_groups + 1 */
+  const int64_t* parents_idx;  /* 0-based block ids of each group's parents, root first (a chain of reference blocks, as
+                                  st_tree_attach returns; limited trees: the direct parent only) */
+} st_new_rows;
+typedef struct {
+  int32_t n_samples;           /* S */
+  const double* theta;         /* npar x S */
+  const double* beta;          /* p x S x q (beta_mcmc's layout) */
+  const double* tausq;         /* q x S */
+  const double* w;             /* n_all rows per sample, boundary order: w(i, s) = w[i * w_row_stride + s * w_sample_stride];
+                                  one of the two strides must be 1 (st_mcmc_out.w_mcmc: 1, n_all; its C-order transpose: S, 1) */
+  int64_t w_row_stride, w_sample_stride;
+  const double* z;             /* n_new x S normals of the w draws, or NULL: drawn on the device */
+  const double* eps;           /* n_new x S normals of the y draws, or NULL */
+  uint64_t seed;               /* device draws: Philox keyed by (seed, new row, position of the sample in this call) */
+} st_pred_samples;
+typedef struct {               /* caller-allocated, NULL pointers are skipped; rows in the caller's order */
+  double* w_new;               /* n_new x S */
+  double* y_new;               /* n_new x S */
+  double* mean;                /* n_new x S: K_{i,pa} K_pa^-1 w_pa,s */
+  double* sd;                  /* n_new x S: the conditional sd */
+  double* w_mean;              /* n_new: mean over the S draws */
+  double* w_sd;                /* n_new: sd over the S draws (ddof = 1; 0 for one sample) */
+  double* y_mean;              /* n_new */
+  double* y_sd;                /* n_new */
+  int64_t n_builds;            /* BUILDs of the reference levels run (one per change of theta along the samples) */
+} st_pred_out;
+int st_predict_new(st_handle* h, const st_new_rows* rows, const st_pred_samples* samples, st_pred_out* out);
+
 /* ---- the Metropolis-Hastings glue (mh_adapt.h / mh_adapt.cpp), as st_mcmc_run uses it; host-only, no handle ---- */
 /* par_huvtransf_fwd / par_huvtransf_back (Rcpp exports), mh_adapt.cpp:3-15: logit / logistic on (bounds[j], bounds[j + npar]).
  * bounds: npar x 2. */
@@ -250,6 +297,15 @@ int st_tree_sizes(const st_tree* t, int64_t* out6);
 int st_tree_get(const st_tree* t, int64_t* blocking, int64_t* res, int64_t* res_is_ref, double* parchimat,
                 int64_t* indexing_ptr, int64_t* indexing_idx, int64_t* parents_ptr, int64_t* parents_idx,
                 int64_t* children_ptr, int64_t* children_idx, double* block_names, double* block_groups);
+/* New rows attached to a built tree (no reference counterpart; the rule is that of the prediction level, R/make_tree.R:317-413):
+ * the nearest row of the last loop level (same margin first when the tree was built with cherrypick_same_margin) names the
+ * parent block b; the new rows of one b form one group, groups numbered by ascending b; a group's parents are the reference
+ * blocks on the chains through b, root first (make_edges' rule for a column appended to parchimat; limited != 0: the last of
+ * them, make_edges_limited).  The tree itself is not changed.  coords_new n_new x 2, mv_new 1-based.
+ * group: n_new (0-based group of each row); par_ptr: n_groups + 1; par_idx: 0-based block ids.
+ * Two-call protocol: with par_idx == NULL only counts[0..1] = {n_groups, #parent entries} are written. */
+int st_tree_attach(const st_tree* t, int64_t n_new, const double* coords_new, const int64_t* mv_new, int32_t limited,
+                   int64_t* group, int64_t* par_ptr, int64_t* par_idx, int64_t* counts);
 
 /* CrossCovarianceAG10 (R export), covariance_functions.cpp:301-355, evaluated on the GPU.
  * coords n x 2 col-major, mv 1-based, Dmat q x q; out n1 x n2. */

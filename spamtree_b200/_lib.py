@@ -75,6 +75,29 @@ class StTreeOpts(C.Structure):
     ]
 
 
+class StNewRows(C.Structure):
+    _fields_ = [
+        ("n_new", C.c_int64), ("coords", c_double_p), ("mv_id", c_int64_p), ("X", c_double_p),
+        ("n_groups", C.c_int64), ("group", c_int64_p), ("parents_ptr", c_int64_p), ("parents_idx", c_int64_p),
+    ]
+
+
+class StPredSamples(C.Structure):
+    _fields_ = [
+        ("n_samples", C.c_int32), ("theta", c_double_p), ("beta", c_double_p), ("tausq", c_double_p), ("w", c_double_p),
+        ("w_row_stride", C.c_int64), ("w_sample_stride", C.c_int64), ("z", c_double_p), ("eps", c_double_p),
+        ("seed", C.c_uint64),
+    ]
+
+
+class StPredOut(C.Structure):
+    _fields_ = [
+        ("w_new", c_double_p), ("y_new", c_double_p), ("mean", c_double_p), ("sd", c_double_p),
+        ("w_mean", c_double_p), ("w_sd", c_double_p), ("y_mean", c_double_p), ("y_sd", c_double_p),
+        ("n_builds", C.c_int64),
+    ]
+
+
 # every symbol include/spamtree_b200.h declares, with its signature
 SIGNATURES = {
     "st_version": (C.c_char_p, []),
@@ -97,6 +120,7 @@ SIGNATURES = {
     "st_get_node_state": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, c_double_p, C.c_int64, c_int64_p]),
     "st_get_index": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.c_int, c_int64_p, C.c_int64, c_int64_p]),
     "st_mcmc_run": (C.c_int, [C.c_void_p, C.POINTER(StMcmcOpts), C.POINTER(StMcmcOut)]),
+    "st_predict_new": (C.c_int, [C.c_void_p, C.POINTER(StNewRows), C.POINTER(StPredSamples), C.POINTER(StPredOut)]),
     "st_bench_iteration": (C.c_int, [C.c_void_p, c_double_p, C.c_int, C.c_uint64, c_double_p, c_float_p]),
     "st_set_beta_index": (C.c_int, [C.c_void_p, C.c_int]),
     "st_get_counters": (C.c_int, [C.c_void_p, c_double_p]),
@@ -118,6 +142,8 @@ SIGNATURES = {
     "st_tree_sizes": (C.c_int, [C.c_void_p, c_int64_p]),
     "st_tree_get": (C.c_int, [C.c_void_p, c_int64_p, c_int64_p, c_int64_p, c_double_p, c_int64_p, c_int64_p,
                               c_int64_p, c_int64_p, c_int64_p, c_int64_p, c_double_p, c_double_p]),
+    "st_tree_attach": (C.c_int, [C.c_void_p, C.c_int64, c_double_p, c_int64_p, C.c_int32, c_int64_p, c_int64_p,
+                                 c_int64_p, c_int64_p]),
     "st_cross_covariance_ag10": (C.c_int, [c_double_p, c_int64_p, C.c_int64, c_double_p, c_int64_p, C.c_int64,
                                            c_double_p, c_double_p, c_double_p, c_double_p, C.c_int32, c_double_p,
                                            C.c_int32, C.c_int32, c_double_p]),

@@ -85,7 +85,10 @@ __device__ __noinline__ bool pair_chol_inv32(double* R, int m, int rs, double* c
 }
 }  // namespace
 
-// MODE 0: reference level, 1: non-reference level, 2: prediction blocks (outG = Hpred receives H, outRi = sd).
+// MODE 0: reference level, 1: non-reference level, 2: prediction blocks (outG = Hpred receives H, outRi = sd),
+// 3: forward-only prediction (new rows of Model::predict_new): the panel carries w_pa in one extra column, and the forward
+// sweep alone gives mean = Z'v = K_{u,pa} K_pa^-1 w_pa (into predG) and sd = sqrt(K_uu - diag(Z'Z)) (into predRi), both
+// indexed by rioff; no backward sweep, no H.
 // phase (MODE 1, childless blocks only): 0 = everything; 1 = forward half: Z, the diagonal Schur complements and the
 // log-density pieces, with Z parked in G's storage (nobody reads a childless block's G unless its slot becomes the
 // current one); 2 = the deferred half: Z is read back, scaled and pushed through the backward sweep into G.
@@ -108,9 +111,9 @@ build_level_body(const DevTree& T, const DevSlots& D, int rel, double* __restric
   // which theta-slot: read from the chain state in device memory (accept_make_change flips it there)
   const int phys = D.chain->cur ^ rel;
   const DevSlot S = pick_slot(D, phys);
-  double* __restrict__ outG = (MODE == 2) ? predG : S.G;
-  double* __restrict__ outH = (MODE != 2 && want_H) ? S.H : nullptr;
-  double* __restrict__ outRi = (MODE == 2) ? predRi : S.Ri;
+  double* __restrict__ outG = (MODE >= 2) ? predG : S.G;
+  double* __restrict__ outH = (MODE < 2 && want_H) ? S.H : nullptr;
+  double* __restrict__ outRi = (MODE >= 2) ? predRi : S.Ri;
   const CovTab& tab = D.chain->tab[phys];
   __shared__ CovTabS ct;
   __shared__ int s_cm[kMaxChain], s_crow[kMaxChain + 1], s_crow0g[kMaxChain], s_cgs[kMaxChain];
@@ -161,7 +164,7 @@ build_level_body(const DevTree& T, const DevSlots& D, int rel, double* __restric
   }
   __syncthreads();
   const int ncols = s_nc0[nn];
-  const int xcol = (MODE == 1 && phase != 0) ? 1 : 0;
+  const int xcol = ((MODE == 1 && phase != 0) || MODE == 3) ? 1 : 0;
   const int nmat = (MODE == 0 && T.limited) ? 2 : 1;  // limited trees factorise K_uu (marginal) next to the Schur complement
   const BuildPlan pl = build_plan(P, ncols + xcol, nmat * s_sumRb, s_maxmd, ns, (MODE == 0) ? min(nmat * nn, kBuildMaxThreads / 32) : 0, nwarps);
   const int Ppad = pl.Ppad, NCp = pl.NCp, NT = pl.NT, LD = pl.LD, SA = pl.SA, slotsz = pl.slot;
@@ -208,7 +211,7 @@ build_level_body(const DevTree& T, const DevSlots& D, int rel, double* __restric
       const int t = c - s_nc0[d], g = s_nrow0[d] + t;
       cxs[c] = T.cx[g]; cys[c] = T.cy[g]; cq[c] = T.mvq[g]; colnode[c] = d;
       colbase[c] = s_ngoff[d] + (long long)t * s_ngs[d];
-      wcol[c] = (MODE == 2) ? 0.0 : w[g];
+      wcol[c] = (MODE >= 2) ? 0.0 : w[g];
     } else {
       cxs[c] = 0; cys[c] = 0; cq[c] = 0; colnode[c] = -1; colbase[c] = -1; wcol[c] = 0;
     }
@@ -515,6 +518,9 @@ build_level_body(const DevTree& T, const DevSlots& D, int rel, double* __restric
         outRi[s_nrioff[d] + t] = ri;
         tvec[c] = ri * wcol[c];
         if (xcol) gw[c] = ri * gsum;  // G w_pa
+      } else if (MODE == 3) {
+        outG[s_nrioff[d] + t] = gsum;
+        outRi[s_nrioff[d] + t] = ok ? sqrt(R) : 0.0;  // as in-chain prediction (:1316-1322)
       } else {
         outRi[s_nrioff[d] + t] = ok ? sqrt(R) : 0.0;  // predict_std zeroes the sd when the Cholesky fails (:1316-1322)
       }
@@ -614,7 +620,9 @@ build_level_body(const DevTree& T, const DevSlots& D, int rel, double* __restric
       }
     }
   };
-  if (MODE == 2) {
+  if (MODE == 3) {
+    // (mean and sd are out)
+  } else if (MODE == 2) {
     bwd_sweep(outG, false, false);  // H of the prediction blocks
   } else if (MODE == 1 && phase == 1) {
     // forward half only: park Z (unscaled) where G will go; the backward sweep runs if and when the slot is taken up
@@ -743,7 +751,8 @@ cudaError_t launch_build(int mode, const DevTree& T, const DevSlots& D, int rel,
   if (ngrp <= 0) return cudaSuccess;
   if (mode == 0) return launch_build_t<0>(T, D, rel, predG, predRi, want_H, grp_slot0, grp_nn, ngrp, w, fail, ns, phase, smem, st, nthreads, prof, pdl, run_flag);
   if (mode == 1) return launch_build_t<1>(T, D, rel, predG, predRi, want_H, grp_slot0, grp_nn, ngrp, w, fail, ns, phase, smem, st, nthreads, prof, pdl, run_flag);
-  return launch_build_t<2>(T, D, rel, predG, predRi, want_H, grp_slot0, grp_nn, ngrp, w, fail, ns, phase, smem, st, nthreads, prof, pdl, run_flag);
+  if (mode == 2) return launch_build_t<2>(T, D, rel, predG, predRi, want_H, grp_slot0, grp_nn, ngrp, w, fail, ns, phase, smem, st, nthreads, prof, pdl, run_flag);
+  return launch_build_t<3>(T, D, rel, predG, predRi, want_H, grp_slot0, grp_nn, ngrp, w, fail, ns, phase, smem, st, nthreads, prof, pdl, run_flag);
 }
 
 }  // namespace st

@@ -151,6 +151,10 @@ int st_get_loglik_w(st_handle* h, int slot, double* out2) {
 }
 int st_accept_make_change(st_handle* h) {
   if (!h) return ST_ERR_INVALID;
+  if (h->model.alter_scratch) {
+    h->model.err = "the alter slot holds a BUILD of st_predict_new: st_get_loglik_comps_w(h, 1, ...) rebuilds it first";
+    return ST_ERR_INVALID;
+  }
   activate(h);
   h->model.accept_make_change();
   return ST_OK;
@@ -222,6 +226,12 @@ int st_mcmc_run(st_handle* h, const st_mcmc_opts* opts, st_mcmc_out* out) {
   if (!h || !opts || !out || !opts->set_unif_bounds || !opts->mcmcsd || opts->keep < 0 || opts->thin < 1) return ST_ERR_INVALID;
   activate(h);
   ST_GUARD_BEGIN return st::mcmc_run(h->model, *opts, *out);
+  ST_GUARD_END(h)
+}
+int st_predict_new(st_handle* h, const st_new_rows* rows, const st_pred_samples* samples, st_pred_out* out) {
+  if (!h || !rows || !samples || !out) return ST_ERR_INVALID;
+  activate(h);
+  ST_GUARD_BEGIN return h->model.predict_new(*rows, *samples, *out);
   ST_GUARD_END(h)
 }
 int st_bench_iteration(st_handle* h, const double* theta_prop, int do_swap, uint64_t seed, double* out3, float* ms_out) {
@@ -350,6 +360,24 @@ int st_make_tree(const st_tree_opts* o, st_tree** out) {
   return ST_OK;
 }
 void st_tree_destroy(st_tree* t) { delete t; }
+int st_tree_attach(const st_tree* t, int64_t n_new, const double* coords_new, const int64_t* mv_new, int32_t limited,
+                   int64_t* group, int64_t* par_ptr, int64_t* par_idx, int64_t* counts) {
+  if (!t || !counts || n_new < 0 || (n_new > 0 && (!coords_new || !mv_new))) return ST_ERR_INVALID;
+  try {
+    st::ivec g;
+    st::CSR par;
+    std::string e;
+    if (!st::tree_attach(t->t, coords_new, mv_new, n_new, limited != 0, g, par, e)) { g_create_error = e; return ST_ERR_INVALID; }
+    counts[0] = (int64_t)par.ptr.size() - 1; counts[1] = (int64_t)par.idx.size();
+    if (par_idx) {
+      if (!group || !par_ptr) return ST_ERR_INVALID;
+      std::copy(g.begin(), g.end(), group);
+      std::copy(par.ptr.begin(), par.ptr.end(), par_ptr);
+      std::copy(par.idx.begin(), par.idx.end(), par_idx);
+    }
+  } catch (const std::exception& ex) { g_create_error = ex.what(); return ST_ERR_INVALID; } catch (...) { return ST_ERR_INVALID; }
+  return ST_OK;
+}
 int st_tree_sizes(const st_tree* t, int64_t* o) {
   if (!t || !o) return ST_ERR_INVALID;
   o[0] = t->t.n_blocks; o[1] = (int64_t)t->t.res_is_ref.size(); o[2] = t->t.parchi_rows; o[3] = t->t.parchi_cols;

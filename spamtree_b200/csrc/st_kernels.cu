@@ -1106,4 +1106,78 @@ cudaError_t launch_chain_tick(ChainDev* C, cudaStream_t st) {
   return cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------ predict_new
+// normals of the draws at new rows: key = stream + row (the caller's index of the new row), counter = position of the sample
+// in the call — the same numbers whatever the launch shape or the layout of the rows into pseudo-blocks
+constexpr unsigned long long kStreamPredW = 5ULL << 48, kStreamPredY = 6ULL << 48;
+
+// w of sample b of a staged block (element (row, b) at src[row * si + b * sb], boundary order) -> node-major order
+__global__ void gather_sample_kernel(const double* __restrict__ src, long long si, long long sb, int b, const long long* __restrict__ perm,
+                                     double* __restrict__ dst, long long n) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) dst[i] = src[perm[i] * si + (long long)b * sb];
+}
+cudaError_t launch_gather_sample(const double* src, long long si, long long sb, int b, const long long* perm, double* dst, long long n,
+                                 cudaStream_t st) {
+  if (n <= 0) return cudaSuccess;
+  gather_sample_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(src, si, sb, b, perm, dst, n);
+  return cudaGetLastError();
+}
+
+// w_new = mean + sd z, y_new = x' beta[:, mv] + w_new + sqrt(tausq[mv]) eps (spamtree_fit.cpp:384), one thread per new row;
+// the running mean / sum of squared deviations of both over the samples of the call (Welford, FP64, in sample order)
+__global__ void predict_draw_kernel(long long n, const long long* __restrict__ lay2row, const int* __restrict__ mvq,
+                                    const double* __restrict__ X, int p, const double* __restrict__ mean, const double* __restrict__ sd,
+                                    const __grid_constant__ PredDrawPack pk, uint64_t seed, int j, const double* __restrict__ z,
+                                    const double* __restrict__ eps, double* __restrict__ wout, double* __restrict__ yout,
+                                    double* __restrict__ mout, double* __restrict__ sdout, double* __restrict__ acc) {
+  const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const long long i = lay2row[k];
+  const int qi = mvq[i];
+  const double zz = z ? z[i] : philox_normal(seed, kStreamPredW + (unsigned long long)i, (uint64_t)j);
+  const double ee = eps ? eps[i] : philox_normal(seed, kStreamPredY + (unsigned long long)i, (uint64_t)j);
+  const double wv = mean[k] + sd[k] * zz;
+  double xb = 0;
+  if (X)
+    for (int a = 0; a < p; a++) xb += X[i + (size_t)a * n] * pk.beta[a + qi * p];
+  const double yv = xb + wv + pk.sdtau[qi] * ee;
+  wout[i] = wv;
+  yout[i] = yv;
+  if (mout) mout[i] = mean[k];
+  if (sdout) sdout[i] = sd[k];
+  const double cnt = (double)(j + 1);
+  double* a = acc + 4 * i;  // {mean w, M2 w, mean y, M2 y}
+  if (j == 0) { a[0] = wv; a[1] = 0.0; a[2] = yv; a[3] = 0.0; return; }
+  const double dw = wv - a[0];
+  a[0] += dw / cnt;
+  a[1] += dw * (wv - a[0]);
+  const double dy = yv - a[2];
+  a[2] += dy / cnt;
+  a[3] += dy * (yv - a[2]);
+}
+cudaError_t launch_predict_draw(long long n, const long long* lay2row, const int* mvq, const double* X, int p, const double* mean,
+                                const double* sd, const PredDrawPack& pk, uint64_t seed, int j, const double* z, const double* eps,
+                                double* wout, double* yout, double* mout, double* sdout, double* acc, cudaStream_t st) {
+  if (n <= 0) return cudaSuccess;
+  predict_draw_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, lay2row, mvq, X, p, mean, sd, pk, seed, j, z, eps, wout, yout, mout,
+                                                                   sdout, acc);
+  return cudaGetLastError();
+}
+// per-row summaries of the call's S samples: mean and sd (ddof = 1; 0 for one sample) of w_new and y_new
+__global__ void predict_moments_kernel(long long n, int S, const double* __restrict__ acc, double* __restrict__ out4) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double* a = acc + 4 * i;
+  out4[i] = a[0];
+  out4[n + i] = S > 1 ? sqrt(a[1] / (S - 1)) : 0.0;
+  out4[2 * n + i] = a[2];
+  out4[3 * n + i] = S > 1 ? sqrt(a[3] / (S - 1)) : 0.0;
+}
+cudaError_t launch_predict_moments(long long n, int S, const double* acc, double* out4, cudaStream_t st) {
+  if (n <= 0 || S <= 0) return cudaSuccess;
+  predict_moments_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, S, acc, out4);
+  return cudaGetLastError();
+}
+
 }  // namespace st

@@ -42,7 +42,8 @@ inline cudaError_t ensure_dynamic_smem(K kern, size_t smem, SmemOptIn& table) {
 
 // Slot arguments: `D` holds both theta-slots and the device chain state; `rel` = 0 selects param_data, 1 alter_data
 // (the kernel reads chain->cur).  `run_flag` (or NULL): device int, the launch is a no-op when it is 0.
-// mode 0 / 1: reference / non-reference level of the slot; mode 2: prediction blocks (predG = Hpred receives H, predRi = sd).
+// mode 0 / 1: reference / non-reference level of the slot; mode 2: prediction blocks (predG = Hpred receives H, predRi = sd);
+// mode 3: forward-only prediction of new rows (predG receives mean = K_{u,pa} K_pa^-1 w_pa, predRi sd, both at rioff).
 cudaError_t launch_build(int mode, const DevTree& T, const DevSlots& D, int rel, double* predG, double* predRi, int want_H,
                          const int* grp_slot0, const int* grp_nn, int ngrp, const double* w, int* fail, int ns, int phase, size_t smem,
                          cudaStream_t st, int nthreads, unsigned long long* prof = nullptr, bool pdl = false,
@@ -108,5 +109,20 @@ struct ThetaPack {
 };
 cudaError_t launch_chain_set_theta(ChainDev* C, int rel, const ThetaPack& pack, cudaStream_t st);
 cudaError_t launch_chain_flip(ChainDev* C, cudaStream_t st);
+// ---- predict_new (Model::predict_new)
+// dst[i] = src[perm[i] * si + b * sb]: sample b of a staged block of samples, boundary order -> node-major order
+cudaError_t launch_gather_sample(const double* src, long long si, long long sb, int b, const long long* perm, double* dst, long long n,
+                                 cudaStream_t st);
+struct PredDrawPack {
+  double beta[kMaxStats];  // p x q of the sample
+  double sdtau[kMaxQ];     // sqrt(tausq) per outcome
+};
+// draws of sample j (position in the call) at n new rows: layout position k (mean / sd) -> caller row lay2row[k] (mvq, X
+// (n x p, column-major, or NULL), z / eps (or NULL: Philox keyed by (seed, row, j)), outputs, acc: 4 doubles per row)
+cudaError_t launch_predict_draw(long long n, const long long* lay2row, const int* mvq, const double* X, int p, const double* mean,
+                                const double* sd, const PredDrawPack& pk, uint64_t seed, int j, const double* z, const double* eps,
+                                double* wout, double* yout, double* mout, double* sdout, double* acc, cudaStream_t st);
+// out4 = {mean w, sd w, mean y, sd y} (n each) from acc after S samples
+cudaError_t launch_predict_moments(long long n, int S, const double* acc, double* out4, cudaStream_t st);
 
 }  // namespace st

@@ -186,6 +186,41 @@ int Model::build_bookkeeping(std::string& e) {
 // ------------------------------------------------------------------------------------------------------ layout
 static inline long long pad2(long long v) { return (v + 1) & ~1LL; }
 
+// BUILD launches of a list of work groups (slot s, nn sibling blocks, NT 8-column tiles): buckets by width (up to 4, 8, 16
+// tiles) so that narrow groups are not launched with the shared memory and CTA size of the widest one, and the ring depth of
+// each bucket; need(g, ns, nwarps) = shared memory of group g.  The groups go to (slot0, nn) in launch order.
+void Model::bucket_groups(const std::vector<GroupSpec>& gs, const std::function<size_t(const GroupSpec&, int, int)>& need,
+                          std::vector<int>& slot0, std::vector<int>& nn, std::vector<LevelInfo::BuildLaunch>& out) const {
+  const int wmax = kBuildMaxThreads / 32;
+  const size_t half_sm = (size_t)113 * 1024;
+  for (int b = 0; b < 3; b++) {
+    const int lo = (b == 0) ? 0 : (b == 1 ? 4 : 8), hi = (b == 0) ? 4 : (b == 1 ? 8 : 16);
+    LevelInfo::BuildLaunch bl;
+    bl.grp0 = (int)slot0.size();
+    size_t need1 = 0, need2 = 0;
+    int maxNT = 1;
+    for (const GroupSpec& g : gs)
+      if (g.NT > lo && g.NT <= hi) maxNT = std::max(maxNT, g.NT);
+    const int nw = std::min(wmax, std::max(4, (2 * maxNT) & ~3));
+    for (const GroupSpec& g : gs)
+      if (g.NT > lo && g.NT <= hi) {
+        slot0.push_back(g.s); nn.push_back(g.nn);
+        need1 = std::max(need1, need(g, 1, nw));
+        need2 = std::max(need2, need(g, 2, nw));
+      }
+    bl.ngrp = (int)slot0.size() - bl.grp0;
+    if (bl.ngrp == 0) continue;
+    // ring depth: double-buffered when it fits; single-buffered when that lets two CTAs share an SM (they overlap instead)
+    if (force_build_ns == 1 || force_build_ns == 2) bl.ns = (force_build_ns == 2 && need2 <= smem_budget) ? 2 : 1;
+    else if (need2 <= half_sm) bl.ns = 2;
+    else if (need1 <= half_sm) bl.ns = 1;
+    else bl.ns = (need2 <= smem_budget) ? 2 : 1;
+    bl.smem = (bl.ns == 2) ? need2 : need1;
+    bl.threads = 32 * nw;
+    out.push_back(bl);
+  }
+}
+
 int Model::build_layout(std::string& e) {
   const int nb = n_blocks;
   slot_of_block.assign(nb, -1);
@@ -431,10 +466,8 @@ int Model::build_layout(std::string& e) {
         if (h_child_ptr[t + 1] > h_child_ptr[t] || h_lastpar[t] < 0) L.deferrable = false;
     }
     const int xcol = L.deferrable ? 1 : 0;  // the deferred scheme carries w_pa as one extra panel column
-    struct Grp { int s, nn, NT; };
     const int wmax = kBuildMaxThreads / 32;
-    auto warps_for = [&](int NT) { return std::min(wmax, std::max(4, (2 * NT) & ~3)); };
-    std::vector<Grp> gs;
+    std::vector<GroupSpec> gs;
     int s = L.slot0;
     while (s < end) {
       int nn = 0;
@@ -455,34 +488,8 @@ int Model::build_layout(std::string& e) {
       L.maxNC = std::max(L.maxNC, best.NCp);
       s += nn;
     }
-    // buckets by width: up to 4, 8, 16 tiles of 8 columns
-    const size_t half_sm = (size_t)113 * 1024;
-    for (int b = 0; b < 3; b++) {
-      const int lo = (b == 0) ? 0 : (b == 1 ? 4 : 8), hi = (b == 0) ? 4 : (b == 1 ? 8 : 16);
-      LevelInfo::BuildLaunch bl;
-      bl.grp0 = (int)h_grp_slot0.size();
-      size_t need1 = 0, need2 = 0;
-      int maxNT = 1;
-      for (const Grp& g : gs)
-        if (g.NT > lo && g.NT <= hi) maxNT = std::max(maxNT, g.NT);
-      const int nw = warps_for(maxNT);
-      for (const Grp& g : gs)
-        if (g.NT > lo && g.NT <= hi) {
-          h_grp_slot0.push_back(g.s); h_grp_nn.push_back(g.nn);
-          need1 = std::max(need1, group_plan(g.s, g.nn, mode, 1, nw, xcol).total);
-          need2 = std::max(need2, group_plan(g.s, g.nn, mode, 2, nw, xcol).total);
-        }
-      bl.ngrp = (int)h_grp_slot0.size() - bl.grp0;
-      if (bl.ngrp == 0) continue;
-      // ring depth: double-buffered when it fits; single-buffered when that lets two CTAs share an SM (they overlap instead)
-      if (force_build_ns == 1 || force_build_ns == 2) bl.ns = (force_build_ns == 2 && need2 <= smem_budget) ? 2 : 1;
-      else if (need2 <= half_sm) bl.ns = 2;
-      else if (need1 <= half_sm) bl.ns = 1;
-      else bl.ns = (need2 <= smem_budget) ? 2 : 1;
-      bl.smem = (bl.ns == 2) ? need2 : need1;
-      bl.threads = 32 * nw;
-      L.build_launches.push_back(bl);
-    }
+    bucket_groups(gs, [&](const GroupSpec& g, int ns, int nw) { return group_plan(g.s, g.nn, mode, ns, nw, xcol).total; }, h_grp_slot0,
+                  h_grp_nn, L.build_launches);
     L.ngrp = (int)h_grp_slot0.size() - L.grp0;
     for (int t = L.slot0; t < end; t++) {
       L.maxP = std::max(L.maxP, h_P[t]); L.maxm = std::max(L.maxm, h_m[t]); L.maxk = std::max(L.maxk, h_k[t]);
@@ -996,6 +1003,7 @@ int Model::get_loglik_comps_w(int slot, double* out3) {
   const bool ok = r3[2] == 0.0;
   if (ok) { loglik_w[ps] = r3[0]; logdetCi[ps] = r3[1]; }  // on failure the reference leaves them untouched (:971-982)
   if (ps == cur) { gram_stale = true; pred_H_valid = false; }
+  else alter_scratch = false;
   out3[0] = loglik_w[ps]; out3[1] = logdetCi[ps]; out3[2] = ok ? 1.0 : 0.0;
   return 0;
 }
@@ -1110,6 +1118,7 @@ int Model::deal_with_w(const double* z, uint64_t seed) {
 int Model::get_loglik_w(int slot, double* out2) {
   if (!stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
   const int ps = phys(slot);
+  if (ps != cur && alter_scratch) { err = "the alter slot holds a BUILD of st_predict_new: st_get_loglik_comps_w(h, 1, ...) rebuilds it first"; return 1; }
   { int rc = complete_slot(ps); if (rc) return rc; }
   ST_CUDA(launch_llw(dt, dslots, ps == cur ? 0 : 1, 0, n_obs_nodes, d_w, llw_maxlen_, stream), "llw_kernel");
   n_launches++;
@@ -1702,6 +1711,7 @@ int Model::bench_iteration(const double* theta_prop, int do_swap, uint64_t seed,
   std::copy(theta_prop, theta_prop + pk.n, pk.theta);
   if (!make_covtab(theta_prop, pk.n, q, pk.tab, e)) { err = e; return 1; }
   ST_CUDA(launch_chain_set_theta(d_mc, 1, pk, stream), "chain_set_theta_kernel");
+  alter_scratch = false;  // (the iteration builds the alter slot for theta_prop)
   st_mcmc_opts o{};
   o.sample_beta = o.sample_tausq = o.sample_theta = o.sample_w = 1;
   o.seed = seed;
@@ -1879,6 +1889,306 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   out.n_chol_fail = h_mc->n_chol_fail;
   if (h_mc->gibbs_fail) { err = "Error at gibbs_sample_w: conditional precision not positive definite"; return 3; }
   if (h_mc->nan_loglik) { err = "At nan loglik: error."; return 5; }
+  return 0;
+}
+
+
+// ------------------------------------------------------------------------------------------------------ predict_new
+// Posterior predictive draws at new rows from saved samples (DESIGN.md, "Prediction at new locations").  The new rows are
+// laid out as extra nodes behind the tree: rows of one parent chain, split into pseudo-blocks narrow enough for one BUILD
+// work group (they are conditionally independent, so any split is exact), appended to temporary copies of the per-node and
+// per-row arrays.  Per sample: BUILD of the reference levels into the alter slot when theta changed, w_s into node order,
+// build_level_kernel<3> (forward sweep only: mean and sd per row), predict_draw_kernel; the draws leave on a copy stream.
+int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_out& out) {
+  if (!stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
+  if (part) { err = "predict_new: partitioned handles are not supported"; return 4; }
+  out.n_builds = 0;
+  const int64_t nn = R.n_new;
+  const int S = PS.n_samples;
+  const int npar = (int)theta[0].size();
+  if (nn < 0 || S < 0) { err = "predict_new: negative n_new or n_samples"; return 1; }
+  if (nn == 0 || S == 0) return 0;
+  if (!R.coords || !R.mv_id || !R.group || !R.parents_ptr || R.n_groups < 1 || !PS.theta || !PS.beta || !PS.tausq || !PS.w) {
+    err = "predict_new: a required input is missing";
+    return 1;
+  }
+  if (nn >= (1LL << 31) - n_all) { err = "predict_new: too many new rows"; return 4; }
+  const int64_t ng = R.n_groups;
+  if (R.parents_ptr[0] != 0) { err = "predict_new: parents_ptr[0] must be 0"; return 1; }
+  for (int64_t g = 0; g < ng; g++)
+    if (R.parents_ptr[g + 1] <= R.parents_ptr[g]) { err = "predict_new: a group has no parents (or parents_ptr decreases)"; return 1; }
+  if (!R.parents_idx) { err = "predict_new: parents_idx missing"; return 1; }
+  // every group's parents must be a chain of observed reference blocks: parents(lp) followed by lp (limited: lp alone)
+  std::vector<int> glast(ng);
+  for (int64_t g = 0; g < ng; g++) {
+    const int64_t* pl = R.parents_idx + R.parents_ptr[g];
+    const int64_t np = R.parents_ptr[g + 1] - R.parents_ptr[g];
+    for (int64_t t = 0; t < np; t++)
+      if (pl[t] < 0 || pl[t] >= n_blocks) { err = "predict_new: a parent id is outside 0..n_blocks-1"; return 1; }
+    const int64_t lp = pl[np - 1];
+    const int sl = slot_of_block[lp];
+    if (sl < 0 || sl >= n_obs_nodes || block_ct_obs[lp] == 0 || !block_is_reference[lp]) {
+      err = "predict_new: the last parent of a group is not an observed reference block";
+      return 1;
+    }
+    if (limited ? np != 1 : (parents.len(lp) != np - 1 || !std::equal(parents.row(lp), parents.row(lp) + (np - 1), pl))) {
+      err = limited ? "predict_new: limited_tree = TRUE: a group lists more than one parent"
+                    : "predict_new: a group's parents are not the ancestor chain of its last parent";
+      return 1;
+    }
+    glast[g] = sl;
+  }
+  for (int64_t i = 0; i < nn; i++) {
+    if (R.group[i] < 0 || R.group[i] >= ng) { err = "predict_new: a group id is outside 0..n_groups-1"; return 1; }
+    if (R.mv_id[i] < 1 || R.mv_id[i] > q) { err = "predict_new: mv_id outside 1..q"; return 1; }
+    if (!std::isfinite(R.coords[i]) || !std::isfinite(R.coords[i + nn])) { err = "predict_new: coords hold a non-finite value"; return 1; }
+  }
+  const bool cmaj = PS.w_row_stride == 1 && PS.w_sample_stride >= n_all;  // one sample per contiguous column
+  const bool rmaj = PS.w_sample_stride == 1 && PS.w_row_stride >= S;       // one row's samples contiguous
+  if (!cmaj && !rmaj) { err = "predict_new: w strides must be (1, >= n_all) or (>= n_samples, 1)"; return 1; }
+  for (int s = 0; s < S; s++)
+    for (int j = 0; j < q; j++)
+      if (!(PS.tausq[j + (size_t)s * q] >= 0.0)) { err = "predict_new: tausq must be non-negative"; return 1; }
+
+  // ---- layout: rows by parent chain (slot of the last parent), caller order inside; pseudo-blocks of at most mcap rows
+  std::vector<int64_t> lay2row(nn);
+  std::iota(lay2row.begin(), lay2row.end(), 0);
+  std::stable_sort(lay2row.begin(), lay2row.end(), [&](int64_t a, int64_t b) { return glast[R.group[a]] < glast[R.group[b]]; });
+  const int wmax = kBuildMaxThreads / 32;
+  const int col_cap = std::min(max_group_cols, kMaxGroupCols);
+  std::vector<int> pm, prow0, pk, pP, pchoff, pchain, pcpoff;
+  std::vector<long long> prioff;
+  for (int64_t k0 = 0; k0 < nn;) {
+    const int lp = glast[R.group[lay2row[k0]]];
+    int64_t k1 = k0;
+    while (k1 < nn && glast[R.group[lay2row[k1]]] == lp) k1++;
+    // the chain: the parent's own chain + the parent (limited trees: the parent alone, its marginal factor)
+    std::vector<int> ch;
+    if (!limited) ch.assign(h_chain.begin() + h_chain_off[lp], h_chain.begin() + h_chain_off[lp] + h_k[lp]);
+    ch.push_back(lp);
+    if ((int)ch.size() > kMaxChain) { err = "predict_new: ancestor chains longer than 32 are not supported"; return 4; }
+    int P = 0;
+    std::vector<int> poff;
+    for (int a : ch) { poff.push_back(P); P += h_m[a]; }
+    int mcap = col_cap - 1;  // (the w_pa column takes one)
+    while (mcap >= 1 && build_plan(P, mcap + 1, 0, mcap, 1, 0, wmax).total > smem_budget) mcap--;
+    if (mcap < 1) { err = "predict_new: a parent set is too large for one BUILD work group (P=" + std::to_string(P) + ")"; return 4; }
+    for (int64_t b0 = k0; b0 < k1; b0 += mcap) {
+      const int m = (int)std::min<int64_t>(mcap, k1 - b0);
+      pm.push_back(m); prow0.push_back((int)(n_all + b0)); prioff.push_back(b0);
+      pk.push_back((int)ch.size()); pP.push_back(P); pchoff.push_back((int)(h_chain.size() + pchain.size()));
+      pchain.insert(pchain.end(), ch.begin(), ch.end());
+      pcpoff.insert(pcpoff.end(), poff.begin(), poff.end());
+    }
+    k0 = k1;
+  }
+  const int npb = (int)pm.size();
+  // work groups: one pseudo-block each (pseudo-blocks of one chain are already as wide as a group may be), bucketed by
+  // width as make_groups buckets a level's groups
+  std::vector<GroupSpec> specs;
+  for (int t = 0; t < npb; t++) specs.push_back({n_nodes + t, 1, build_plan(pP[t], pm[t] + 1, 0, pm[t], 1, 0, wmax).NT});
+  std::vector<LevelInfo::BuildLaunch> launches;
+  std::vector<int> gslot0, gnn;
+  bucket_groups(specs, [&](const GroupSpec& g, int ns, int nw) {
+    const int t = g.s - n_nodes;
+    return build_plan(pP[t], pm[t] + 1, 0, pm[t], ns, 0, nw).total;
+  }, gslot0, gnn, launches);
+
+  // ---- temporary device state (freed on every exit)
+  struct Scratch {
+    std::vector<void*> dev;
+    std::vector<void*> reg;
+    std::vector<cudaEvent_t> evs;
+    cudaStream_t cs = nullptr;
+    ~Scratch() {
+      if (cs) cudaStreamSynchronize(cs);
+      for (void* p : reg) cudaHostUnregister(p);
+      for (cudaEvent_t e : evs) cudaEventDestroy(e);
+      if (cs) cudaStreamDestroy(cs);
+      for (void* p : dev) cudaFree(p);
+    }
+  } X;
+  auto dalloc = [&](void** p, size_t bytes) -> cudaError_t {
+    cudaError_t e = cudaMalloc(p, std::max<size_t>(bytes, 8));
+    if (e == cudaSuccess) X.dev.push_back(*p);
+    return e;
+  };
+  // make sure the stream is idle before the scratch is freed on an early exit
+  struct StreamSync { cudaStream_t s; ~StreamSync() { cudaStreamSynchronize(s); } } ssync{stream};
+  const int64_t nrow2 = n_all + nn;
+  double *d_cx2, *d_cy2;
+  int* d_mvq2;
+  ST_CUDA(dalloc((void**)&d_cx2, nrow2 * sizeof(double)), "alloc");
+  ST_CUDA(dalloc((void**)&d_cy2, nrow2 * sizeof(double)), "alloc");
+  ST_CUDA(dalloc((void**)&d_mvq2, nrow2 * sizeof(int)), "alloc");
+  ST_CUDA(cudaMemcpyAsync(d_cx2, dt.cx, n_all * sizeof(double), cudaMemcpyDeviceToDevice, stream), "D2D cx");
+  ST_CUDA(cudaMemcpyAsync(d_cy2, dt.cy, n_all * sizeof(double), cudaMemcpyDeviceToDevice, stream), "D2D cy");
+  ST_CUDA(cudaMemcpyAsync(d_mvq2, dt.mvq, n_all * sizeof(int), cudaMemcpyDeviceToDevice, stream), "D2D mvq");
+  dvec ncx(nn), ncy(nn);
+  std::vector<int> nmvq(nn), cmvq(nn);
+  for (int64_t k = 0; k < nn; k++) {
+    const int64_t i = lay2row[k];
+    ncx[k] = R.coords[i]; ncy[k] = R.coords[i + nn]; nmvq[k] = (int)R.mv_id[i] - 1;
+  }
+  for (int64_t i = 0; i < nn; i++) cmvq[i] = (int)R.mv_id[i] - 1;
+  ST_CUDA(cudaMemcpyAsync(d_cx2 + n_all, ncx.data(), nn * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D new rows");
+  ST_CUDA(cudaMemcpyAsync(d_cy2 + n_all, ncy.data(), nn * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D new rows");
+  ST_CUDA(cudaMemcpyAsync(d_mvq2 + n_all, nmvq.data(), nn * sizeof(int), cudaMemcpyHostToDevice, stream), "H2D new rows");
+  // per node / per chain entry: the tree's arrays followed by the pseudo-blocks'
+  auto ext = [&](const auto& base, const auto& add, auto** d) -> cudaError_t {
+    using T = typename std::decay_t<decltype(base)>::value_type;
+    std::vector<T> v(base.begin(), base.end());
+    v.insert(v.end(), add.begin(), add.end());
+    cudaError_t e = dalloc((void**)d, v.size() * sizeof(T));
+    if (e != cudaSuccess) return e;
+    // (from pageable memory: the call returns once v has been staged, so v may go out of scope)
+    return cudaMemcpyAsync(*d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, stream);
+  };
+  std::vector<long long> zeros_ll(npb, 0);
+  std::vector<int> zeros_i(npb, 0);
+  int *d_m2, *d_row02, *d_k2, *d_P2, *d_choff2, *d_gs2, *d_chain2, *d_cpoff2;
+  long long *d_goff2, *d_rioff2;
+  ST_CUDA(ext(h_m, pm, &d_m2), "upload new nodes");
+  ST_CUDA(ext(h_row0, prow0, &d_row02), "upload new nodes");
+  ST_CUDA(ext(h_k, pk, &d_k2), "upload new nodes");
+  ST_CUDA(ext(h_P, pP, &d_P2), "upload new nodes");
+  ST_CUDA(ext(h_chain_off, pchoff, &d_choff2), "upload new nodes");
+  ST_CUDA(ext(h_gs, zeros_i, &d_gs2), "upload new nodes");
+  ST_CUDA(ext(h_goff, zeros_ll, &d_goff2), "upload new nodes");
+  ST_CUDA(ext(h_rioff, prioff, &d_rioff2), "upload new nodes");
+  ST_CUDA(ext(h_chain, pchain, &d_chain2), "upload new nodes");
+  ST_CUDA(ext(h_chain_poff, pcpoff, &d_cpoff2), "upload new nodes");
+  DevTree T2 = dt;
+  T2.cx = d_cx2; T2.cy = d_cy2; T2.mvq = d_mvq2;
+  T2.m = d_m2; T2.row0 = d_row02; T2.k = d_k2; T2.P = d_P2; T2.chain_off = d_choff2; T2.gs = d_gs2; T2.goff = d_goff2;
+  T2.rioff = d_rioff2; T2.chain = d_chain2; T2.chain_poff = d_cpoff2;
+  int *d_gslot0, *d_gnn, *d_cmvq;
+  long long *d_lay2row, *d_perm;
+  ST_CUDA(ext(std::vector<int>(), gslot0, &d_gslot0), "upload groups");
+  ST_CUDA(ext(std::vector<int>(), gnn, &d_gnn), "upload groups");
+  ST_CUDA(ext(std::vector<int>(), cmvq, &d_cmvq), "upload new rows");
+  ST_CUDA(ext(std::vector<long long>(), std::vector<long long>(lay2row.begin(), lay2row.end()), &d_lay2row), "upload layout");
+  ST_CUDA(ext(std::vector<long long>(), std::vector<long long>(perm.begin(), perm.end()), &d_perm), "upload perm");
+  double* d_Xn = nullptr;
+  if (R.X) {
+    ST_CUDA(dalloc((void**)&d_Xn, (size_t)nn * p * sizeof(double)), "alloc");
+    ST_CUDA(cudaMemcpyAsync(d_Xn, R.X, (size_t)nn * p * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D X_new");
+  }
+  // samples of w staged in blocks of B (one 2D copy each), the node-ordered w_s, mean / sd, normals, two output slots
+  const int B = (int)std::max<int64_t>(1, std::min<int64_t>(S, (256LL << 20) / (8 * n_all)));
+  double *d_wblk, *d_wnode, *d_mean, *d_sd, *d_acc, *d_zn = nullptr, *d_en = nullptr;
+  ST_CUDA(dalloc((void**)&d_wblk, (size_t)B * n_all * sizeof(double)), "alloc");
+  ST_CUDA(dalloc((void**)&d_wnode, n_all * sizeof(double)), "alloc");
+  ST_CUDA(dalloc((void**)&d_mean, nn * sizeof(double)), "alloc");
+  ST_CUDA(dalloc((void**)&d_sd, nn * sizeof(double)), "alloc");
+  ST_CUDA(dalloc((void**)&d_acc, 4 * nn * sizeof(double)), "alloc");
+  if (PS.z) ST_CUDA(dalloc((void**)&d_zn, nn * sizeof(double)), "alloc");
+  if (PS.eps) ST_CUDA(dalloc((void**)&d_en, nn * sizeof(double)), "alloc");
+  double* d_out[2][4];
+  for (int r = 0; r < 2; r++)
+    for (int c = 0; c < 4; c++) ST_CUDA(dalloc((void**)&d_out[r][c], nn * sizeof(double)), "alloc");
+  double* hout[4] = {out.w_new, out.y_new, out.mean, out.sd};
+  const bool any_draw_out = hout[0] || hout[1] || hout[2] || hout[3];
+  ST_CUDA(cudaStreamCreateWithFlags(&X.cs, cudaStreamNonBlocking), "cudaStreamCreate");
+  cudaEvent_t ready[2], copied[2];
+  for (int r = 0; r < 2; r++) {
+    ST_CUDA(cudaEventCreateWithFlags(&ready[r], cudaEventDisableTiming), "cudaEventCreate"); X.evs.push_back(ready[r]);
+    ST_CUDA(cudaEventCreateWithFlags(&copied[r], cudaEventDisableTiming), "cudaEventCreate"); X.evs.push_back(copied[r]);
+  }
+  bool pending[2] = {false, false};
+  for (double* hp : hout)  // page-locked for the duration of the call, so that the copies overlap the next sample
+    if (hp) {
+      if (cudaHostRegister(hp, (size_t)nn * S * sizeof(double), cudaHostRegisterPortable) == cudaSuccess) X.reg.push_back(hp);
+      else (void)cudaGetLastError();
+    }
+
+  int last_ref = 0;
+  while (last_ref < (int)levels.size() && levels[last_ref].is_ref) last_ref++;
+  dvec built;  // theta of the alter slot's BUILD (empty: none yet)
+  std::vector<int> build_of(S);  // the BUILD each sample is predicted from
+  int* d_bfail;                  // failed factorisations of each BUILD
+  ST_CUDA(dalloc((void**)&d_bfail, (size_t)S * sizeof(int)), "alloc");
+  const int alt = phys(1);
+  int si = 0, sb = 0;
+  for (int j = 0; j < S; j++) {
+    if (j % B == 0) {
+      const int nb = std::min(B, S - j);
+      if (rmaj) {
+        ST_CUDA(cudaMemcpy2DAsync(d_wblk, nb * sizeof(double), PS.w + j, PS.w_row_stride * sizeof(double), nb * sizeof(double), n_all,
+                                  cudaMemcpyHostToDevice, stream), "H2D w samples");
+        si = nb; sb = 1;
+      } else {
+        ST_CUDA(cudaMemcpy2DAsync(d_wblk, n_all * sizeof(double), PS.w + (size_t)j * PS.w_sample_stride, PS.w_sample_stride * sizeof(double),
+                                  n_all * sizeof(double), nb, cudaMemcpyHostToDevice, stream), "H2D w samples");
+        si = 1; sb = (int)n_all;
+      }
+    }
+    const double* th = PS.theta + (size_t)j * npar;
+    if (built.empty() || std::memcmp(built.data(), th, npar * sizeof(double)) != 0) {
+      ThetaPack pkk;
+      std::string e;
+      pkk.n = npar;
+      std::copy(th, th + npar, pkk.theta);
+      if (!make_covtab(th, npar, q, pkk.tab, e)) { err = "predict_new: sample " + std::to_string(j) + ": " + e; return 1; }
+      ST_CUDA(launch_chain_set_theta(d_mc, 1, pkk, stream), "chain_set_theta_kernel");
+      deferred_[alt] = false;  // (from here on the slot holds the reference levels of this theta only)
+      alter_scratch = true;
+      const int rc = launch_build_levels(1, 0, last_ref, true, stream);
+      if (rc) return rc;
+      // the BUILD's failure count, kept per BUILD; the counter is the chain's and starts from zero again
+      ST_CUDA(cudaMemcpyAsync(d_bfail + out.n_builds, d_fail, sizeof(int), cudaMemcpyDeviceToDevice, stream), "D2D fail");
+      ST_CUDA(cudaMemsetAsync(d_fail, 0, sizeof(int), stream), "memset");
+      built.assign(th, th + npar);
+      out.n_builds++;
+    }
+    build_of[j] = (int)out.n_builds - 1;
+    ST_CUDA(launch_gather_sample(d_wblk, si, sb, j % B, d_perm, d_wnode, n_all, stream), "gather_sample_kernel");
+    for (const LevelInfo::BuildLaunch& L : launches)
+      ST_CUDA(launch_build(3, T2, dslots, 1, d_mean, d_sd, 0, d_gslot0 + L.grp0, d_gnn + L.grp0, L.ngrp, d_wnode, d_fail + 2, L.ns, 0,
+                           L.smem, stream, L.threads),
+              "build_level_kernel(predict_new)");
+    if (d_zn) ST_CUDA(cudaMemcpyAsync(d_zn, PS.z + (size_t)j * nn, nn * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D z");
+    if (d_en) ST_CUDA(cudaMemcpyAsync(d_en, PS.eps + (size_t)j * nn, nn * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D eps");
+    const int r = j & 1;
+    if (pending[r]) ST_CUDA(cudaStreamWaitEvent(stream, copied[r], 0), "wait for the copy of an earlier sample");
+    PredDrawPack pack{};
+    for (int jq = 0; jq < q; jq++) {
+      for (int a = 0; a < p; a++) pack.beta[a + jq * p] = PS.beta[a + (size_t)j * p + (size_t)jq * p * S];
+      pack.sdtau[jq] = std::sqrt(PS.tausq[jq + (size_t)j * q]);
+    }
+    ST_CUDA(launch_predict_draw(nn, d_lay2row, d_cmvq, d_Xn, p, d_mean, d_sd, pack, PS.seed, j, d_zn, d_en, d_out[r][0], d_out[r][1],
+                                d_out[r][2], d_out[r][3], d_acc, stream),
+            "predict_draw_kernel");
+    n_launches += 2 + (double)launches.size();
+    if (any_draw_out) {
+      ST_CUDA(cudaEventRecord(ready[r], stream), "event");
+      ST_CUDA(cudaStreamWaitEvent(X.cs, ready[r], 0), "wait");
+      for (int c = 0; c < 4; c++)
+        if (hout[c]) ST_CUDA(cudaMemcpyAsync(hout[c] + (size_t)j * nn, d_out[r][c], nn * sizeof(double), cudaMemcpyDeviceToHost, X.cs), "D2H draws");
+      ST_CUDA(cudaEventRecord(copied[r], X.cs), "event");
+      pending[r] = true;
+    }
+  }
+  double* hm[4] = {out.w_mean, out.w_sd, out.y_mean, out.y_sd};
+  if (hm[0] || hm[1] || hm[2] || hm[3]) {
+    double* d_mom = d_wblk;  // (free once the last gather has run: 4 nn doubles fit when nn <= B n_all / 4, else its own)
+    if (4 * nn > (int64_t)B * n_all) ST_CUDA(dalloc((void**)&d_mom, 4 * nn * sizeof(double)), "alloc");
+    ST_CUDA(launch_predict_moments(nn, S, d_acc, d_mom, stream), "predict_moments_kernel");
+    for (int c = 0; c < 4; c++)
+      if (hm[c]) ST_CUDA(cudaMemcpyAsync(hm[c], d_mom + (size_t)c * nn, nn * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H moments");
+  }
+  std::vector<int> bfail(out.n_builds);
+  ST_CUDA(cudaMemcpyAsync(bfail.data(), d_bfail, bfail.size() * sizeof(int), cudaMemcpyDeviceToHost, stream), "D2H fail");
+  // the one synchronisation
+  ST_CUDA(cudaStreamSynchronize(stream), "sync");
+  ST_CUDA(cudaStreamSynchronize(X.cs), "sync copies");
+  // a theta whose covariance is not positive definite on some reference block: the chain would have rejected it, and its
+  // draws are not draws of the model (the factor rows of that block are zeroed)
+  for (int j = 0; j < S; j++)
+    if (bfail[build_of[j]] != 0) {
+      err = "predict_new: theta of sample " + std::to_string(j) + ": a reference-level Cholesky factorisation failed (covariance not positive definite)";
+      return 3;
+    }
   return 0;
 }
 

@@ -10,6 +10,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <functional>
 #include <string>
 
 #include "../../include/spamtree_b200.h"
@@ -90,6 +91,8 @@ struct LevelInfo {
   bool gram_skip = false;          // every block of the level is fused into its parent
 };
 
+struct GroupSpec { int s, nn, NT; };  // a BUILD work group: nn sibling blocks from slot s, NT tiles of 8 columns
+
 class Model {
  public:
   ~Model();
@@ -163,6 +166,7 @@ class Model {
   HostRng rng;
   bool gram_stale = true;         // message Grams depend on the param slot's theta only
   bool pred_H_valid = false;
+  bool alter_scratch = false;     // the alter slot holds a predict_new BUILD, not theta[alter]'s: rebuilt before it is read
   uint64_t sweep_counter = 0;
   // ---- device
   DevTree dt{};
@@ -238,11 +242,15 @@ class Model {
   int set_widx_mode(bool faithful_index);
   // ---- the device-resident chain (rng_mode 1): spamtree_fit.cpp:167-391 without a host round trip per iteration
   int chain_run(const st_mcmc_opts& o, st_mcmc_out& out);
+  // ---- prediction at new rows from saved samples (include/spamtree_b200.h: st_predict_new)
+  int predict_new(const st_new_rows& rows, const st_pred_samples& ps, st_pred_out& out);
 
  private:
   int phys(int slot) const { return slot ? 1 - cur : cur; }
   int build_bookkeeping(std::string& e);
   int build_layout(std::string& e);
+  void bucket_groups(const std::vector<GroupSpec>& gs, const std::function<size_t(const GroupSpec&, int, int)>& need,
+                     std::vector<int>& slot0, std::vector<int>& nn, std::vector<LevelInfo::BuildLaunch>& out) const;
   int upload(std::string& e);
   int launch_build_levels(int rel, int l0, int l1, bool no_density, cudaStream_t st);
   int complete_slot(int pslot);  // the deferred half of BUILD for the slot's childless levels, if pending

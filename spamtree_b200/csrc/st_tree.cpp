@@ -273,6 +273,37 @@ struct NNGrid {
 
 }  // namespace
 
+// per-margin 1-NN targets among rows of the last loop level (:218, :322): parent_block[i] = block of the target nearest to
+// query i, among the targets of the query's own margin when same_margin is set (any margin when that one has none)
+void nn_assign(const NNTargets& t, const double* qx, const double* qy, const int64_t* qmv, int64_t nq, bool same_margin,
+               ivec& parent_block) {
+  parent_block.assign(nq, 0);
+  std::vector<int64_t> margins;
+  if (same_margin) {
+    margins.assign(qmv, qmv + nq);
+    std::sort(margins.begin(), margins.end());
+    margins.erase(std::unique(margins.begin(), margins.end()), margins.end());
+  } else {
+    margins.push_back(-1);
+  }
+  const int64_t nt = (int64_t)t.x.size();
+  for (int64_t vv : margins) {
+    ivec tsel;
+    for (int64_t r = 0; r < nt; r++)
+      if (vv < 0 || t.mv[r] == vv) tsel.push_back(r);
+    if (tsel.empty())  // FNN would stop here; fall back to any margin
+      for (int64_t r = 0; r < nt; r++) tsel.push_back(r);
+    dvec tx(tsel.size()), ty(tsel.size());
+    for (size_t i = 0; i < tsel.size(); i++) { tx[i] = t.x[tsel[i]]; ty[i] = t.y[tsel[i]]; }
+    NNGrid g;
+    g.build(tx.data(), ty.data(), (int64_t)tsel.size());
+    for (int64_t qi = 0; qi < nq; qi++) {
+      if (vv >= 0 && qmv[qi] != vv) continue;
+      parent_block[qi] = t.block[tsel[g.query(qx[qi], qy[qi])]];
+    }
+  }
+}
+
 // R/make_tree.R:1-420 (structure) + the tail of spamtree() that turns it into the boundary inputs
 // (R/spamtree_fit.R:288-324).
 bool make_tree(const double* coords, const double* y, const int64_t* mv_id, int64_t n_all, int cell_size, int K0,
@@ -454,32 +485,18 @@ bool make_tree(const double* coords, const double* y, const int64_t* mv_id, int6
   for (int64_t i = 0; i < n_all; i++) max_block_number = std::max(max_block_number, T.blocking[i]);
   const int64_t loop_max_res = nlev > 0 ? (start_level + nlev) : start_level;
 
-  // per-margin 1-NN targets among rows of the last loop level (:218, :322)
-  auto nn_assign = [&](const ivec& queries, const ivec& targets, ivec& parent_block) {
-    parent_block.assign(queries.size(), 0);
-    std::vector<int64_t> margins;
-    if (cherrypick_same_margin) {
-      for (int64_t r : queries) margins.push_back(mv_id[r]);
-      std::sort(margins.begin(), margins.end());
-      margins.erase(std::unique(margins.begin(), margins.end()), margins.end());
-    } else {
-      margins.push_back(-1);
-    }
-    for (int64_t vv : margins) {
-      ivec tsel;
-      for (int64_t r : targets)
-        if (vv < 0 || mv_id[r] == vv) tsel.push_back(r);
-      if (tsel.empty()) tsel = targets;  // FNN would stop here; fall back to any margin
-      dvec tx(tsel.size()), ty(tsel.size());
-      for (size_t i = 0; i < tsel.size(); i++) { tx[i] = X0[tsel[i]]; ty[i] = X1[tsel[i]]; }
-      NNGrid g;
-      g.build(tx.data(), ty.data(), (int64_t)tsel.size());
-      for (size_t qi = 0; qi < queries.size(); qi++) {
-        const int64_t r = queries[qi];
-        if (vv >= 0 && mv_id[r] != vv) continue;
-        parent_block[qi] = T.blocking[tsel[g.query(X0[r], X1[r])]];
-      }
-    }
+  // the 1-NN targets: rows of the last loop level (kept with the tree, st_tree_attach attaches new rows by the same rule)
+  T.last = NNTargets();
+  for (int64_t r : last_level_rows) {
+    T.last.x.push_back(X0[r]); T.last.y.push_back(X1[r]); T.last.mv.push_back(mv_id[r]); T.last.block.push_back(T.blocking[r]);
+  }
+  T.cherrypick_same_margin = cherrypick_same_margin;
+  T.n_loop_levels = nlev;
+  auto nn_rows = [&](const ivec& queries, ivec& parent_block) {
+    dvec qx(queries.size()), qy(queries.size());
+    ivec qmv(queries.size());
+    for (size_t i = 0; i < queries.size(); i++) { qx[i] = X0[queries[i]]; qy[i] = X1[queries[i]]; qmv[i] = mv_id[queries[i]]; }
+    nn_assign(T.last, qx.data(), qy.data(), qmv.data(), (int64_t)queries.size(), cherrypick_same_margin, parent_block);
   };
   // new block names: as.numeric(factor(parent block)) + max_block_number (:280, :385)
   auto rank_blocks = [&](const ivec& parent_block, ivec& newblock) {
@@ -504,7 +521,7 @@ bool make_tree(const double* coords, const double* y, const int64_t* mv_id, int6
   int64_t cur_max_res = loop_max_res;
   if (!cx.empty()) {  // leftovers (:213-305)
     ivec pblock, nblock;
-    nn_assign(cx, last_level_rows, pblock);
+    nn_rows(cx, pblock);
     rank_blocks(pblock, nblock);
     const int64_t res_left = loop_max_res + 1;
     for (size_t i = 0; i < cx.size(); i++) { T.blocking[cx[i]] = nblock[i]; T.res[cx[i]] = res_left; }
@@ -517,7 +534,7 @@ bool make_tree(const double* coords, const double* y, const int64_t* mv_id, int6
   if (T.res_is_ref.size() == 1) T.res_is_ref[0] = 1;  // :307-309
   if (!missing.empty()) {  // rows to predict (:317-413)
     ivec pblock, nblock;
-    nn_assign(missing, last_level_rows, pblock);
+    nn_rows(missing, pblock);
     rank_blocks(pblock, nblock);
     const int64_t res_miss = cur_max_res + 1;
     for (size_t i = 0; i < missing.size(); i++) { T.blocking[missing[i]] = nblock[i]; T.res[missing[i]] = res_miss; }
@@ -572,6 +589,56 @@ bool make_tree(const double* coords, const double* y, const int64_t* mv_id, int6
   ivec fill(T.indexing.ptr.begin(), T.indexing.ptr.end() - 1);
   for (int64_t i = 0; i < n_all; i++) T.indexing.idx[fill[T.blocking[i] - 1]++] = i;
   lap("names, groups, indexing");
+  return true;
+}
+
+// New rows attached to a built tree by the rule that makes the prediction level of make_tree (:317-413): the nearest row of
+// the last loop level names the parent block b, the rows of one b form one group (groups ordered by b, as rank_blocks
+// numbers them), and a group's parents are what make_edges / make_edges_limited would give a block in a column appended
+// to parchimat: the reference blocks on the chains through b, root first.
+bool tree_attach(const TreeResult& T, const double* coords_new, const int64_t* mv_new, int64_t n_new, bool limited, ivec& group,
+                 CSR& parents, std::string& err) {
+  group.assign(n_new, 0);
+  parents.ptr.assign(1, 0);
+  parents.idx.clear();
+  if (n_new == 0) return true;
+  if (T.last.x.empty() || T.n_loop_levels < 1) { err = "the tree has no loop level to attach rows to"; return false; }
+  for (int64_t i = 0; i < n_new; i++)
+    if (!std::isfinite(coords_new[i]) || !std::isfinite(coords_new[i + n_new])) { err = "coords_new holds a non-finite value"; return false; }
+  ivec pblock;
+  nn_assign(T.last, coords_new, coords_new + n_new, mv_new, n_new, T.cherrypick_same_margin, pblock);
+  ivec u(pblock);
+  std::sort(u.begin(), u.end());
+  u.erase(std::unique(u.begin(), u.end()), u.end());
+  for (int64_t i = 0; i < n_new; i++) group[i] = (int64_t)(std::lower_bound(u.begin(), u.end(), pblock[i]) - u.begin());
+  // make_edges' colselect for a column L = parchi_cols
+  const int L = T.parchi_cols;
+  const int64_t nr = T.parchi_rows;
+  ivec colselect;
+  for (int l = 0; l < L && l < (int)T.res_is_ref.size(); l++)
+    if (T.res_is_ref[l] == 1) colselect.push_back(l);
+  if (colselect.empty())
+    for (int c = 0; c < L; c++) colselect.push_back(c);
+  if (limited) colselect.assign(1, colselect.back());
+  // the chain rows through each b (the column of the last loop level)
+  const double* bcol = T.parchimat.data() + (size_t)(T.n_loop_levels - 1) * nr;
+  std::vector<ivec> par(u.size());
+  for (int64_t r = 0; r < nr; r++) {
+    if (!std::isfinite(bcol[r])) continue;
+    const auto it = std::lower_bound(u.begin(), u.end(), (int64_t)bcol[r]);
+    if (it == u.end() || *it != (int64_t)bcol[r]) continue;
+    ivec& vals = par[it - u.begin()];
+    for (int64_t c : colselect) {
+      const double v = T.parchimat[r + (size_t)c * nr];
+      if (std::isfinite(v)) vals.push_back((int64_t)v - 1);
+    }
+  }
+  for (auto& vals : par) {
+    std::sort(vals.begin(), vals.end());
+    vals.erase(std::unique(vals.begin(), vals.end()), vals.end());
+    parents.idx.insert(parents.idx.end(), vals.begin(), vals.end());
+    parents.ptr.push_back((int64_t)parents.idx.size());
+  }
   return true;
 }
 
