@@ -212,7 +212,7 @@ void Model::bucket_groups(const std::vector<GroupSpec>& gs, const std::function<
     if (bl.ngrp == 0) continue;
     // ring depth: double-buffered when it fits; single-buffered when that lets two CTAs share an SM (they overlap instead)
     if (force_build_ns == 1 || force_build_ns == 2) bl.ns = (force_build_ns == 2 && need2 <= smem_budget) ? 2 : 1;
-    else if (need2 <= half_sm) bl.ns = 2;
+    else if (need2 <= std::min(half_sm, smem_budget)) bl.ns = 2;  // (a budget set below half an SM holds for the ring too)
     else if (need1 <= half_sm) bl.ns = 1;
     else bl.ns = (need2 <= smem_budget) ? 2 : 1;
     bl.smem = (bl.ns == 2) ? need2 : need1;
@@ -465,8 +465,15 @@ int Model::build_layout(std::string& e) {
       for (int t = L.slot0; t < end; t++)
         if (h_child_ptr[t + 1] > h_child_ptr[t] || h_lastpar[t] < 0) L.deferrable = false;
     }
-    const int xcol = L.deferrable ? 1 : 0;  // the deferred scheme carries w_pa as one extra panel column
     const int wmax = kBuildMaxThreads / 32;
+    // the deferred scheme carries w_pa as one extra panel column: a block that fits one work group only without it (a leaf
+    // of 128 rows, or one at the edge of the shared-memory budget) keeps the whole level on the eager scheme
+    if (L.deferrable)
+      for (int t = L.slot0; t < end && L.deferrable; t++) {
+        const BuildPlan pl = group_plan(t, 1, mode, 1, wmax, 1);
+        if (pl.total > smem_budget || pl.NCp > kMaxGroupCols) L.deferrable = false;
+      }
+    const int xcol = L.deferrable ? 1 : 0;
     std::vector<GroupSpec> gs;
     int s = L.slot0;
     while (s < end) {
@@ -517,6 +524,8 @@ int Model::build_layout(std::string& e) {
         tiles = std::max(tiles, (td + 1) & ~1LL);
         maxitems = std::max(maxitems, items);
       }
+      L.gram_maxrows = maxrows;
+      L.gram_maxitems = maxitems;
       if (tiles * 8 > 160 * 1024) { e = "a block's message Gram tiles do not fit the Gram kernel's shared memory"; return 4; }
       L.gram_ldx = ldx;
       L.gram_tiles = (int)tiles;
@@ -1396,6 +1405,68 @@ int Model::get_index(const std::string& which, int u, int c, int64_t* out, int64
   if (which == "u_by_block_groups") {
     if (u < 0 || u >= n_actual_groups) { err = "group out of range"; return 1; }
     return emit(u_by_block_groups[u]);
+  }
+  if (which == "build_plan") {
+    // The launch plan chosen at creation (host-only handles too), for tests that must know which kernel paths a tree reaches.
+    // [n_launch, n_level], then n_launch records of 9 for the BUILD launches of every observed level and of the prediction
+    // level: {level (-1: prediction blocks), mode, groups, ns, threads, dynamic smem bytes, largest nn, largest NCp,
+    // largest npair}; then n_level records of 9 for the observed levels: {deferrable, early (BUILD underneath the sweep of
+    // a device-resident chain), gram_rch, largest staged rows of a block, gram_stage_off, gram_threads, largest children
+    // count, largest nch * ntile, largest Gram item count} (the last five over the blocks gram_level_kernel processes, i.e.
+    // not fused)
+    ivec lr;
+    int nlaunch = 0;
+    auto launches = [&](const LevelInfo& L, int lev, int mode) {
+      const int xcol = L.deferrable ? 1 : 0;
+      for (const auto& B : L.build_launches) {
+        long long mnn = 0, mncp = 0, mpair = 0;
+        for (int g = B.grp0; g < B.grp0 + B.ngrp; g++) {
+          int ncols = xcol;
+          for (int d = 0; d < h_grp_nn[g]; d++) ncols += h_m[h_grp_slot0[g] + d];
+          const int ncp = (ncols + 7) & ~7;
+          mnn = std::max<long long>(mnn, h_grp_nn[g]);
+          mncp = std::max<long long>(mncp, ncp);
+          mpair = std::max<long long>(mpair, build_npair(ncp >> 3, B.threads / 32));
+        }
+        r.insert(r.end(), {(int64_t)lev, (int64_t)mode, (int64_t)B.ngrp, (int64_t)B.ns, (int64_t)B.threads, (int64_t)B.smem, mnn, mncp, mpair});
+        nlaunch++;
+      }
+    };
+    for (int l = 0; l < (int)levels.size(); l++) {
+      const LevelInfo& L = levels[l];
+      launches(L, l, L.is_ref ? 0 : 1);
+      long long mch = 0, mct = 0;
+      for (int t = L.slot0; t < L.slot0 + L.nslots; t++) {
+        if (h_ufused[t]) continue;
+        const int nch = h_child_ptr[t + 1] - h_child_ptr[t];
+        mch = std::max<long long>(mch, nch);
+        mct = std::max<long long>(mct, (long long)nch * (h_k[t] + (h_soff[t] >= 0 ? 1 : 0)));
+      }
+      lr.insert(lr.end(), {(int64_t)L.deferrable, (int64_t)(overlap && l < n_early_levels_), (int64_t)L.gram_rch, (int64_t)L.gram_maxrows,
+                           (int64_t)L.gram_stage_off, (int64_t)L.gram_threads, mch, mct, (int64_t)L.gram_maxitems});
+    }
+    launches(pred_level, -1, 2);
+    r.insert(r.begin(), {(int64_t)nlaunch, (int64_t)levels.size()});
+    r.insert(r.end(), lr.begin(), lr.end());
+    return emit(r);
+  }
+  if (which == "build_groups") {
+    // every BUILD work group in launch order, 6 per group: {level (-1: prediction blocks), first slot, nn, NCp, threads,
+    // npair}.  Two handles whose groups agree run the same reductions for every block.
+    auto groups = [&](const LevelInfo& L, int lev) {
+      const int xcol = L.deferrable ? 1 : 0;
+      for (const auto& B : L.build_launches)
+        for (int g = B.grp0; g < B.grp0 + B.ngrp; g++) {
+          int ncols = xcol;
+          for (int d = 0; d < h_grp_nn[g]; d++) ncols += h_m[h_grp_slot0[g] + d];
+          const int ncp = (ncols + 7) & ~7;
+          r.insert(r.end(), {(int64_t)lev, (int64_t)h_grp_slot0[g], (int64_t)h_grp_nn[g], (int64_t)ncp, (int64_t)B.threads,
+                             (int64_t)build_npair(ncp >> 3, B.threads / 32)});
+        }
+    };
+    for (int l = 0; l < (int)levels.size(); l++) groups(levels[l], l);
+    groups(pred_level, -1);
+    return emit(r);
   }
   if (u < 0 || u >= n_blocks) { err = "block id out of range"; return 1; }
   if (which == "parents_indexing") {  // init_indexing :325-335

@@ -89,6 +89,7 @@ struct LevelInfo {
   size_t smem_gibbs = 0;
   int gram_rch = 1, gram_ldx = 2, gram_tiles = 2, gram_stage_off = 2, gram_threads = 256;  // gram_level_kernel: staged rows per chunk, their leading dimension, doubles of the assembled tiles
   bool gram_skip = false;          // every block of the level is fused into its parent
+  int gram_maxrows = 0, gram_maxitems = 0;  // largest rows a block stages (own + fused children), largest (tile, sub-block) item count
 };
 
 struct GroupSpec { int s, nn, NT; };  // a BUILD work group: nn sibling blocks from slot s, NT tiles of 8 columns
