@@ -214,6 +214,40 @@ typedef struct {               /* caller-allocated, NULL pointers are skipped; r
 } st_pred_out;
 int st_predict_new(st_handle* h, const st_new_rows* rows, const st_pred_samples* samples, st_pred_out* out);
 
+/* ---- draws kept on the device and summarised there (no reference counterpart; DESIGN.md §5c) ----
+ * st_keep_samples_on_device: for the following st_mcmc_run calls with rng_mode = 1, keep the saved iterations' w and / or
+ * yhat in device memory, [sample][row] (one contiguous n_all vector per saved iteration, boundary order).  Host copies are
+ * still made where st_mcmc_out.w_mcmc / yhat_mcmc are not NULL, and the chain draws exactly what it draws without the store.
+ * The store (n_all x keep x 8 bytes per quantity) is checked against the free device memory before a run allocates or
+ * launches anything: ST_ERR_UNSUPPORTED, with the bytes needed and free, and the handle as it was.  It holds the last completed
+ * run, is replaced by the next one, and is freed by what = 0 or st_destroy.  ST_ERR_UNSUPPORTED: a store with rng_mode = 0,
+ * or on a partitioned handle. */
+#define ST_KEEP_W 1
+#define ST_KEEP_YHAT 2
+int st_keep_samples_on_device(st_handle* h, int32_t what);
+/* Per-row summaries of stored draws.  which: 0 = w, 1 = yhat of the last stored run (rows in boundary order); 2 = w_new,
+ * 3 = y_new of the last st_predict_new_stored with keep_draws (rows in the caller's order).  Over the S draws of a row:
+ *   mean; sd (ddof = 1, 0 for S = 1); quantiles at probs[0..n_probs) exactly as numpy.quantile(method="linear") (R type 7);
+ *   batch means with b = floor(sqrt(S)) draws per batch over the first B = floor(S / b) batches: sigma2 = b var(batch means,
+ *   ddof = 1), mcse = sqrt(sigma2 / S), ess = S var(draws, ddof = 1) / sigma2, both NaN when S < 2 or sigma2 = 0.
+ * Every reduction runs in a fixed order: repeated calls are bit-identical.  ST_ERR_INVALID: nothing stored for `which`, or a
+ * prob outside [0, 1] or NaN; ST_ERR_UNSUPPORTED: S above what one CTA can stage (the limit is in the message). */
+typedef struct {               /* caller-allocated; NULL pointers are skipped (all NULL: only the sizes are returned) */
+  double* mean;                /* n_rows */
+  double* sd;                  /* n_rows */
+  double* quantiles;           /* n_rows x n_probs */
+  double* mcse;                /* n_rows */
+  double* ess;                 /* n_rows */
+  int64_t n_rows;              /* out */
+  int32_t n_samples;           /* out */
+} st_summary_out;
+int st_summarize(st_handle* h, int32_t which, const double* probs, int32_t n_probs, st_summary_out* out);
+/* st_predict_new from every saved iteration of the last stored run (ST_KEEP_W required, else ST_ERR_INVALID): theta, beta and
+ * tausq of the run, w_s read from the device store; normals from the device (seed as st_pred_samples.seed).  The outputs are
+ * those st_predict_new gives for the same samples as host arrays.  keep_draws != 0: the w_new / y_new draws also go to a device
+ * store (n_new x S each, [sample][row], checked against the free memory like the run's) for st_summarize(which = 2, 3). */
+int st_predict_new_stored(st_handle* h, const st_new_rows* rows, uint64_t seed, int32_t keep_draws, st_pred_out* out);
+
 /* ---- the Metropolis-Hastings glue (mh_adapt.h / mh_adapt.cpp), as st_mcmc_run uses it; host-only, no handle ---- */
 /* par_huvtransf_fwd / par_huvtransf_back (Rcpp exports), mh_adapt.cpp:3-15: logit / logistic on (bounds[j], bounds[j + npar]).
  * bounds: npar x 2. */

@@ -98,6 +98,16 @@ class StPredOut(C.Structure):
     ]
 
 
+class StSummaryOut(C.Structure):
+    _fields_ = [
+        ("mean", c_double_p), ("sd", c_double_p), ("quantiles", c_double_p), ("mcse", c_double_p), ("ess", c_double_p),
+        ("n_rows", C.c_int64), ("n_samples", C.c_int32),
+    ]
+
+
+ST_KEEP_W, ST_KEEP_YHAT = 1, 2
+
+
 # every symbol include/spamtree_b200.h declares, with its signature
 SIGNATURES = {
     "st_version": (C.c_char_p, []),
@@ -121,6 +131,9 @@ SIGNATURES = {
     "st_get_index": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.c_int, c_int64_p, C.c_int64, c_int64_p]),
     "st_mcmc_run": (C.c_int, [C.c_void_p, C.POINTER(StMcmcOpts), C.POINTER(StMcmcOut)]),
     "st_predict_new": (C.c_int, [C.c_void_p, C.POINTER(StNewRows), C.POINTER(StPredSamples), C.POINTER(StPredOut)]),
+    "st_keep_samples_on_device": (C.c_int, [C.c_void_p, C.c_int32]),
+    "st_summarize": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, C.c_int32, C.POINTER(StSummaryOut)]),
+    "st_predict_new_stored": (C.c_int, [C.c_void_p, C.POINTER(StNewRows), C.c_uint64, C.c_int32, C.POINTER(StPredOut)]),
     "st_bench_iteration": (C.c_int, [C.c_void_p, c_double_p, C.c_int, C.c_uint64, c_double_p, c_float_p]),
     "st_set_beta_index": (C.c_int, [C.c_void_p, C.c_int]),
     "st_get_counters": (C.c_int, [C.c_void_p, c_double_p]),

@@ -234,6 +234,27 @@ int st_predict_new(st_handle* h, const st_new_rows* rows, const st_pred_samples*
   ST_GUARD_BEGIN return h->model.predict_new(*rows, *samples, *out);
   ST_GUARD_END(h)
 }
+int st_keep_samples_on_device(st_handle* h, int32_t what) {
+  if (!h) return ST_ERR_INVALID;
+  activate(h);
+  ST_GUARD_BEGIN return h->model.keep_samples_on_device(what);
+  ST_GUARD_END(h)
+}
+int st_summarize(st_handle* h, int32_t which, const double* probs, int32_t n_probs, st_summary_out* out) {
+  if (!h || !out) return ST_ERR_INVALID;
+  activate(h);
+  ST_GUARD_BEGIN return h->model.summarize(which, probs, n_probs, *out);
+  ST_GUARD_END(h)
+}
+int st_predict_new_stored(st_handle* h, const st_new_rows* rows, uint64_t seed, int32_t keep_draws, st_pred_out* out) {
+  if (!h || !rows || !out) return ST_ERR_INVALID;
+  activate(h);
+  ST_GUARD_BEGIN
+  st_pred_samples ps{};
+  ps.seed = seed;
+  return h->model.predict_new(*rows, ps, *out, true, keep_draws != 0);
+  ST_GUARD_END(h)
+}
 int st_bench_iteration(st_handle* h, const double* theta_prop, int do_swap, uint64_t seed, double* out3, float* ms_out) {
   if (!h || !theta_prop || !out3) return ST_ERR_INVALID;
   activate(h);

@@ -1180,4 +1180,150 @@ cudaError_t launch_predict_moments(long long n, int S, const double* acc, double
   return cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------ summaries of stored draws
+// Doubles as 64-bit keys whose unsigned order is the numeric order (negative: all bits flipped; otherwise: sign bit set)
+__device__ __forceinline__ unsigned long long summary_key(double x) {
+  const unsigned long long u = (unsigned long long)__double_as_longlong(x);
+  return (u >> 63) ? ~u : (u | 0x8000000000000000ULL);
+}
+__device__ __forceinline__ double summary_val(unsigned long long k) {
+  return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffULL) : ~k));
+}
+
+// sum over the G threads of each row group (threads [r G, (r + 1) G)), pairwise in a fixed order; every thread gets its
+// group's total.  red: blockDim.x doubles.  Called by every thread of the CTA.
+__device__ __forceinline__ double summary_group_sum(double v, double* red, int G) {
+  const int t = threadIdx.x, lane = t % G;
+  red[t] = v;
+  __syncthreads();
+  for (int s = G >> 1; s > 0; s >>= 1) {
+    if (lane < s) red[t] += red[t + s];
+    __syncthreads();
+  }
+  const double total = red[t - lane];
+  __syncthreads();
+  return total;
+}
+
+// One CTA per tile of R rows of a [sample][row] store (element (s, i) at src[s * n + i]).  The tile's S x R values are read
+// once with coalesced loads (consecutive threads, consecutive rows), staged as order-preserving keys (row-major: key[r S + s]),
+// and every statistic is formed from the staged copy: the moments and batch means in sample order, then the quantiles after a
+// bitonic sort of each row in shared memory.  The sort is the all-ascending form of the network (a "flip" stage then
+// half-cleaners), so positions >= S act as +inf and are never touched: no padding is staged.  Every reduction is over G = T / R
+// threads per row in a fixed order.  Outputs: mean, sd (ddof 1), quant (n x np, column-major), mcse, ess (batch means).
+__global__ void __launch_bounds__(kSummaryThreads)
+summary_kernel(const double* __restrict__ src, long long n, int S, int R, const double* __restrict__ probs, int np,
+               double* __restrict__ mean_out, double* __restrict__ sd_out, double* __restrict__ quant, double* __restrict__ mcse_out,
+               double* __restrict__ ess_out) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double* red = reinterpret_cast<double*>(smem_raw);                                 // T doubles
+  unsigned long long* key = reinterpret_cast<unsigned long long*>(red + blockDim.x);  // R x S keys
+  const int T = blockDim.x, t = threadIdx.x, G = T / R, r = t / G, lane = t % G;
+  const long long row0 = (long long)blockIdx.x * R;
+  const int nr = (int)min((long long)R, n - row0);
+  // ---- stage: element e of the tile is (sample e / R, row e % R)
+  const long long tot = (long long)S * R;
+  for (long long e = t; e < tot; e += T) {
+    const int s = (int)(e / R), rr = (int)(e % R);
+    key[(long long)rr * S + s] = rr < nr ? summary_key(src[(long long)s * n + row0 + rr]) : 0ULL;
+  }
+  __syncthreads();
+  const unsigned long long* kr = key + (long long)r * S;
+  // ---- mean and sd (two passes over the staged row, in sample order per thread)
+  double acc = 0.0;
+  for (int s = lane; s < S; s += G) acc += summary_val(kr[s]);
+  const double mean = summary_group_sum(acc, red, G) / S;
+  acc = 0.0;
+  for (int s = lane; s < S; s += G) { const double dv = summary_val(kr[s]) - mean; acc += dv * dv; }
+  const double ss = summary_group_sum(acc, red, G);
+  const double var = S > 1 ? ss / (S - 1) : 0.0;
+  // ---- batch means: b = floor(sqrt(S)) draws per batch, B = floor(S / b) batches over the first B b draws
+  int b = (int)sqrt((double)S);
+  while ((long long)(b + 1) * (b + 1) <= S) b++;
+  while (b > 1 && (long long)b * b > S) b--;
+  const int B = S / b;
+  acc = 0.0;
+  for (int k = lane; k < B; k += G) {
+    double bs = 0.0;
+    for (int s = k * b; s < k * b + b; s++) bs += summary_val(kr[s]);
+    acc += bs / b;
+  }
+  const double bmean = summary_group_sum(acc, red, G) / B;
+  acc = 0.0;
+  for (int k = lane; k < B; k += G) {
+    double bs = 0.0;
+    for (int s = k * b; s < k * b + b; s++) bs += summary_val(kr[s]);
+    const double dv = bs / b - bmean;
+    acc += dv * dv;
+  }
+  const double bss = summary_group_sum(acc, red, G);
+  if (lane == 0 && r < nr) {
+    const long long i = row0 + r;
+    const double sig2 = B > 1 ? (double)b * (bss / (B - 1)) : 0.0;
+    const bool ok = S >= 2 && sig2 > 0.0;
+    mean_out[i] = mean;
+    sd_out[i] = sqrt(var);
+    mcse_out[i] = ok ? sqrt(sig2 / S) : __longlong_as_double(0x7ff8000000000000LL);
+    ess_out[i] = ok ? (double)S * var / sig2 : __longlong_as_double(0x7ff8000000000000LL);
+  }
+  if (np == 0) return;
+  // ---- sort every row of the tile: all ascending, pairs (i, j > i), j >= S skipped
+  int P2 = 1;
+  while (P2 < S) P2 <<= 1;
+  const int half = P2 >> 1;
+  const long long pairs = (long long)R * half;
+  for (int k = 2; k <= P2; k <<= 1) {
+    for (int d = k >> 1; d > 0; d >>= 1) {
+      const bool flip = d == (k >> 1);
+      for (long long e = t; e < pairs; e += T) {
+        const int rr = (int)(e / half), pp = (int)(e % half);
+        const int i = (pp / d) * 2 * d + pp % d;
+        const int j = flip ? (i ^ (k - 1)) : i + d;
+        if (j < S) {
+          unsigned long long* kk = key + (long long)rr * S;
+          const unsigned long long a = kk[i], c = kk[j];
+          if (a > c) { kk[i] = c; kk[j] = a; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  // ---- quantiles: numpy's method "linear" (R type 7) with its virtual-index and _lerp formulas, without contraction
+  for (int e = t; e < R * np; e += T) {
+    const int rr = e / np, jp = e % np;
+    if (rr >= nr) continue;
+    const unsigned long long* kk = key + (long long)rr * S;
+    const double vi = __dmul_rn((double)(S - 1), probs[jp]);
+    double res;
+    if (vi >= (double)(S - 1)) {
+      res = summary_val(kk[S - 1]);
+    } else {
+      const int lo = (int)floor(vi);
+      const double g = __dsub_rn(vi, (double)lo);
+      const double a = summary_val(kk[lo]), c = summary_val(kk[lo + 1]);
+      const double diff = __dsub_rn(c, a);
+      res = g >= 0.5 ? __dsub_rn(c, __dmul_rn(diff, __dsub_rn(1.0, g))) : __dadd_rn(a, __dmul_rn(diff, g));
+    }
+    quant[row0 + rr + (long long)jp * n] = res;
+  }
+}
+int summary_rows_per_cta(int S, size_t smem_cap) {
+  if (S < 1) return 0;
+  const size_t avail = smem_cap - (size_t)kSummaryThreads * sizeof(double);
+  int R = kSummaryMaxRows;
+  while (R >= 1 && (size_t)R * S * sizeof(unsigned long long) > avail) R >>= 1;
+  return R;
+}
+size_t summary_smem_bytes(int S, int R) { return (size_t)kSummaryThreads * sizeof(double) + (size_t)R * S * sizeof(unsigned long long); }
+cudaError_t launch_summary(const double* src, long long n, int S, int R, const double* probs, int np, double* mean, double* sd, double* quant,
+                           double* mcse, double* ess, cudaStream_t st) {
+  if (n <= 0 || S <= 0) return cudaSuccess;
+  static SmemOptIn opt;
+  const size_t smem = summary_smem_bytes(S, R);
+  cudaError_t e = ensure_dynamic_smem(summary_kernel, smem, opt);
+  if (e != cudaSuccess) return e;
+  summary_kernel<<<(unsigned)((n + R - 1) / R), kSummaryThreads, smem, st>>>(src, n, S, R, probs, np, mean, sd, quant, mcse, ess);
+  return cudaGetLastError();
+}
+
 }  // namespace st

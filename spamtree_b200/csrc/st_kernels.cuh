@@ -124,5 +124,16 @@ cudaError_t launch_predict_draw(long long n, const long long* lay2row, const int
                                 double* wout, double* yout, double* mout, double* sdout, double* acc, cudaStream_t st);
 // out4 = {mean w, sd w, mean y, sd y} (n each) from acc after S samples
 cudaError_t launch_predict_moments(long long n, int S, const double* acc, double* out4, cudaStream_t st);
+// ---- per-row summaries of a [sample][row] store of S draws of n rows (st_summarize; DESIGN.md §5c)
+constexpr int kSummaryThreads = 512;
+constexpr int kSummaryMaxRows = 32;   // rows one CTA stages at most (the tile shape at small S)
+// rows per CTA for S draws in smem_cap bytes of shared memory: the largest power of two <= kSummaryMaxRows whose keys fit;
+// 0 when not even one row fits
+int summary_rows_per_cta(int S, size_t smem_cap);
+size_t summary_smem_bytes(int S, int R);
+// mean, sd (ddof 1), quant (n x np, column-major; numpy's "linear" quantiles of probs[np], a device array), mcse and ess
+// (batch means); every output a device array of n (quant: n np)
+cudaError_t launch_summary(const double* src, long long n, int S, int R, const double* probs, int np, double* mean, double* sd, double* quant,
+                           double* mcse, double* ess, cudaStream_t st);
 
 }  // namespace st

@@ -28,6 +28,10 @@ int mcmc_run(Model& M, const st_mcmc_opts& o, st_mcmc_out& out) {
   // rng_mode 1: the device-resident chain — proposal, accept decision, RAM adaptation, tausq / beta draws and yhat on the
   // device, no host round trip per iteration (st_model.cu: Model::chain_run)
   if (o.rng_mode == 1) return M.chain_run(o, out);
+  if (M.keep_mask) {
+    M.err = "st_mcmc_run: the device sample store (st_keep_samples_on_device) needs the device-resident chain (rng_mode = 1)";
+    return ST_ERR_UNSUPPORTED;
+  }
   // rng_mode 0: every draw from one host stream, in the reference's order (lock-step with the oracle and with the
   // reference's own driver); a partitioned run draws for every row of the whole problem on every rank and keeps its own
   if (M.part && M.global_rows.empty()) {

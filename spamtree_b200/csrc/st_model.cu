@@ -81,6 +81,7 @@ Model::~Model() {
   cudaSetDevice(device);
   if (nccl_comm) { cudaStreamSynchronize(stream); nccl().CommDestroy(nccl_comm); nccl_comm = nullptr; }
   for (void* p : owned) cudaFree(p);
+  for (SampleStore& s : store_) s.release();
   if (h_scalars) cudaFreeHost(h_scalars);
   if (h_mc) cudaFreeHost(h_mc);
   for (void* g : graph_exec_) if (g) cudaGraphExecDestroy((cudaGraphExec_t)g);
@@ -1276,14 +1277,22 @@ int Model::save_begin(double* host_base, size_t bytes) {
   return 0;
 }
 
-int Model::save_w_async(double* host_dst) {
-  if (!save_registered) return get_w(host_dst);
-  if (save_pending) ST_CUDA(cudaStreamWaitEvent(stream, ev_wcopied, 0), "wait for the previous save");  // d_wsave is reused
-  ST_CUDA(launch_permute(d_w, d_wsave, d_iperm, n_all, stream), "permute_kernel");
+int Model::save_w_async(double* host_dst, double* dev_dst) {
+  if (!dev_dst && !save_registered) return get_w(host_dst);
+  // (a slot of the device store is written once: only the shared staging buffer waits for the copy before it)
+  if (!dev_dst && save_pending) ST_CUDA(cudaStreamWaitEvent(stream, ev_wcopied, 0), "wait for the previous save");  // d_wsave is reused
+  double* buf = dev_dst ? dev_dst : d_wsave;
+  ST_CUDA(launch_permute(d_w, buf, d_iperm, n_all, stream), "permute_kernel");
   n_launches++;
+  if (!host_dst) return 0;
+  if (!save_registered) {
+    ST_CUDA(cudaMemcpyAsync(host_dst, buf, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H w");
+    ST_CUDA(cudaStreamSynchronize(stream), "sync");
+    return 0;
+  }
   ST_CUDA(cudaEventRecord(ev_wready, stream), "event");
   ST_CUDA(cudaStreamWaitEvent(copy_stream, ev_wready, 0), "wait");
-  ST_CUDA(cudaMemcpyAsync(host_dst, d_wsave, n_all * sizeof(double), cudaMemcpyDeviceToHost, copy_stream), "D2H w (async)");
+  ST_CUDA(cudaMemcpyAsync(host_dst, buf, n_all * sizeof(double), cudaMemcpyDeviceToHost, copy_stream), "D2H w (async)");
   ST_CUDA(cudaEventRecord(ev_wcopied, copy_stream), "event");
   save_pending = true;
   return 0;
@@ -1820,11 +1829,12 @@ int Model::bench_iteration(const double* theta_prop, int do_swap, uint64_t seed,
   return 0;
 }
 
-// S.dbuf (n_all doubles, boundary order, written by the kernel just enqueued on `stream`) -> host_dst on the copy stream
-int Model::save_rows_async(AsyncSave& S, double* host_dst) {
+// src (n_all doubles, boundary order, written by the kernel just enqueued on `stream`: S.dbuf or a slot of the device store)
+// -> host_dst on the copy stream
+int Model::save_rows_async(AsyncSave& S, double* host_dst, const double* src) {
   ST_CUDA(cudaEventRecord(S.ready, stream), "event");
   ST_CUDA(cudaStreamWaitEvent(copy_stream, S.ready, 0), "wait");
-  ST_CUDA(cudaMemcpyAsync(host_dst, S.dbuf, n_all * sizeof(double), cudaMemcpyDeviceToHost, copy_stream), "D2H rows (async)");
+  ST_CUDA(cudaMemcpyAsync(host_dst, src, n_all * sizeof(double), cudaMemcpyDeviceToHost, copy_stream), "D2H rows (async)");
   ST_CUDA(cudaEventRecord(S.copied, copy_stream), "event");
   S.pending = true;
   return 0;
@@ -1840,6 +1850,26 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
     err = "partitioned runs support only the corrected beta row index (faithful_index = 0): the reference's mis-indexing "
           "(SURVEY App. D #12) mixes rows that live on different ranks";
     return 4;
+  }
+  // the device sample store (st_keep_samples_on_device): sized and checked before anything is allocated or launched, so that a
+  // refused run leaves the handle as it was; a run replaces the last run's store
+  const bool store_w = (keep_mask & ST_KEEP_W) != 0, store_y = (keep_mask & ST_KEEP_YHAT) != 0;
+  if (keep_mask) {
+    if (part) { err = "st_mcmc_run: the device sample store is not supported on partitioned handles"; return 4; }
+    const size_t per = (size_t)n_all * (size_t)std::max(o.keep, 0) * sizeof(double);
+    int rc = check_store_fits((store_w ? per : 0) + (store_y ? per : 0), store_[0].cap + store_[1].cap, "st_mcmc_run");
+    if (rc) return rc;
+    store_samp_.clear();
+    for (int k = 0; k < 2; k++) {
+      SampleStore& s = store_[k];
+      if (!(keep_mask & (1 << k))) { s.release(); continue; }
+      if (s.reserve(std::max<size_t>(per, 8)) != cudaSuccess) {
+        (void)cudaGetLastError();
+        s.release();
+        err = "st_mcmc_run: allocating " + std::to_string(per) + " bytes for the device sample store failed";
+        return 4;
+      }
+    }
   }
   double o3[3];
   int rc = get_loglik_comps_w(0, o3);  // spamtree_fit.cpp:110-111
@@ -1865,7 +1895,10 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   if (rc) return rc;
   // saved rows: w through the existing staging (un-permute kernel), yhat through its own
   const bool save_w = out.w_mcmc != nullptr, save_y = out.yhat_mcmc != nullptr;
-  if (save_w || save_y) { rc = save_begin(save_w ? out.w_mcmc : nullptr, (size_t)keep * n_all * sizeof(double)); if (rc) return rc; }
+  if (save_w || save_y || store_w || store_y) {
+    rc = save_begin(save_w ? out.w_mcmc : nullptr, (size_t)keep * n_all * sizeof(double));
+    if (rc) return rc;
+  }
   if (save_y) {
     if (!save_y_.dbuf) {
       ST_CUDA(dev_zeros(save_y_.dbuf, n_all, owned), "alloc yhat");
@@ -1929,14 +1962,18 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
     }
     if (!launched) { rc = enqueue_iteration(o, predicting, 0, first, !last, saved ? keep : 0); if (rc) return rc; }
     if (saved) {  // :376-389
-      if (save_w) { rc = save_w_async(out.w_mcmc + (size_t)msaved * n_all); if (rc) return rc; }
-      if (save_y) {
-        if (save_y_.pending) ST_CUDA(cudaStreamWaitEvent(stream, save_y_.copied, 0), "wait for the previous save");
-        ST_CUDA(launch_yhat(dt, d_w, d_xb, d_tausq_inv, d_iperm, d_rowkey, n_all, d_mc, save_y_.dbuf, stream), "yhat_kernel");
+      if (save_w || store_w) {
+        rc = save_w_async(save_w ? out.w_mcmc + (size_t)msaved * n_all : nullptr, store_w ? store_[0].d + (size_t)msaved * n_all : nullptr);
+        if (rc) return rc;
+      }
+      if (save_y || store_y) {
+        double* ybuf = store_y ? store_[1].d + (size_t)msaved * n_all : save_y_.dbuf;
+        if (!store_y && save_y_.pending) ST_CUDA(cudaStreamWaitEvent(stream, save_y_.copied, 0), "wait for the previous save");
+        ST_CUDA(launch_yhat(dt, d_w, d_xb, d_tausq_inv, d_iperm, d_rowkey, n_all, d_mc, ybuf, stream), "yhat_kernel");
         n_launches++;
-        if (save_y_.registered) { rc = save_rows_async(save_y_, out.yhat_mcmc + (size_t)msaved * n_all); if (rc) return rc; }
-        else {
-          ST_CUDA(cudaMemcpyAsync(out.yhat_mcmc + (size_t)msaved * n_all, save_y_.dbuf, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H yhat");
+        if (save_y && save_y_.registered) { rc = save_rows_async(save_y_, out.yhat_mcmc + (size_t)msaved * n_all, ybuf); if (rc) return rc; }
+        else if (save_y) {
+          ST_CUDA(cudaMemcpyAsync(out.yhat_mcmc + (size_t)msaved * n_all, ybuf, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H yhat");
           ST_CUDA(cudaStreamSynchronize(stream), "sync");
         }
       }
@@ -1960,6 +1997,80 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   out.n_chol_fail = h_mc->n_chol_fail;
   if (h_mc->gibbs_fail) { err = "Error at gibbs_sample_w: conditional precision not positive definite"; return 3; }
   if (h_mc->nan_loglik) { err = "At nan loglik: error."; return 5; }
+  if (keep_mask && keep > 0) {  // the run completed: its store and the samples st_predict_new_stored predicts from
+    for (int k = 0; k < 2; k++)
+      if (keep_mask & (1 << k)) { store_[k].n = n_all; store_[k].S = keep; }
+    store_samp_.assign(hs.begin(), hs.begin() + (n_th + n_be + n_ta));
+  }
+  return 0;
+}
+
+int Model::check_store_fits(size_t need, size_t reusable, const char* what) {
+  size_t fr = 0, tot = 0;
+  ST_CUDA(cudaMemGetInfo(&fr, &tot), "cudaMemGetInfo");
+  if (need > fr + reusable) {
+    err = std::string(what) + ": the device sample store needs " + std::to_string(need) + " bytes and " + std::to_string(fr + reusable) +
+          " bytes of device memory are free";
+    return 4;
+  }
+  return 0;
+}
+
+int Model::keep_samples_on_device(int what) {
+  if (what < 0 || what > (ST_KEEP_W | ST_KEEP_YHAT)) { err = "st_keep_samples_on_device: what must be a mask of ST_KEEP_W | ST_KEEP_YHAT"; return 1; }
+  if (what && !stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
+  if (what && part) { err = "st_keep_samples_on_device: partitioned handles are not supported"; return 4; }
+  keep_mask = what;
+  if (what == 0) {
+    if (stream) cudaStreamSynchronize(stream);
+    for (SampleStore& s : store_) s.release();
+    store_samp_.clear();
+  }
+  return 0;
+}
+
+int Model::summarize(int which, const double* probs, int n_probs, st_summary_out& out) {
+  static const char* names[4] = {"w", "yhat", "w_new", "y_new"};
+  if (which < 0 || which > 3) { err = "st_summarize: which must be 0 (w), 1 (yhat), 2 (w_new) or 3 (y_new)"; return 1; }
+  const SampleStore& s = store_[which];
+  out.n_rows = 0;
+  out.n_samples = 0;
+  if (!s.d || s.S < 1) {
+    err = std::string("st_summarize: no stored draws of ") + names[which] +
+          (which < 2 ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)" : " (st_predict_new_stored with keep_draws)");
+    return 1;
+  }
+  if (n_probs < 0 || (n_probs > 0 && !probs)) { err = "st_summarize: n_probs < 0, or probs missing"; return 1; }
+  for (int j = 0; j < n_probs; j++)
+    if (!(probs[j] >= 0.0 && probs[j] <= 1.0)) { err = "st_summarize: every prob must lie in [0, 1] (NaN is refused)"; return 1; }
+  const size_t cap = 227 * 1024;
+  const int R = summary_rows_per_cta(s.S, cap);
+  if (R < 1) {
+    err = "st_summarize: " + std::to_string(s.S) + " draws per row exceed what one CTA stages in shared memory (at most " +
+          std::to_string((cap - (size_t)kSummaryThreads * sizeof(double)) / sizeof(unsigned long long)) + ")";
+    return 4;
+  }
+  out.n_rows = s.n;
+  out.n_samples = s.S;
+  double* hdst[5] = {out.mean, out.sd, out.quantiles, out.mcse, out.ess};
+  if (!(hdst[0] || hdst[1] || hdst[2] || hdst[3] || hdst[4]) || s.n == 0) return 0;
+  // one device buffer: mean | sd | mcse | ess | quantiles (n x n_probs) | probs
+  const size_t n = (size_t)s.n, nd = (4 + (size_t)n_probs) * n + (size_t)n_probs;
+  double* d = nullptr;
+  ST_CUDA(cudaMalloc((void**)&d, nd * sizeof(double)), "alloc summaries");
+  struct Free { double* p; ~Free() { cudaFree(p); } } fr{d};
+  struct StreamSync { cudaStream_t s; ~StreamSync() { cudaStreamSynchronize(s); } } ssync{stream};
+  double* dq = d + 4 * n;
+  double* dp = dq + (size_t)n_probs * n;
+  if (n_probs) ST_CUDA(cudaMemcpyAsync(dp, probs, n_probs * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D probs");
+  ST_CUDA(launch_summary(s.d, s.n, s.S, R, dp, n_probs, d, d + n, dq, d + 2 * n, d + 3 * n, stream), "summary_kernel");
+  n_launches++;
+  const double* dsrc[5] = {d, d + n, dq, d + 2 * n, d + 3 * n};
+  for (int c = 0; c < 5; c++) {
+    const size_t cnt = c == 2 ? (size_t)n_probs * n : n;
+    if (hdst[c] && cnt) ST_CUDA(cudaMemcpyAsync(hdst[c], dsrc[c], cnt * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H summaries");
+  }
+  ST_CUDA(cudaStreamSynchronize(stream), "sync");
   return 0;
 }
 
@@ -1970,14 +2081,44 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
 // work group (they are conditionally independent, so any split is exact), appended to temporary copies of the per-node and
 // per-row arrays.  Per sample: BUILD of the reference levels into the alter slot when theta changed, w_s into node order,
 // build_level_kernel<3> (forward sweep only: mean and sd per row), predict_draw_kernel; the draws leave on a copy stream.
-int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_out& out) {
+// from_store: the samples are the last stored run's (theta / beta / tausq from its host copy, w_s gathered straight from the
+// device store); keep_draws: w_new / y_new are written into the prediction's device store instead of scratch.
+int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pred_out& out, bool from_store, bool keep_draws) {
   if (!stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
   if (part) { err = "predict_new: partitioned handles are not supported"; return 4; }
   out.n_builds = 0;
+  const int npar = (int)theta[0].size();
+  st_pred_samples PS = PS_in;
+  if (from_store) {
+    const int Ss = store_[0].S;
+    if (!store_[0].d || Ss < 1 || store_samp_.empty()) {
+      err = "st_predict_new_stored: the last device-resident run kept no w on the device (st_keep_samples_on_device with ST_KEEP_W)";
+      return 1;
+    }
+    PS.n_samples = Ss;
+    PS.theta = store_samp_.data();
+    PS.beta = PS.theta + (size_t)npar * Ss;
+    PS.tausq = PS.beta + (size_t)p * Ss * q;
+    PS.w = store_[0].d;  // (a device pointer: read by gather_sample_kernel only)
+    PS.w_row_stride = 1;
+    PS.w_sample_stride = n_all;
+    PS.z = PS.eps = nullptr;
+  }
   const int64_t nn = R.n_new;
   const int S = PS.n_samples;
-  const int npar = (int)theta[0].size();
   if (nn < 0 || S < 0) { err = "predict_new: negative n_new or n_samples"; return 1; }
+  if (keep_draws) {  // checked before anything is allocated; the previous prediction's store is replaced
+    const size_t per = (size_t)std::max<int64_t>(nn, 0) * S * sizeof(double);
+    const int rc = check_store_fits(2 * per, store_[2].cap + store_[3].cap, "st_predict_new_stored");
+    if (rc) return rc;
+    for (int k = 2; k < 4; k++)
+      if (store_[k].reserve(std::max<size_t>(per, 8)) != cudaSuccess) {
+        (void)cudaGetLastError();
+        store_[k].release();
+        err = "st_predict_new_stored: allocating " + std::to_string(per) + " bytes for the device draw store failed";
+        return 4;
+      }
+  }
   if (nn == 0 || S == 0) return 0;
   if (!R.coords || !R.mv_id || !R.group || !R.parents_ptr || R.n_groups < 1 || !PS.theta || !PS.beta || !PS.tausq || !PS.w) {
     err = "predict_new: a required input is missing";
@@ -2146,9 +2287,10 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_
     ST_CUDA(cudaMemcpyAsync(d_Xn, R.X, (size_t)nn * p * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D X_new");
   }
   // samples of w staged in blocks of B (one 2D copy each), the node-ordered w_s, mean / sd, normals, two output slots
-  const int B = (int)std::max<int64_t>(1, std::min<int64_t>(S, (256LL << 20) / (8 * n_all)));
-  double *d_wblk, *d_wnode, *d_mean, *d_sd, *d_acc, *d_zn = nullptr, *d_en = nullptr;
-  ST_CUDA(dalloc((void**)&d_wblk, (size_t)B * n_all * sizeof(double)), "alloc");
+  // (from the store: every sample is already on the device, one block of S)
+  const int B = from_store ? S : (int)std::max<int64_t>(1, std::min<int64_t>(S, (256LL << 20) / (8 * n_all)));
+  double *d_wblk = nullptr, *d_wnode, *d_mean, *d_sd, *d_acc, *d_zn = nullptr, *d_en = nullptr;
+  if (!from_store) ST_CUDA(dalloc((void**)&d_wblk, (size_t)B * n_all * sizeof(double)), "alloc");
   ST_CUDA(dalloc((void**)&d_wnode, n_all * sizeof(double)), "alloc");
   ST_CUDA(dalloc((void**)&d_mean, nn * sizeof(double)), "alloc");
   ST_CUDA(dalloc((void**)&d_sd, nn * sizeof(double)), "alloc");
@@ -2180,9 +2322,10 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_
   int* d_bfail;                  // failed factorisations of each BUILD
   ST_CUDA(dalloc((void**)&d_bfail, (size_t)S * sizeof(int)), "alloc");
   const int alt = phys(1);
-  int si = 0, sb = 0;
+  int si = 1, sb = (int)n_all;
+  const double* wsrc = from_store ? store_[0].d : d_wblk;
   for (int j = 0; j < S; j++) {
-    if (j % B == 0) {
+    if (!from_store && j % B == 0) {
       const int nb = std::min(B, S - j);
       if (rmaj) {
         ST_CUDA(cudaMemcpy2DAsync(d_wblk, nb * sizeof(double), PS.w + j, PS.w_row_stride * sizeof(double), nb * sizeof(double), n_all,
@@ -2213,7 +2356,7 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_
       out.n_builds++;
     }
     build_of[j] = (int)out.n_builds - 1;
-    ST_CUDA(launch_gather_sample(d_wblk, si, sb, j % B, d_perm, d_wnode, n_all, stream), "gather_sample_kernel");
+    ST_CUDA(launch_gather_sample(wsrc, si, sb, j % B, d_perm, d_wnode, n_all, stream), "gather_sample_kernel");
     for (const LevelInfo::BuildLaunch& L : launches)
       ST_CUDA(launch_build(3, T2, dslots, 1, d_mean, d_sd, 0, d_gslot0 + L.grp0, d_gnn + L.grp0, L.ngrp, d_wnode, d_fail + 2, L.ns, 0,
                            L.smem, stream, L.threads),
@@ -2227,15 +2370,17 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_
       for (int a = 0; a < p; a++) pack.beta[a + jq * p] = PS.beta[a + (size_t)j * p + (size_t)jq * p * S];
       pack.sdtau[jq] = std::sqrt(PS.tausq[jq + (size_t)j * q]);
     }
-    ST_CUDA(launch_predict_draw(nn, d_lay2row, d_cmvq, d_Xn, p, d_mean, d_sd, pack, PS.seed, j, d_zn, d_en, d_out[r][0], d_out[r][1],
-                                d_out[r][2], d_out[r][3], d_acc, stream),
+    double* dsrc[4] = {keep_draws ? store_[2].d + (size_t)j * nn : d_out[r][0], keep_draws ? store_[3].d + (size_t)j * nn : d_out[r][1],
+                       d_out[r][2], d_out[r][3]};
+    ST_CUDA(launch_predict_draw(nn, d_lay2row, d_cmvq, d_Xn, p, d_mean, d_sd, pack, PS.seed, j, d_zn, d_en, dsrc[0], dsrc[1],
+                                dsrc[2], dsrc[3], d_acc, stream),
             "predict_draw_kernel");
     n_launches += 2 + (double)launches.size();
     if (any_draw_out) {
       ST_CUDA(cudaEventRecord(ready[r], stream), "event");
       ST_CUDA(cudaStreamWaitEvent(X.cs, ready[r], 0), "wait");
       for (int c = 0; c < 4; c++)
-        if (hout[c]) ST_CUDA(cudaMemcpyAsync(hout[c] + (size_t)j * nn, d_out[r][c], nn * sizeof(double), cudaMemcpyDeviceToHost, X.cs), "D2H draws");
+        if (hout[c]) ST_CUDA(cudaMemcpyAsync(hout[c] + (size_t)j * nn, dsrc[c], nn * sizeof(double), cudaMemcpyDeviceToHost, X.cs), "D2H draws");
       ST_CUDA(cudaEventRecord(copied[r], X.cs), "event");
       pending[r] = true;
     }
@@ -2243,7 +2388,7 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_
   double* hm[4] = {out.w_mean, out.w_sd, out.y_mean, out.y_sd};
   if (hm[0] || hm[1] || hm[2] || hm[3]) {
     double* d_mom = d_wblk;  // (free once the last gather has run: 4 nn doubles fit when nn <= B n_all / 4, else its own)
-    if (4 * nn > (int64_t)B * n_all) ST_CUDA(dalloc((void**)&d_mom, 4 * nn * sizeof(double)), "alloc");
+    if (!d_wblk || 4 * nn > (int64_t)B * n_all) ST_CUDA(dalloc((void**)&d_mom, 4 * nn * sizeof(double)), "alloc");
     ST_CUDA(launch_predict_moments(nn, S, d_acc, d_mom, stream), "predict_moments_kernel");
     for (int c = 0; c < 4; c++)
       if (hm[c]) ST_CUDA(cudaMemcpyAsync(hm[c], d_mom + (size_t)c * nn, nn * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H moments");
@@ -2260,6 +2405,8 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS, st_pred_
       err = "predict_new: theta of sample " + std::to_string(j) + ": a reference-level Cholesky factorisation failed (covariance not positive definite)";
       return 3;
     }
+  if (keep_draws)
+    for (int k = 2; k < 4; k++) { store_[k].n = nn; store_[k].S = S; }
   return 0;
 }
 

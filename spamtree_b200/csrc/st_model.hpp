@@ -231,7 +231,7 @@ class Model {
   // stream, so that the copy overlaps the next iteration; save_end waits for the copies in flight
   int save_begin(double* host_base, size_t bytes);
   int save_sync();  // waits for the copies in flight (every saved w is on the host); save_end also releases the page lock
-  int save_w_async(double* host_dst);
+  int save_w_async(double* host_dst, double* dev_dst = nullptr);  // dev_dst: a slot of the device store (then host_dst may be NULL)
   int save_end();
   int set_w(const double* in);
   int get_xb(double* out);
@@ -243,8 +243,32 @@ class Model {
   int set_widx_mode(bool faithful_index);
   // ---- the device-resident chain (rng_mode 1): spamtree_fit.cpp:167-391 without a host round trip per iteration
   int chain_run(const st_mcmc_opts& o, st_mcmc_out& out);
-  // ---- prediction at new rows from saved samples (include/spamtree_b200.h: st_predict_new)
-  int predict_new(const st_new_rows& rows, const st_pred_samples& ps, st_pred_out& out);
+  // ---- prediction at new rows from saved samples (include/spamtree_b200.h: st_predict_new); from_store: the samples are
+  // the last stored run's (st_predict_new_stored: ps carries only the seed), keep_draws: the draws go to the device store too
+  int predict_new(const st_new_rows& rows, const st_pred_samples& ps, st_pred_out& out, bool from_store = false,
+                  bool keep_draws = false);
+  // ---- device sample store (st_keep_samples_on_device, st_summarize; DESIGN.md §5c)
+  int keep_samples_on_device(int what);
+  int summarize(int which, const double* probs, int n_probs, st_summary_out& out);
+  int keep_mask = 0;                   // ST_KEEP_W | ST_KEEP_YHAT for the following device-resident runs
+  struct SampleStore {                 // [sample][row] draws of one quantity, n rows x S samples
+    double* d = nullptr;
+    size_t cap = 0;                    // bytes allocated (reused by the next run when large enough)
+    int64_t n = 0;
+    int S = 0;                         // 0: holds nothing
+    void release() { if (d) cudaFree(d); d = nullptr; cap = 0; n = 0; S = 0; }
+    cudaError_t reserve(size_t bytes) {
+      S = 0;
+      if (bytes <= cap) return cudaSuccess;
+      release();
+      const cudaError_t e = cudaMalloc((void**)&d, bytes);
+      if (e == cudaSuccess) cap = bytes; else d = nullptr;
+      return e;
+    }
+  };
+  SampleStore store_[4];               // w, yhat of the last run; w_new, y_new of the last stored prediction
+  dvec store_samp_;                    // theta (npar x S), beta (p x S x q), tausq (q x S) of the last stored run
+  int check_store_fits(size_t need, size_t reusable, const char* what);
 
  private:
   int phys(int slot) const { return slot ? 1 - cur : cur; }
@@ -272,7 +296,7 @@ class Model {
     bool pending = false;
   };
   AsyncSave save_y_;
-  int save_rows_async(AsyncSave& S, double* host_dst);
+  int save_rows_async(AsyncSave& S, double* host_dst, const double* src);
   bool deferred_[2] = {false, false};
   int refresh_grams(const int* run_flag = nullptr, cudaStream_t st = nullptr);
   int gibbs_launch_only(int* fail_ptr);
