@@ -248,6 +248,47 @@ int st_summarize(st_handle* h, int32_t which, const double* probs, int32_t n_pro
  * store (n_new x S each, [sample][row], checked against the free memory like the run's) for st_summarize(which = 2, 3). */
 int st_predict_new_stored(st_handle* h, const st_new_rows* rows, uint64_t seed, int32_t keep_draws, st_pred_out* out);
 
+/* ---- several chains: pooled summaries and convergence diagnostics (no reference counterpart; DESIGN.md §5d) ----
+ * K chains of S draws per row.  Over all K S draws of a row, pooled: mean; sd (ddof = 1, 0 for one draw); quantiles at
+ * probs[0..n_probs) exactly as numpy.quantile(method="linear").  Per row, as ArviZ's rhat(method="rank") and
+ * ess(method="bulk" | "tail") define them (Vehtari, Gelman, Simpson, Carpenter and Buerkner 2021), with h = S / 2:
+ *   split: each chain gives its first h and its last h draws, M = 2K chains of h (odd S: the middle draw is in no split chain,
+ *   but is in the pooled statistics and the tail thresholds); z-scale: Phi^-1((r - 3/8) / (M h + 1/4)) of the average ranks
+ *   r (ties averaged) of the M h split draws;
+ *   rhat = max(R(z-scale(split x)), R(z-scale(|split x - median(split x)|))), R(y) = sqrt((B / W + h - 1) / h) with B = h
+ *   var(chain means, ddof 1), W = mean of the within-chain variances (ddof 1); NaN if either R is (W = 0);
+ *   ess_bulk = ESS(z-scale(split x)); ess_tail = min(ESS(split 1[x <= q05]), ESS(split 1[x <= q95])), q05 / q95 the pooled
+ *   0.05 / 0.95 quantiles, NaN if either is; ESS: Geyer's initial positive and monotone sequences over the mean biased
+ *   autocovariances, tau >= 1 / log10(M h), NaN when the pooled variance estimate is 0;
+ *   rhat, ess_bulk and ess_tail are NaN for S < 4 (h < 2).
+ * Draws must be finite: a chain's stored draws are (a run with a NaN log-likelihood stops with ST_ERR_NAN), and
+ * st_summarize_draws refuses non-finite host draws (ST_ERR_INVALID, with the index of the first).
+ * Every reduction runs in a fixed order: repeated calls are bit-identical.  Refused: n_chains < 1, n_samples < 1, a prob
+ * outside [0, 1] or NaN (ST_ERR_INVALID); n_chains x (n_samples + 1) above what one CTA stages in shared memory
+ * (ST_ERR_UNSUPPORTED, the limit in the message). */
+typedef struct {            /* caller-allocated; NULL pointers are skipped (all NULL: only the sizes are returned) */
+  double* mean;             /* n_rows */
+  double* sd;               /* n_rows */
+  double* quantiles;        /* n_rows x n_probs (column-major) */
+  double* rhat;             /* n_rows */
+  double* ess_bulk;         /* n_rows */
+  double* ess_tail;         /* n_rows */
+  int64_t n_rows;           /* out */
+  int32_t n_chains, n_samples;  /* out */
+} st_chains_summary_out;
+/* The device stores of `which` (as st_summarize: 0 = w, 1 = yhat, 2 = w_new, 3 = y_new) on n_chains handles, read in place.
+ * Every handle must be on the same device and store the same n_rows and S, else ST_ERR_INVALID naming the first handle that
+ * differs; a handle with nothing stored for `which` gives ST_ERR_INVALID.  That the handles were built from the same problem
+ * (so that row i means the same location on each) is the caller's responsibility.  Waits for every handle's stream, runs on
+ * that of hs[0] and returns when done; changes no handle's state (store, chain, slots, st_keep_samples_on_device mask).
+ * Errors: st_last_error(hs[0]); st_last_error(NULL) when there is no handle to report to (hs or hs[0] NULL, n_chains < 1). */
+int st_summarize_chains(st_handle* const* hs, int32_t n_chains, int32_t which, const double* probs, int32_t n_probs,
+                        st_chains_summary_out* out);
+/* The same on host draws [chain][sample][row] (n_chains x n_samples x n_rows), copied to `device` for the call and freed after
+ * it: ST_ERR_UNSUPPORTED when the copy does not fit in the free device memory.  No handle: errors are st_last_error(NULL). */
+int st_summarize_draws(int32_t device, const double* draws, int64_t n_rows, int32_t n_chains, int32_t n_samples,
+                       const double* probs, int32_t n_probs, st_chains_summary_out* out);
+
 /* ---- the Metropolis-Hastings glue (mh_adapt.h / mh_adapt.cpp), as st_mcmc_run uses it; host-only, no handle ---- */
 /* par_huvtransf_fwd / par_huvtransf_back (Rcpp exports), mh_adapt.cpp:3-15: logit / logistic on (bounds[j], bounds[j + npar]).
  * bounds: npar x 2. */

@@ -105,6 +105,13 @@ class StSummaryOut(C.Structure):
     ]
 
 
+class StChainsSummaryOut(C.Structure):
+    _fields_ = [
+        ("mean", c_double_p), ("sd", c_double_p), ("quantiles", c_double_p), ("rhat", c_double_p), ("ess_bulk", c_double_p),
+        ("ess_tail", c_double_p), ("n_rows", C.c_int64), ("n_chains", C.c_int32), ("n_samples", C.c_int32),
+    ]
+
+
 ST_KEEP_W, ST_KEEP_YHAT = 1, 2
 
 
@@ -134,6 +141,10 @@ SIGNATURES = {
     "st_keep_samples_on_device": (C.c_int, [C.c_void_p, C.c_int32]),
     "st_summarize": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, C.c_int32, C.POINTER(StSummaryOut)]),
     "st_predict_new_stored": (C.c_int, [C.c_void_p, C.POINTER(StNewRows), C.c_uint64, C.c_int32, C.POINTER(StPredOut)]),
+    "st_summarize_chains": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_int32, c_double_p, C.c_int32,
+                                      C.POINTER(StChainsSummaryOut)]),
+    "st_summarize_draws": (C.c_int, [C.c_int32, c_double_p, C.c_int64, C.c_int32, C.c_int32, c_double_p, C.c_int32,
+                                     C.POINTER(StChainsSummaryOut)]),
     "st_bench_iteration": (C.c_int, [C.c_void_p, c_double_p, C.c_int, C.c_uint64, c_double_p, c_float_p]),
     "st_set_beta_index": (C.c_int, [C.c_void_p, C.c_int]),
     "st_get_counters": (C.c_int, [C.c_void_p, c_double_p]),

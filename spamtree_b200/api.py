@@ -584,6 +584,65 @@ class SpamTreeMV:
         }
 
 
+# --------------------------------------------------------------------------------------------- several chains (§5d)
+def _chains_result(call, probs):
+    """call(probs array, StChainsSummaryOut) -> status, made twice: for the sizes, then for the outputs"""
+    pr = _f64(np.atleast_1d(np.asarray(probs, dtype=np.float64)).reshape(-1))
+    o = _lib.StChainsSummaryOut()
+    call(pr, o)
+    n = int(o.n_rows)
+    res = {k: np.zeros(n) for k in ("mean", "sd", "rhat", "ess_bulk", "ess_tail")}
+    qt = np.zeros(n * pr.size)
+    o.mean, o.sd, o.rhat, o.ess_bulk, o.ess_tail = [_dp(res[k]) for k in ("mean", "sd", "rhat", "ess_bulk", "ess_tail")]
+    o.quantiles = _dp(qt)
+    call(pr, o)
+    res["quantiles"] = qt.reshape(pr.size, n).T.copy()
+    res["probs"] = pr.copy()
+    res["n_chains"], res["n_samples"] = int(o.n_chains), int(o.n_samples)
+    return res
+
+
+def summarize_chains(models, which, probs=(0.025, 0.5, 0.975)):
+    """Pooled summaries and convergence diagnostics of the draws several chains keep on the device (st_summarize_chains):
+    which = "w" / "yhat" of each model's last run with device_samples, or "w_new" / "yhat_new" of its last
+    predict_new(samples=None, keep_draws=True).  The models must be on one device and store the same number of rows and
+    draws; that they were built from the same problem is the caller's responsibility.  Returns per row "mean", "sd" (ddof 1)
+    and "quantiles" (n x len(probs), numpy.quantile's "linear" method) over all chains' draws, rank-normalised split "rhat",
+    "ess_bulk" and "ess_tail" (Vehtari et al. 2021, as ArviZ computes them; NaN below 4 draws per chain), and "probs",
+    "n_chains", "n_samples".  R-hat can only detect what the chains' starting points expose: chains started from the same
+    values that have not moved look converged to it."""
+    if which not in SpamTreeMV._SUMMARY_WHICH:
+        raise SpamTreeError(1, f"summarize_chains: which must be one of {sorted(SpamTreeMV._SUMMARY_WHICH)}")
+    models = list(models)
+    if not models:
+        raise SpamTreeError(1, "summarize_chains: no models")
+    hs = (C.c_void_p * len(models))(*[m._h for m in models])
+    w = SpamTreeMV._SUMMARY_WHICH[which]
+
+    def call(pr, o):
+        models[0]._chk(lib.st_summarize_chains(hs, len(models), w, _dp(pr), pr.size, C.byref(o)))
+    return _chains_result(call, probs)
+
+
+def summarize_draws(draws, probs=(0.025, 0.5, 0.975), device=0):
+    """summarize_chains on host draws (st_summarize_draws): draws (n_chains, n_samples, n_rows), or (n_chains, n_samples)
+    for a scalar, are copied to the GPU for the call.  The same outputs, one row per trailing index.  The draws must be
+    finite: a NaN or infinite draw is refused (SpamTreeError code 1)."""
+    d = np.asarray(draws, dtype=np.float64)
+    if d.ndim == 2:
+        d = d[:, :, None]
+    if d.ndim != 3:
+        raise SpamTreeError(1, "summarize_draws: draws must be (n_chains, n_samples[, n_rows])")
+    d = _f64(d)
+    K, S, n = d.shape
+
+    def call(pr, o):
+        rc = lib.st_summarize_draws(int(device), _dp(d), n, K, S, _dp(pr), pr.size, C.byref(o))
+        if rc:
+            raise SpamTreeError(rc, lib.st_last_error(None).decode())
+    return _chains_result(call, probs)
+
+
 def spamtree_mv_mcmc(y, X, Z, coords, mv_id, blocking, gix_block, res_is_ref, parents, children, limited_tree,
                      layer_names, layer_gibbs_group, indexing, set_unif_bounds_in, start_w, theta, beta, tausq, mcmcsd,
                      mcmc_keep=100, mcmc_burn=100, mcmc_thin=1, num_threads=1, use_alg='S', adapting=False,
@@ -618,7 +677,8 @@ def _mv_mcmc_on(model, indexing, set_unif_bounds_in, mcmcsd, mcmc_keep, mcmc_bur
 def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree_depth=np.inf, last_not_reference=True,
              limited_tree=False, cherrypick_same_margin=True, cherrypick_group_locations=True, mvbias=0,
              mcmc=None, num_threads=4, verbose=False, settings=None, prior=None, starting=None, debug=None, *,
-             device=0, seed=1, rng_mode=1, tree_seed=0, coords_new=None, x_new=None, mv_id_new=None, summary_probs=None):
+             device=0, seed=1, rng_mode=1, tree_seed=0, coords_new=None, x_new=None, mv_id_new=None, summary_probs=None,
+             n_chains=1):
     """Mirror of the R entry point spamtree() (R/spamtree_fit.R:1-371): same arguments and defaults, same returned
     names (`coords`, `coordsinfo`, `mv_id` + everything spamtree_mv_mcmc returns).  The tree is built by the
     deterministic stand-in for make_tree() (mvbias other than 0 is not supported).
@@ -633,7 +693,18 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
     summarised there (SpamTreeMV.summarize): the result gains "w_summary" and "yhat_summary" (with coords_new also
     "w_new_summary" and "yhat_new_summary"), each a dict of per-row "mean", "sd", "quantiles" at summary_probs, "mcse",
     "ess" and "probs", and "w_mcmc" / "yhat_mcmc" (and "w_new_mcmc" / "yhat_new_mcmc") are None instead of host copies of
-    every draw.  Needs rng_mode = 1.  Every other key is unchanged."""
+    every draw.  Needs rng_mode = 1.  Every other key is unchanged.
+
+    n_chains = K > 1 (rng_mode = 1): K chains, chain k on its own handle with seed + k, one after another; starting may be
+    a list of K dicts, one per chain, else every chain starts from the same values.  As in the single-chain call, only the
+    "beta" and "tausq" starts are used (theta starts at the middle of its bounds and w at 0, as in the reference), so a
+    per-chain dict that sets "theta" or "w" is refused rather than ignored.  The result holds "coords",
+    "coordsinfo", "mv_id" and "chains", a list of K dicts, dict k being what spamtree(..., seed=seed + k) returns besides
+    those three.  It also holds the pooled summaries and diagnostics of summarize_chains / summarize_draws at summary_probs
+    (default (0.025, 0.5, 0.975)): "w_summary" and "yhat_summary" (with coords_new also "w_new_summary" and
+    "yhat_new_summary"), and "theta_summary", "beta_summary" (rows in beta_mcmc's p x q order, column-major) and
+    "tausq_summary" over the chains' samples.  R-hat can only detect what the starting points expose: identical starts are
+    the default only because the reference has a single start, so pass dispersed beta / tausq starts to test convergence."""
     y = np.asarray(y, dtype=np.float64).reshape(-1)
     x = np.asarray(x, dtype=np.float64).reshape(y.size, -1)
     coords = np.asarray(coords, dtype=np.float64)
@@ -642,7 +713,21 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
     mcmc = {"keep": 1000, "burn": 0, "thin": 1, **(mcmc or {})}
     settings = {"adapting": True, "mcmcsd": .01, "debug": False, "printall": False, **(settings or {})}
     prior = {"set_unif_bounds": None, "btmlim": None, "toplim": None, "vlim": None, **(prior or {})}
-    starting = {"beta": None, "tausq": None, "theta": None, "w": None, **(starting or {})}
+    n_chains = int(n_chains)
+    if n_chains < 1:
+        raise SpamTreeError(1, "n_chains must be at least 1")
+    if n_chains > 1 and rng_mode != 1:
+        raise SpamTreeError(1, "n_chains > 1 needs rng_mode = 1: the pooled summaries read every chain's draws on the device")
+    if isinstance(starting, (list, tuple)):
+        if len(starting) != n_chains:
+            raise SpamTreeError(1, "starting: one dict per chain")
+        if any((st or {}).get(key) is not None for st in starting for key in ("theta", "w")):
+            raise SpamTreeError(4, "starting: per-chain theta or w starts are not supported (theta starts at the middle of its "
+                                   "bounds and w at 0, as in the reference); disperse beta and tausq instead")
+        starts = [{"beta": None, "tausq": None, "theta": None, "w": None, **(st or {})} for st in starting]
+    else:
+        starts = [{"beta": None, "tausq": None, "theta": None, "w": None, **(starting or {})}] * n_chains
+    starting = starts[0]
     debug = {"sample_beta": True, "sample_tausq": True, "sample_theta": True, "sample_w": True, "sample_predicts": True,
              **(debug or {})}
     if mvbias != 0:
@@ -654,7 +739,6 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
         raise SpamTreeError(4, "Not implemented in domains of dimension d>2.")  # R/spamtree_fit.R:58-60
     q = int(np.unique(mv_id).size)
     k = q * (q - 1) // 2
-    start_beta = np.zeros(p) if starting["beta"] is None else np.asarray(starting["beta"], dtype=np.float64)
     btmlim = 1e-3 if prior["btmlim"] is None else prior["btmlim"]
     toplim = 1e3 if prior["toplim"] is None else prior["toplim"]
     vlim = toplim if prior["vlim"] is None else prior["vlim"]
@@ -673,7 +757,6 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
     start_theta = bounds.mean(axis=1)  # :138
     sd = settings["mcmcsd"]
     mcmc_mh_sd = np.eye(start_theta.size) * sd if np.ndim(sd) == 0 else np.asarray(sd, dtype=np.float64)
-    start_tausq = .1 if starting["tausq"] is None else starting["tausq"]
     # rows sorted by coordinates, ties by input order (:214, :267-269)
     ix = np.arange(y.size)
     order = np.lexsort((ix, coords[:, 1], coords[:, 0]))
@@ -687,30 +770,62 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
            tree["children_idx"])
     if limited_tree:  # R/spamtree_fit.R:310-311: make_edges_limited on the same parent-child map
         csr = csr[:2] + limited_edges_csr(tree, ys)
-    # (the arguments spamtree_mv_mcmc receives, R/spamtree_fit.R:327-362, on a handle that stays open for the prediction)
-    model = SpamTreeMV(ys, xs, cs, mvs, tree["res_is_ref"], None, None, limited_tree, tree["block_names"], tree["block_groups"],
-                       None, start_beta, start_theta, start_tausq, device=device, csr=csr, keep_H=False)
+    coordsinfo = {"Var1": cs[:, 0], "Var2": cs[:, 1], "ix": order + 1, "block": tree["blocking"], "res": tree["res"]}
+
+    def open_chain(st):
+        # (the arguments spamtree_mv_mcmc receives, R/spamtree_fit.R:327-362, on a handle that stays open for the prediction)
+        sb = np.zeros(p) if st["beta"] is None else np.asarray(st["beta"], dtype=np.float64)
+        stau = .1 if st["tausq"] is None else st["tausq"]
+        return SpamTreeMV(ys, xs, cs, mvs, tree["res_is_ref"], None, None, limited_tree, tree["block_names"], tree["block_groups"],
+                          None, sb, start_theta, stau, device=device, csr=csr, keep_H=False)
+
     summ = summary_probs is not None
-    try:
+
+    def run_chain(model, seed_k, on_device):
+        """the chain and its prediction; on_device: the draws also stay on the device for the pooled summaries"""
         results = _mv_mcmc_on(model, None, bounds, mcmc_mh_sd, mcmc["keep"], mcmc["burn"], mcmc["thin"], settings["adapting"],
                               debug["sample_beta"], debug["sample_tausq"], debug["sample_theta"], debug["sample_w"],
-                              debug["sample_predicts"], rng_mode, seed, not summ, not summ,
-                              device_samples=("w", "yhat") if summ else ())
+                              debug["sample_predicts"], rng_mode, seed_k, not summ, not summ,
+                              device_samples=("w", "yhat") if summ or on_device else ())
         if summ:
             results["w_summary"] = model.summarize("w", summary_probs)
             results["yhat_summary"] = model.summarize("yhat", summary_probs)
         if coords_new is not None:
+            if summ or on_device:  # (the same draws as from the host samples: DESIGN.md §5c)
+                pr = model.predict_new(coords_new, x_new, mv_id_new, tree["new"], None, seed=seed_k, draws=not summ, keep_draws=True)
+            else:
+                pr = model.predict_new(coords_new, x_new, mv_id_new, tree["new"], results, seed=seed_k)
             if summ:
-                pr = model.predict_new(coords_new, x_new, mv_id_new, tree["new"], None, seed=seed, draws=False, keep_draws=True)
                 results["w_new_mcmc"] = results["yhat_new_mcmc"] = None
                 results["w_new_summary"] = model.summarize("w_new", summary_probs)
                 results["yhat_new_summary"] = model.summarize("yhat_new", summary_probs)
             else:
-                pr = model.predict_new(coords_new, x_new, mv_id_new, tree["new"], results, seed=seed)
                 results["w_new_mcmc"], results["yhat_new_mcmc"] = np.ascontiguousarray(pr["w_new"]), np.ascontiguousarray(pr["yhat_new"])
             for k in ("w_new_mean", "w_new_sd", "yhat_new_mean", "yhat_new_sd"):
                 results[k] = pr[k]
+        return results
+
+    if n_chains == 1:
+        model = open_chain(starting)
+        try:
+            results = run_chain(model, seed, False)
+        finally:
+            model.close()
+        return {"coords": cs, "coordsinfo": coordsinfo, "mv_id": mv_id, **results}
+    models, chains = [], []
+    probs = summary_probs if summ else (0.025, 0.5, 0.975)
+    out = {"coords": cs, "coordsinfo": coordsinfo, "mv_id": mv_id, "chains": chains}
+    try:
+        for k in range(n_chains):  # every handle keeps its draws on the device until the pooled summaries are formed
+            models.append(open_chain(starts[k]))
+            chains.append(run_chain(models[-1], seed + k, True))
+        for which in ("w", "yhat") + (("w_new", "yhat_new") if coords_new is not None else ()):
+            out[which + "_summary"] = summarize_chains(models, which, probs)
     finally:
-        model.close()
-    coordsinfo = {"Var1": cs[:, 0], "Var2": cs[:, 1], "ix": order + 1, "block": tree["blocking"], "res": tree["res"]}
-    return {"coords": cs, "coordsinfo": coordsinfo, "mv_id": mv_id, **results}
+        for m in models:
+            m.close()
+    out["theta_summary"] = summarize_draws(np.stack([c["theta_mcmc"].T for c in chains]), probs, device=device)
+    out["beta_summary"] = summarize_draws(np.stack([c["beta_mcmc"].transpose(1, 2, 0).reshape(-1, p * q) for c in chains]),
+                                          probs, device=device)
+    out["tausq_summary"] = summarize_draws(np.stack([c["tausq_mcmc"].T for c in chains]), probs, device=device)
+    return out

@@ -3,6 +3,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <vector>
 
 #include "../../include/spamtree_b200.h"
 #include "st_kernels.cuh"
@@ -254,6 +255,96 @@ int st_predict_new_stored(st_handle* h, const st_new_rows* rows, uint64_t seed, 
   ps.seed = seed;
   return h->model.predict_new(*rows, ps, *out, true, keep_draws != 0);
   ST_GUARD_END(h)
+}
+int st_summarize_chains(st_handle* const* hs, int32_t n_chains, int32_t which, const double* probs, int32_t n_probs,
+                        st_chains_summary_out* out) {
+  if (!hs || n_chains < 1 || !hs[0]) {  // (no handle to report to)
+    g_create_error = n_chains < 1 ? "st_summarize_chains: n_chains must be at least 1" : "st_summarize_chains: hs or hs[0] is NULL";
+    return ST_ERR_INVALID;
+  }
+  st_handle* h0 = hs[0];
+  st::Model& M0 = h0->model;
+  if (!out) { M0.err = "st_summarize_chains: out is NULL"; return ST_ERR_INVALID; }
+  activate(h0);
+  ST_GUARD_BEGIN
+  static const char* names[4] = {"w", "yhat", "w_new", "y_new"};
+  if (which < 0 || which > 3) { M0.err = "st_summarize_chains: which must be 0 (w), 1 (yhat), 2 (w_new) or 3 (y_new)"; return ST_ERR_INVALID; }
+  const int64_t n = M0.store_[which].n;
+  const int S = M0.store_[which].S;
+  int rc = st::chains_check("st_summarize_chains", n_chains, std::max(S, 1), probs, n_probs, M0.err);
+  if (rc) return rc;
+  std::vector<const double*> src(n_chains);
+  for (int k = 0; k < n_chains; k++) {
+    const std::string hk = "st_summarize_chains: handle " + std::to_string(k);
+    if (!hs[k]) { M0.err = hk + " is NULL"; return ST_ERR_INVALID; }
+    const st::Model& Mk = hs[k]->model;
+    const st::Model::SampleStore& s = Mk.store_[which];
+    if (Mk.device != M0.device) {
+      M0.err = hk + " is on device " + std::to_string(Mk.device) + ", handle 0 on device " + std::to_string(M0.device);
+      return ST_ERR_INVALID;
+    }
+    if (!s.d || s.S < 1) {
+      M0.err = hk + " has no stored draws of " + names[which] +
+               (which < 2 ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)" : " (st_predict_new_stored with keep_draws)");
+      return ST_ERR_INVALID;
+    }
+    if (s.n != n || s.S != S) {
+      M0.err = hk + " stores " + std::to_string(s.S) + " draws of " + std::to_string(s.n) + " rows, handle 0 " + std::to_string(S) +
+               " draws of " + std::to_string(n) + " rows";
+      return ST_ERR_INVALID;
+    }
+    src[k] = s.d;
+  }
+  for (int k = 1; k < n_chains; k++)  // every store is complete before the kernel reads it on hs[0]'s stream
+    if (const cudaError_t e = cudaStreamSynchronize(hs[k]->model.stream)) {
+      M0.err = std::string("st_summarize_chains: CUDA error in sync of handle ") + std::to_string(k) + ": " + cudaGetErrorString(e);
+      return ST_ERR_CUDA;
+    }
+  return st::summarize_chains(src.data(), n, n_chains, S, probs, n_probs, *out, M0.stream, M0.err);
+  ST_GUARD_END(h0)
+}
+int st_summarize_draws(int32_t device, const double* draws, int64_t n_rows, int32_t n_chains, int32_t n_samples,
+                       const double* probs, int32_t n_probs, st_chains_summary_out* out) {
+  if (!out || n_rows < 0 || (n_rows > 0 && !draws)) { g_create_error = "st_summarize_draws: out or draws missing, or n_rows < 0"; return ST_ERR_INVALID; }
+  try {
+    int rc = st::chains_check("st_summarize_draws", n_chains, n_samples, probs, n_probs, g_create_error);
+    if (rc) return rc;
+    const size_t all = (size_t)n_rows * n_samples * n_chains;
+    for (size_t j = 0; j < all; j++)
+      if (!std::isfinite(draws[j])) {
+        g_create_error = "st_summarize_draws: draw " + std::to_string(j) + " ([chain][sample][row] order) is not finite";
+        return ST_ERR_INVALID;
+      }
+    const bool any = out->mean || out->sd || out->quantiles || out->rhat || out->ess_bulk || out->ess_tail;
+    if (!any || n_rows == 0) return st::summarize_chains(nullptr, n_rows, n_chains, n_samples, probs, n_probs, *out, 0, g_create_error);
+    if (cudaSetDevice(device) != cudaSuccess) { (void)cudaGetLastError(); g_create_error = "st_summarize_draws: cudaSetDevice failed"; return ST_ERR_CUDA; }
+    const size_t per = (size_t)n_rows * n_samples, bytes = per * n_chains * sizeof(double);
+    size_t fr = 0, tot = 0;
+    if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { (void)cudaGetLastError(); g_create_error = "st_summarize_draws: cudaMemGetInfo failed"; return ST_ERR_CUDA; }
+    // (the copy, plus the outputs' buffer and some headroom)
+    const size_t need = bytes + (size_t)n_rows * (5 + n_probs) * sizeof(double) + (64u << 20);
+    if (need > fr) {
+      g_create_error = "st_summarize_draws: the draws need " + std::to_string(need) + " bytes of device memory and " + std::to_string(fr) +
+                       " bytes are free";
+      return ST_ERR_UNSUPPORTED;
+    }
+    double* d = nullptr;
+    cudaError_t e = cudaMalloc((void**)&d, bytes);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); g_create_error = std::string("st_summarize_draws: ") + cudaGetErrorString(e); return ST_ERR_UNSUPPORTED; }
+    e = cudaMemcpyAsync(d, draws, bytes, cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess) {
+      std::vector<const double*> src(n_chains);
+      for (int c = 0; c < n_chains; c++) src[c] = d + (size_t)c * per;
+      rc = st::summarize_chains(src.data(), n_rows, n_chains, n_samples, probs, n_probs, *out, 0, g_create_error);
+    } else {
+      g_create_error = std::string("CUDA error in H2D draws: ") + cudaGetErrorString(e);
+      rc = ST_ERR_CUDA;
+    }
+    cudaStreamSynchronize(0);
+    cudaFree(d);
+    return rc;
+  } catch (const std::exception& ex) { g_create_error = ex.what(); } catch (...) { g_create_error = "unknown exception"; }
+  return ST_ERR_INVALID;
 }
 int st_bench_iteration(st_handle* h, const double* theta_prop, int do_swap, uint64_t seed, double* out3, float* ms_out) {
   if (!h || !theta_prop || !out3) return ST_ERR_INVALID;

@@ -1205,11 +1205,49 @@ __device__ __forceinline__ double summary_group_sum(double v, double* red, int G
   return total;
 }
 
+// sort each of the R rows of S keys at key[r S ..) ascending: the all-ascending form of the bitonic network (a "flip" stage
+// then half-cleaners) over pairs (i, j > i), so positions >= S act as +inf and are never touched (no padding is staged).
+// Called by every thread of the CTA; ends with a barrier.
+__device__ void summary_sort_rows(unsigned long long* key, int R, int S) {
+  const int t = threadIdx.x, T = blockDim.x;
+  int P2 = 1;
+  while (P2 < S) P2 <<= 1;
+  const int half = P2 >> 1;
+  const long long pairs = (long long)R * half;
+  for (int k = 2; k <= P2; k <<= 1) {
+    for (int d = k >> 1; d > 0; d >>= 1) {
+      const bool flip = d == (k >> 1);
+      for (long long e = t; e < pairs; e += T) {
+        const int rr = (int)(e / half), pp = (int)(e % half);
+        const int i = (pp / d) * 2 * d + pp % d;
+        const int j = flip ? (i ^ (k - 1)) : i + d;
+        if (j < S) {
+          unsigned long long* kk = key + (long long)rr * S;
+          const unsigned long long a = kk[i], c = kk[j];
+          if (a > c) { kk[i] = c; kk[j] = a; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// the p-quantile of S sorted keys: numpy's method "linear" (R type 7) with its virtual-index and _lerp formulas, without
+// contraction
+__device__ double summary_quantile(const unsigned long long* kk, int S, double p) {
+  const double vi = __dmul_rn((double)(S - 1), p);
+  if (vi >= (double)(S - 1)) return summary_val(kk[S - 1]);
+  const int lo = (int)floor(vi);
+  const double g = __dsub_rn(vi, (double)lo);
+  const double a = summary_val(kk[lo]), c = summary_val(kk[lo + 1]);
+  const double diff = __dsub_rn(c, a);
+  return g >= 0.5 ? __dsub_rn(c, __dmul_rn(diff, __dsub_rn(1.0, g))) : __dadd_rn(a, __dmul_rn(diff, g));
+}
+
 // One CTA per tile of R rows of a [sample][row] store (element (s, i) at src[s * n + i]).  The tile's S x R values are read
 // once with coalesced loads (consecutive threads, consecutive rows), staged as order-preserving keys (row-major: key[r S + s]),
 // and every statistic is formed from the staged copy: the moments and batch means in sample order, then the quantiles after a
-// bitonic sort of each row in shared memory.  The sort is the all-ascending form of the network (a "flip" stage then
-// half-cleaners), so positions >= S act as +inf and are never touched: no padding is staged.  Every reduction is over G = T / R
+// bitonic sort of each row in shared memory (summary_sort_rows).  Every reduction is over G = T / R
 // threads per row in a fixed order.  Outputs: mean, sd (ddof 1), quant (n x np, column-major), mcse, ess (batch means).
 __global__ void __launch_bounds__(kSummaryThreads)
 summary_kernel(const double* __restrict__ src, long long n, int S, int R, const double* __restrict__ probs, int np,
@@ -1267,44 +1305,10 @@ summary_kernel(const double* __restrict__ src, long long n, int S, int R, const 
     ess_out[i] = ok ? (double)S * var / sig2 : __longlong_as_double(0x7ff8000000000000LL);
   }
   if (np == 0) return;
-  // ---- sort every row of the tile: all ascending, pairs (i, j > i), j >= S skipped
-  int P2 = 1;
-  while (P2 < S) P2 <<= 1;
-  const int half = P2 >> 1;
-  const long long pairs = (long long)R * half;
-  for (int k = 2; k <= P2; k <<= 1) {
-    for (int d = k >> 1; d > 0; d >>= 1) {
-      const bool flip = d == (k >> 1);
-      for (long long e = t; e < pairs; e += T) {
-        const int rr = (int)(e / half), pp = (int)(e % half);
-        const int i = (pp / d) * 2 * d + pp % d;
-        const int j = flip ? (i ^ (k - 1)) : i + d;
-        if (j < S) {
-          unsigned long long* kk = key + (long long)rr * S;
-          const unsigned long long a = kk[i], c = kk[j];
-          if (a > c) { kk[i] = c; kk[j] = a; }
-        }
-      }
-      __syncthreads();
-    }
-  }
-  // ---- quantiles: numpy's method "linear" (R type 7) with its virtual-index and _lerp formulas, without contraction
+  summary_sort_rows(key, R, S);
   for (int e = t; e < R * np; e += T) {
     const int rr = e / np, jp = e % np;
-    if (rr >= nr) continue;
-    const unsigned long long* kk = key + (long long)rr * S;
-    const double vi = __dmul_rn((double)(S - 1), probs[jp]);
-    double res;
-    if (vi >= (double)(S - 1)) {
-      res = summary_val(kk[S - 1]);
-    } else {
-      const int lo = (int)floor(vi);
-      const double g = __dsub_rn(vi, (double)lo);
-      const double a = summary_val(kk[lo]), c = summary_val(kk[lo + 1]);
-      const double diff = __dsub_rn(c, a);
-      res = g >= 0.5 ? __dsub_rn(c, __dmul_rn(diff, __dsub_rn(1.0, g))) : __dadd_rn(a, __dmul_rn(diff, g));
-    }
-    quant[row0 + rr + (long long)jp * n] = res;
+    if (rr < nr) quant[row0 + rr + (long long)jp * n] = summary_quantile(key + (long long)rr * S, S, probs[jp]);
   }
 }
 int summary_rows_per_cta(int S, size_t smem_cap) {
@@ -1323,6 +1327,263 @@ cudaError_t launch_summary(const double* src, long long n, int S, int R, const d
   cudaError_t e = ensure_dynamic_smem(summary_kernel, smem, opt);
   if (e != cudaSuccess) return e;
   summary_kernel<<<(unsigned)((n + R - 1) / R), kSummaryThreads, smem, st>>>(src, n, S, R, probs, np, mean, sd, quant, mcse, ess);
+  return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------ several chains: pooled summaries and
+// rank-normalised split-R-hat, bulk-ESS and tail-ESS (st_summarize_chains / st_summarize_draws; DESIGN.md §5d)
+typedef unsigned long long u64;
+__device__ __forceinline__ int keys_lower(const u64* b, int N, u64 k) {  // first j with b[j] >= k
+  int lo = 0, hi = N;
+  while (lo < hi) { const int m = (lo + hi) >> 1; if (b[m] < k) lo = m + 1; else hi = m; }
+  return lo;
+}
+__device__ __forceinline__ int keys_upper(const u64* b, int N, u64 k) {  // first j with b[j] > k
+  int lo = 0, hi = N;
+  while (lo < hi) { const int m = (lo + hi) >> 1; if (b[m] <= k) lo = m + 1; else hi = m; }
+  return lo;
+}
+
+// One row of a tile: a = its K x S draws as keys in sample order (a[c S + s]), b = the same sorted, cm = 2K doubles of
+// scratch.  Split chain c (of M = 2K, h draws each) is the first (c even) or the last (c odd) h draws of chain c / 2; for odd
+// S each chain's middle draw a[c S + h] belongs to no split chain.
+struct ChainsRow {
+  u64* a;
+  const u64* b;
+  double* cm;
+  int K, S, h, N;
+  __device__ int pos(int c, int i) const { return (c >> 1) * S + ((c & 1) ? S - h : 0) + i; }
+  __device__ bool odd() const { return S & 1; }
+  __device__ u64 mid(int k) const { return a[k * S + h]; }
+  // (count < v, count <= v) of the split draws: of all N from b, less the middle draws for odd S
+  __device__ void rank_counts(u64 v, int& lt, int& le) const {
+    lt = keys_lower(b, N, v);
+    le = keys_upper(b, N, v);
+    if (odd())
+      for (int k = 0; k < K; k++) { const u64 m = mid(k); lt -= m < v; le -= m <= v; }
+  }
+  // the j-th smallest split draw (0-based): the first b[i] with more than j split draws <= b[i]
+  __device__ double split_order_stat(int j) const {
+    int lo = 0, hi = N - 1;
+    while (lo < hi) {
+      const int m = (lo + hi) >> 1;
+      int lt, le;
+      rank_counts(b[m], lt, le);
+      if (le > j) hi = m; else lo = m + 1;
+    }
+    return summary_val(b[lo]);
+  }
+  // z-scale of a key among the 2 K h split draws: Phi^-1((r - 3/8) / (N' + 1/4)), r its average rank
+  __device__ double z_bulk(u64 v) const {
+    int lt, le;
+    rank_counts(v, lt, le);
+    return normcdfinv(((double)(lt + 1 + le) / 2.0 - 0.375) / ((double)(2 * K * h) + 0.25));
+  }
+  // z-scale of f = |x - med| among the folded split draws.  b[0, m) (values < med) folds to a non-increasing run and b[m, N)
+  // to a non-decreasing one, so each count is a binary search on either side of m with the folded values formed on the fly
+  // exactly as |x - med| is formed for x itself
+  __device__ double z_fold(double f, double med, int m) const {
+    int l0 = 0, l1 = m, r0 = m, r1 = N;  // l: first j < m with |b_j - med| < f; r: first j >= m with |b_j - med| >= f
+    while (l0 < l1) { const int q = (l0 + l1) >> 1; if (fabs(summary_val(b[q]) - med) < f) l1 = q; else l0 = q + 1; }
+    while (r0 < r1) { const int q = (r0 + r1) >> 1; if (fabs(summary_val(b[q]) - med) >= f) r1 = q; else r0 = q + 1; }
+    int lt = r0 - l0;
+    int u0 = 0, u1 = m, v0 = m, v1 = N;  // the same with <= f / > f
+    while (u0 < u1) { const int q = (u0 + u1) >> 1; if (fabs(summary_val(b[q]) - med) <= f) u1 = q; else u0 = q + 1; }
+    while (v0 < v1) { const int q = (v0 + v1) >> 1; if (fabs(summary_val(b[q]) - med) > f) v1 = q; else v0 = q + 1; }
+    int le = v0 - u0;
+    if (odd())
+      for (int k = 0; k < K; k++) { const double g = fabs(summary_val(mid(k)) - med); lt -= g < f; le -= g <= f; }
+    return normcdfinv(((double)(lt + 1 + le) / 2.0 - 0.375) / ((double)(2 * K * h) + 0.25));
+  }
+};
+
+// Chain means of f(c, i) (c < M split chains, i < h) into row.cm, then every thread of the row gets mean_var (= W, the mean
+// within-chain variance, ddof 1) and var_m (the variance of the chain means, ddof 1).  Every sum runs in a fixed order.
+// Called by every thread of the CTA.
+template <class F>
+__device__ void chains_moments(const ChainsRow& row, F f, int G, int lane, double* red, double& mean_var, double& var_m) {
+  const int M = 2 * row.K, h = row.h, t = threadIdx.x;
+  const int tpc = max(1, G / M), cpp = G / tpc;  // threads per chain, chains per pass
+  for (int c0 = 0; c0 < M; c0 += cpp) {
+    const int c = c0 + lane / tpc, part = lane % tpc;
+    const bool mine = lane / tpc < cpp && c < M;
+    double acc = 0.0;
+    if (mine)
+      for (int i = part; i < h; i += tpc) acc += f(c, i);
+    red[t] = acc;
+    __syncthreads();
+    if (mine && part == 0) {
+      double s = 0.0;
+      for (int j = 0; j < tpc; j++) s += red[t + j];
+      row.cm[c] = s / h;
+    }
+    __syncthreads();
+  }
+  double acc = 0.0;
+  for (long long e = lane; e < (long long)M * h; e += G) {
+    const int c = (int)(e / h), i = (int)(e % h);
+    const double d = f(c, i) - row.cm[c];
+    acc += d * d;
+  }
+  const double ss = summary_group_sum(acc, red, G);
+  mean_var = ss / ((double)M * h) * h / (h - 1);
+  double mm = 0.0;
+  for (int c = 0; c < M; c++) mm += row.cm[c];
+  mm /= M;
+  double vm = 0.0;
+  for (int c = 0; c < M; c++) { const double d = row.cm[c] - mm; vm += d * d; }
+  var_m = vm / (M - 1);
+}
+
+__device__ __forceinline__ double chains_rhat(double mean_var, double var_m, int h) {
+  return mean_var > 0.0 ? sqrt(((double)h * var_m / mean_var + h - 1) / h) : __longlong_as_double(0x7ff8000000000000LL);
+}
+
+// ESS of f after chains_moments (row.cm holds its chain means): autocovariances by direct sums over lags, two lags per step,
+// until Geyer's initial positive sequence stops (row by row; the CTA steps while any row goes on).  The initial monotone
+// sequence is applied on the fly: it replaces each pair sum by the running minimum of the pair sums before it.
+template <class F>
+__device__ double chains_ess(const ChainsRow& row, F f, int G, int lane, double* red, double mean_var, double var_m, bool live) {
+  const int M = 2 * row.K, h = row.h;
+  const double var_plus = mean_var * (h - 1) / h + var_m;
+  bool act = live && var_plus > 0.0;
+  auto lag_mean = [&](int lag, bool on) {  // mean over the chains of the biased autocovariance at lag
+    double acc = 0.0;
+    if (on) {
+      const int L = h - lag;
+      for (long long e = lane; e < (long long)M * L; e += G) {
+        const int c = (int)(e / L), i = (int)(e % L);
+        acc += (f(c, i) - row.cm[c]) * (f(c, i + lag) - row.cm[c]);
+      }
+    }
+    return summary_group_sum(acc, red, G) / h / M;
+  };
+  const double a1 = lag_mean(1, act);
+  double ev = 1.0, od = act ? 1.0 - (mean_var - a1) / var_plus : 0.0;
+  double pmin = 0.0, sum_p = 0.0, last = 0.0;
+  for (int k = 0;; k++) {
+    if (act) {  // pair k = (rho_2k, rho_2k+1): inside the sequence, or the pair that ends it
+      const double P = ev + od;
+      if (2 * k + 1 < h - 3 && P > 0.0) {
+        pmin = k ? fmin(pmin, P) : P;
+        sum_p += pmin;
+      } else {
+        last = (ev > 0.0 || P >= 0.0) ? ev : 0.0;
+        act = false;
+      }
+    }
+    if (!__syncthreads_or(act)) break;
+    const double ae = lag_mean(2 * k + 2, act), ao = lag_mean(2 * k + 3, act);
+    if (act) { ev = 1.0 - (mean_var - ae) / var_plus; od = 1.0 - (mean_var - ao) / var_plus; }
+  }
+  if (!(live && var_plus > 0.0)) return __longlong_as_double(0x7ff8000000000000LL);
+  const double n = (double)M * h;
+  const double tau = fmax(-1.0 + 2.0 * sum_p + last, 1.0 / log10(n));
+  return n / tau;
+}
+
+// One CTA per tile of R rows; chain c's draws of row i at src[c][s n + i].  The tile's K S draws per row are read with
+// coalesced loads into keys in sample order (a) and copied (b), -0 staged as +0; b is sorted (summary_sort_rows).  Pooled mean and sd come
+// from a, pooled quantiles, q05 / q95 and the split median from b.  Then, in this order: tail-ESS of the indicators
+// x <= q05 / q95 (read from a); the folded R-hat from z-scales formed on the fly; the bulk z-scales, written over a in place
+// (each thread reads and writes only its own draws, and the middle draws for odd S stay keys); bulk R-hat and ESS.
+__global__ void __launch_bounds__(kSummaryThreads)
+chains_summary_kernel(const double* const* __restrict__ src, long long n, int K, int S, int R, const double* __restrict__ probs,
+                      int np, double* __restrict__ mean_out, double* __restrict__ sd_out, double* __restrict__ quant,
+                      double* __restrict__ rhat_out, double* __restrict__ essb_out, double* __restrict__ esst_out) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int T = blockDim.x, t = threadIdx.x, G = T / R, r = t / G, lane = t % G;
+  const int N = K * S, h = S / 2, M = 2 * K;
+  double* red = reinterpret_cast<double*>(smem_raw);  // T
+  double* cmb = red + T;                              // R x M
+  u64* akey = reinterpret_cast<u64*>(cmb + (size_t)R * M);
+  u64* bkey = akey + (size_t)R * N;
+  const long long row0 = (long long)blockIdx.x * R;
+  const int nr = (int)min((long long)R, n - row0);
+  // ---- stage: element e of the tile is (chain e / (S R), sample (e / R) % S, row e % R); rows past n hold zeros
+  const long long tot = (long long)N * R;
+  for (long long e = t; e < tot; e += T) {
+    const int c = (int)(e / ((long long)S * R)), s = (int)((e / R) % S), rr = (int)(e % R);
+    const double v = rr < nr ? src[c][(long long)s * n + row0 + rr] : 0.0;
+    const u64 k = summary_key(v == 0.0 ? 0.0 : v);  // -0 as +0: ranks treat them as a tie, as numpy compares them
+    akey[(size_t)rr * N + (size_t)c * S + s] = k;
+    bkey[(size_t)rr * N + (size_t)c * S + s] = k;
+  }
+  __syncthreads();
+  ChainsRow row{akey + (size_t)r * N, bkey + (size_t)r * N, cmb + (size_t)r * M, K, S, h, N};
+  // ---- pooled mean and sd (two passes in sample order)
+  double acc = 0.0;
+  for (int j = lane; j < N; j += G) acc += summary_val(row.a[j]);
+  const double mean = summary_group_sum(acc, red, G) / N;
+  acc = 0.0;
+  for (int j = lane; j < N; j += G) { const double d = summary_val(row.a[j]) - mean; acc += d * d; }
+  const double ss = summary_group_sum(acc, red, G);
+  summary_sort_rows(bkey, R, N);
+  for (int e = t; e < R * np; e += T) {
+    const int rr = e / np, jp = e % np;
+    if (rr < nr) quant[row0 + rr + (long long)jp * n] = summary_quantile(bkey + (size_t)rr * N, N, probs[jp]);
+  }
+  const bool live = r < nr;
+  double rhat = __longlong_as_double(0x7ff8000000000000LL), essb = rhat, esst = rhat;
+  if (h >= 2) {
+    double mv, vm;
+    // ---- tail-ESS: split indicators of x <= q05 and x <= q95 (pooled quantiles, all K S draws)
+    double e2[2];
+    for (int j = 0; j < 2; j++) {
+      const double q = summary_quantile(row.b, N, j ? 0.95 : 0.05);
+      auto ind = [&](int c, int i) { return summary_val(row.a[row.pos(c, i)]) <= q ? 1.0 : 0.0; };
+      chains_moments(row, ind, G, lane, red, mv, vm);
+      e2[j] = chains_ess(row, ind, G, lane, red, mv, vm, live);
+    }
+    esst = (isnan(e2[0]) || isnan(e2[1])) ? __longlong_as_double(0x7ff8000000000000LL) : fmin(e2[0], e2[1]);
+    // ---- folded R-hat: z-scale of |x - median of the split draws|
+    const int Ns = M * h;  // even
+    const double med = (row.split_order_stat(Ns / 2 - 1) + row.split_order_stat(Ns / 2)) / 2.0;
+    int m0 = 0, m1 = N;
+    while (m0 < m1) { const int q = (m0 + m1) >> 1; if (summary_val(row.b[q]) < med) m0 = q + 1; else m1 = q; }
+    auto zf = [&](int c, int i) { return row.z_fold(fabs(summary_val(row.a[row.pos(c, i)]) - med), med, m0); };
+    chains_moments(row, zf, G, lane, red, mv, vm);
+    const double rf = chains_rhat(mv, vm, h);
+    // ---- bulk: z-scales in place of the split draws' keys
+    double* za = reinterpret_cast<double*>(row.a);
+    for (int e = lane; e < Ns; e += G) {
+      const int p = row.pos(e / h, e % h);
+      za[p] = row.z_bulk(row.a[p]);
+    }
+    __syncthreads();
+    auto zb = [&](int c, int i) { return za[row.pos(c, i)]; };
+    chains_moments(row, zb, G, lane, red, mv, vm);
+    const double rb = chains_rhat(mv, vm, h);
+    rhat = (isnan(rb) || isnan(rf)) ? __longlong_as_double(0x7ff8000000000000LL) : fmax(rb, rf);
+    essb = chains_ess(row, zb, G, lane, red, mv, vm, live);
+  }
+  if (lane == 0 && live) {
+    const long long i = row0 + r;
+    mean_out[i] = mean;
+    sd_out[i] = N > 1 ? sqrt(ss / (N - 1)) : 0.0;
+    rhat_out[i] = rhat;
+    essb_out[i] = essb;
+    esst_out[i] = esst;
+  }
+}
+size_t chains_smem_bytes(int K, int S, int R) {
+  return (size_t)kSummaryThreads * sizeof(double) + (size_t)R * 2 * K * sizeof(double) + (size_t)R * 2 * K * S * sizeof(u64);
+}
+int chains_rows_per_cta(int K, int S, size_t smem_cap) {
+  if (K < 1 || S < 1) return 0;
+  int R = kSummaryMaxRows;
+  while (R >= 1 && chains_smem_bytes(K, S, R) > smem_cap) R >>= 1;
+  return R;
+}
+cudaError_t launch_chains_summary(const double* const* src, long long n, int K, int S, int R, const double* probs, int np, double* mean,
+                                  double* sd, double* quant, double* rhat, double* ess_bulk, double* ess_tail, cudaStream_t st) {
+  if (n <= 0 || K <= 0 || S <= 0) return cudaSuccess;
+  static SmemOptIn opt;
+  const size_t smem = chains_smem_bytes(K, S, R);
+  cudaError_t e = ensure_dynamic_smem(chains_summary_kernel, smem, opt);
+  if (e != cudaSuccess) return e;
+  chains_summary_kernel<<<(unsigned)((n + R - 1) / R), kSummaryThreads, smem, st>>>(src, n, K, S, R, probs, np, mean, sd, quant, rhat,
+                                                                                   ess_bulk, ess_tail);
   return cudaGetLastError();
 }
 

@@ -135,5 +135,12 @@ size_t summary_smem_bytes(int S, int R);
 // (batch means); every output a device array of n (quant: n np)
 cudaError_t launch_summary(const double* src, long long n, int S, int R, const double* probs, int np, double* mean, double* sd, double* quant,
                            double* mcse, double* ess, cudaStream_t st);
+// ---- K chains of S draws of n rows, chain c's draw (s, i) at src[c][s * n + i] (src: a device array of K device pointers):
+// pooled mean, sd (ddof 1), quantiles, and rank-normalised split-R-hat, bulk-ESS and tail-ESS (st_summarize_chains; §5d).
+// Shared memory per row: 2 K S keys and 2 K doubles, so one row fits while K (S + 1) <= (smem_cap - 8 kSummaryThreads) / 16
+size_t chains_smem_bytes(int K, int S, int R);
+int chains_rows_per_cta(int K, int S, size_t smem_cap);  // as summary_rows_per_cta; 0 when not even one row fits
+cudaError_t launch_chains_summary(const double* const* src, long long n, int K, int S, int R, const double* probs, int np, double* mean,
+                                  double* sd, double* quant, double* rhat, double* ess_bulk, double* ess_tail, cudaStream_t st);
 
 }  // namespace st

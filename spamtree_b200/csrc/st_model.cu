@@ -2074,6 +2074,57 @@ int Model::summarize(int which, const double* probs, int n_probs, st_summary_out
   return 0;
 }
 
+// ---- several chains (st_summarize_chains, st_summarize_draws; DESIGN.md §5d)
+static const size_t kChainsSmemCap = 227 * 1024;
+
+int chains_check(const char* what, int K, int S, const double* probs, int n_probs, std::string& err) {
+  if (K < 1 || S < 1) { err = std::string(what) + ": n_chains and n_samples must be at least 1"; return 1; }
+  if (n_probs < 0 || (n_probs > 0 && !probs)) { err = std::string(what) + ": n_probs < 0, or probs missing"; return 1; }
+  for (int j = 0; j < n_probs; j++)
+    if (!(probs[j] >= 0.0 && probs[j] <= 1.0)) { err = std::string(what) + ": every prob must lie in [0, 1] (NaN is refused)"; return 1; }
+  if (chains_rows_per_cta(K, S, kChainsSmemCap) < 1) {
+    err = std::string(what) + ": " + std::to_string(K) + " chains of " + std::to_string(S) + " draws exceed what one CTA stages in "
+          "shared memory (n_chains x (n_samples + 1) = " + std::to_string((long long)K * (S + 1)) + ", at most " +
+          std::to_string((kChainsSmemCap - (size_t)kSummaryThreads * sizeof(double)) / (2 * sizeof(double))) + ")";
+    return 4;
+  }
+  return 0;
+}
+
+int summarize_chains(const double* const* src, int64_t n, int K, int S, const double* probs, int n_probs, st_chains_summary_out& out,
+                     cudaStream_t st, std::string& err) {
+  out.n_rows = n;
+  out.n_chains = K;
+  out.n_samples = S;
+  double* hdst[6] = {out.mean, out.sd, out.quantiles, out.rhat, out.ess_bulk, out.ess_tail};
+  if (!(hdst[0] || hdst[1] || hdst[2] || hdst[3] || hdst[4] || hdst[5]) || n == 0) return 0;
+  // one device buffer: mean | sd | rhat | ess_bulk | ess_tail | quantiles (n x n_probs) | probs | the K chain pointers
+  const size_t nn = (size_t)n, nd = (5 + (size_t)n_probs) * nn + (size_t)n_probs + (size_t)K;
+  double* d = nullptr;
+  cudaError_t e = cudaMalloc((void**)&d, nd * sizeof(double));
+  if (e != cudaSuccess) { (void)cudaGetLastError(); err = std::string("CUDA error in alloc summaries: ") + cudaGetErrorString(e); return 2; }
+  struct Free { double* p; ~Free() { cudaFree(p); } } fr{d};
+  double* dq = d + 5 * nn;
+  double* dp = dq + (size_t)n_probs * nn;
+  const double** dsrc = reinterpret_cast<const double**>(dp + n_probs);
+  const double* outs[6] = {d, d + nn, dq, d + 2 * nn, d + 3 * nn, d + 4 * nn};
+  auto chk = [&](cudaError_t c, const char* what) {
+    if (c != cudaSuccess && e == cudaSuccess) { e = c; err = std::string("CUDA error in ") + what + ": " + cudaGetErrorString(c); }
+  };
+  if (n_probs) chk(cudaMemcpyAsync(dp, probs, n_probs * sizeof(double), cudaMemcpyHostToDevice, st), "H2D probs");
+  chk(cudaMemcpyAsync(dsrc, src, K * sizeof(double*), cudaMemcpyHostToDevice, st), "H2D chain pointers");
+  if (e == cudaSuccess)
+    chk(launch_chains_summary(dsrc, n, K, S, chains_rows_per_cta(K, S, kChainsSmemCap), dp, n_probs, d, d + nn, dq, d + 2 * nn,
+                              d + 3 * nn, d + 4 * nn, st),
+        "chains_summary_kernel");
+  for (int c = 0; c < 6 && e == cudaSuccess; c++) {
+    const size_t cnt = c == 2 ? (size_t)n_probs * nn : nn;
+    if (hdst[c] && cnt) chk(cudaMemcpyAsync(hdst[c], outs[c], cnt * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H summaries");
+  }
+  chk(cudaStreamSynchronize(st), "sync");  // (before the buffer is freed, whatever failed)
+  return e == cudaSuccess ? 0 : 2;
+}
+
 
 // ------------------------------------------------------------------------------------------------------ predict_new
 // Posterior predictive draws at new rows from saved samples (DESIGN.md, "Prediction at new locations").  The new rows are

@@ -314,4 +314,12 @@ class Model {
   int* d_obs_widx = nullptr;
 };
 
+// ---- several chains (st_summarize_chains, st_summarize_draws; DESIGN.md §5d).  chains_check: K, S and probs as both
+// entry points refuse them (1), or K chains of S draws beyond one CTA's shared memory (4).  summarize_chains: src = K device
+// pointers (a host array), chain c's draw (s, i) at src[c][s * n + i]; runs on st and synchronises it; outputs as
+// st_chains_summary_out (NULL skipped, all NULL: the sizes only)
+int chains_check(const char* what, int K, int S, const double* probs, int n_probs, std::string& err);
+int summarize_chains(const double* const* src, int64_t n, int K, int S, const double* probs, int n_probs, st_chains_summary_out& out,
+                     cudaStream_t st, std::string& err);
+
 }  // namespace st
