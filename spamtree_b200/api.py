@@ -459,27 +459,21 @@ class SpamTreeMV:
         thf, bef, taf = [_f64(np.ravel(a, order="F")) for a in (th, be, ta)]
         zf = None if z is None else _f64(np.ravel(np.asarray(z, dtype=np.float64).reshape(nn, S), order="F"))
         ef = None if eps is None else _f64(np.ravel(np.asarray(eps, dtype=np.float64).reshape(nn, S), order="F"))
-        r = _lib.StNewRows()
-        r.n_new, r.coords, r.mv_id, r.X = nn, _dp(cm), _ip(mv), _dp(Xn)
-        r.n_groups, r.group, r.parents_ptr, r.parents_idx = pp.size - 1, _ip(grp), _ip(pp), _ip(pi)
         sm = _lib.StPredSamples()
         sm.n_samples, sm.theta, sm.beta, sm.tausq = S, _dp(thf), _dp(bef), _dp(taf)
         sm.w, sm.w_row_stride, sm.w_sample_stride = w.ctypes.data_as(_lib.c_double_p), rs, ss
         sm.z, sm.eps, sm.seed = _dp(zf), _dp(ef), int(seed)
-        res = {k: np.zeros(nn) for k in ("w_new_mean", "w_new_sd", "yhat_new_mean", "yhat_new_sd")}
-        dr = {k: np.zeros((S, nn)) for k in (("w_new", "yhat_new") if draws else ()) + (("mean", "sd") if moments else ())}
-        o = _lib.StPredOut()
-        o.w_new, o.y_new, o.mean, o.sd = [_dp(dr.get(k)) for k in ("w_new", "yhat_new", "mean", "sd")]
-        o.w_mean, o.w_sd, o.y_mean, o.y_sd = [_dp(res[k]) for k in ("w_new_mean", "w_new_sd", "yhat_new_mean", "yhat_new_sd")]
-        self._chk(lib.st_predict_new(self._h, C.byref(r), C.byref(sm), C.byref(o)))
-        res.update({k: v.T for k, v in dr.items()})  # n_new x S (column-major views of the ABI's layout)
-        res["n_builds"] = int(o.n_builds)
-        return res
+        return self._predict(cm, mv, Xn, grp, pp, pi, nn, S, draws, moments,
+                             lambda r, o: lib.st_predict_new(self._h, r, C.byref(sm), o))
 
     def _predict_new_stored(self, cm, mv, Xn, grp, pp, pi, nn, seed, draws, moments, z, eps, keep_draws):
         if z is not None or eps is not None:
             raise SpamTreeError(1, "z / eps need host samples: a prediction from the device store draws its normals on the device")
-        S = self._stored("w")[1]
+        return self._predict(cm, mv, Xn, grp, pp, pi, nn, self._stored("w")[1], draws, moments,
+                             lambda r, o: lib.st_predict_new_stored(self._h, r, int(seed), int(bool(keep_draws)), o))
+
+    def _predict(self, cm, mv, Xn, grp, pp, pi, nn, S, draws, moments, call):
+        """the new rows and the outputs of S samples for call(rows, out) -> status (st_predict_new or st_predict_new_stored)"""
         r = _lib.StNewRows()
         r.n_new, r.coords, r.mv_id, r.X = nn, _dp(cm), _ip(mv), _dp(Xn)
         r.n_groups, r.group, r.parents_ptr, r.parents_idx = pp.size - 1, _ip(grp), _ip(pp), _ip(pi)
@@ -488,8 +482,8 @@ class SpamTreeMV:
         o = _lib.StPredOut()
         o.w_new, o.y_new, o.mean, o.sd = [_dp(dr.get(k)) for k in ("w_new", "yhat_new", "mean", "sd")]
         o.w_mean, o.w_sd, o.y_mean, o.y_sd = [_dp(res[k]) for k in ("w_new_mean", "w_new_sd", "yhat_new_mean", "yhat_new_sd")]
-        self._chk(lib.st_predict_new_stored(self._h, C.byref(r), int(seed), int(bool(keep_draws)), C.byref(o)))
-        res.update({k: v.T for k, v in dr.items()})
+        self._chk(call(C.byref(r), C.byref(o)))
+        res.update({k: v.T for k, v in dr.items()})  # n_new x S (column-major views of the ABI's layout)
         res["n_builds"] = int(o.n_builds)
         return res
 

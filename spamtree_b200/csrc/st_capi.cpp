@@ -267,10 +267,9 @@ int st_summarize_chains(st_handle* const* hs, int32_t n_chains, int32_t which, c
   if (!out) { M0.err = "st_summarize_chains: out is NULL"; return ST_ERR_INVALID; }
   activate(h0);
   ST_GUARD_BEGIN
-  static const char* names[4] = {"w", "yhat", "w_new", "y_new"};
   if (which < 0 || which > 3) { M0.err = "st_summarize_chains: which must be 0 (w), 1 (yhat), 2 (w_new) or 3 (y_new)"; return ST_ERR_INVALID; }
-  const int64_t n = M0.store_[which].n;
-  const int S = M0.store_[which].S;
+  const int64_t n = M0.store.get(which).n;
+  const int S = M0.store.get(which).S;
   int rc = st::chains_check("st_summarize_chains", n_chains, std::max(S, 1), probs, n_probs, M0.err);
   if (rc) return rc;
   std::vector<const double*> src(n_chains);
@@ -278,22 +277,18 @@ int st_summarize_chains(st_handle* const* hs, int32_t n_chains, int32_t which, c
     const std::string hk = "st_summarize_chains: handle " + std::to_string(k);
     if (!hs[k]) { M0.err = hk + " is NULL"; return ST_ERR_INVALID; }
     const st::Model& Mk = hs[k]->model;
-    const st::Model::SampleStore& s = Mk.store_[which];
     if (Mk.device != M0.device) {
       M0.err = hk + " is on device " + std::to_string(Mk.device) + ", handle 0 on device " + std::to_string(M0.device);
       return ST_ERR_INVALID;
     }
-    if (!s.d || s.S < 1) {
-      M0.err = hk + " has no stored draws of " + names[which] +
-               (which < 2 ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)" : " (st_predict_new_stored with keep_draws)");
-      return ST_ERR_INVALID;
-    }
-    if (s.n != n || s.S != S) {
-      M0.err = hk + " stores " + std::to_string(s.S) + " draws of " + std::to_string(s.n) + " rows, handle 0 " + std::to_string(S) +
+    const st::DrawStore::Store* s = Mk.store.find(which, hk + " has ", M0.err);
+    if (!s) return ST_ERR_INVALID;
+    if (s->n != n || s->S != S) {
+      M0.err = hk + " stores " + std::to_string(s->S) + " draws of " + std::to_string(s->n) + " rows, handle 0 " + std::to_string(S) +
                " draws of " + std::to_string(n) + " rows";
       return ST_ERR_INVALID;
     }
-    src[k] = s.d;
+    src[k] = s->d;
   }
   for (int k = 1; k < n_chains; k++)  // every store is complete before the kernel reads it on hs[0]'s stream
     if (const cudaError_t e = cudaStreamSynchronize(hs[k]->model.stream)) {

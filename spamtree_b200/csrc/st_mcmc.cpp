@@ -63,8 +63,8 @@ int mcmc_run(Model& M, const st_mcmc_opts& o, st_mcmc_out& out) {
   // w of a saved iteration goes to the caller's buffer asynchronously (overlapping the next iteration) unless yhat, which
   // is formed on the host from w, is requested too
   const bool async_save = out.w_mcmc && !out.yhat_mcmc;
-  if (async_save) { rc = M.save_begin(out.w_mcmc, (size_t)o.keep * M.n_all * sizeof(double)); if (rc) return rc; }
-  struct SaveGuard { Model& M; bool on; ~SaveGuard() { if (on) M.save_end(); } } guard{M, async_save};
+  CopyOut co(M.stream, M.copy_stream, M.err);
+  if (async_save) { rc = co.open({out.w_mcmc}, (size_t)o.keep * M.n_all * sizeof(double), 1, M.n_all); if (rc) return rc; }
   // ST_PROFILE_MCMC=1: host wall-clock per phase of the loop, printed by every rank at the end (development aid)
   static const bool prof = getenv("ST_PROFILE_MCMC") != nullptr;
   double tph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -147,7 +147,7 @@ int mcmc_run(Model& M, const st_mcmc_opts& o, st_mcmc_out& out) {
       if (out.theta_mcmc)
         for (int j = 0; j < npar; j++) out.theta_mcmc[j + (size_t)msaved * npar] = M.theta[M.cur][j];
       const bool want_rows = (out.w_mcmc || out.yhat_mcmc) && !async_save;
-      if (async_save) { rc = M.save_w_async(out.w_mcmc + (size_t)msaved * M.n_all); if (rc) return rc; }
+      if (async_save) { rc = M.save_rows(co, 0, nullptr, out.w_mcmc + (size_t)msaved * M.n_all); if (rc) return rc; }
       if (want_rows) {
         wbuf.resize(M.n_all);
         rc = M.get_w(wbuf.data());
@@ -172,8 +172,9 @@ int mcmc_run(Model& M, const st_mcmc_opts& o, st_mcmc_out& out) {
     }
     lap(6, tl);
   }
-  if (async_save) { rc = M.save_sync(); if (rc) return rc; }  // the timed region ends when every saved w is on the host
-  out.mcmc_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();  // (the guard releases the page lock)
+  rc = co.finish();  // the timed region ends when every saved w is on the host
+  if (rc) return rc;
+  out.mcmc_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   if (prof)
     fprintf(stderr, "[mcmc profile] rank %d: %d iterations, %lld accepted; ms/iteration: gibbs %.3f llw %.3f build %.3f accept+adapt %.3f predict %.3f tausq+beta %.3f save %.3f | total %.3f\n",
             M.rank, mcmc, (long long)out.n_accepted, 1e3 * tph[0] / mcmc, 1e3 * tph[1] / mcmc, 1e3 * tph[2] / mcmc, 1e3 * tph[3] / mcmc,

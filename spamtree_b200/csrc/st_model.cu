@@ -81,17 +81,12 @@ Model::~Model() {
   cudaSetDevice(device);
   if (nccl_comm) { cudaStreamSynchronize(stream); nccl().CommDestroy(nccl_comm); nccl_comm = nullptr; }
   for (void* p : owned) cudaFree(p);
-  for (SampleStore& s : store_) s.release();
+  store.release();
   if (h_scalars) cudaFreeHost(h_scalars);
   if (h_mc) cudaFreeHost(h_mc);
   for (void* g : graph_exec_) if (g) cudaGraphExecDestroy((cudaGraphExec_t)g);
-  if (save_y_.ready) cudaEventDestroy(save_y_.ready);
-  if (save_y_.copied) cudaEventDestroy(save_y_.copied);
   if (h_stage) cudaFreeHost(h_stage);
   for (auto& e : ev) if (e) cudaEventDestroy(e);
-  if (save_registered) cudaHostUnregister(save_registered);
-  if (ev_wready) cudaEventDestroy(ev_wready);
-  if (ev_wcopied) cudaEventDestroy(ev_wcopied);
   if (copy_stream) cudaStreamDestroy(copy_stream);
   if (stream2) cudaStreamDestroy(stream2);
   if (stream3) cudaStreamDestroy(stream3);
@@ -621,6 +616,7 @@ int Model::upload(std::string& e) {
     ST_CUDA(cudaStreamCreateWithPriority(&stream, cudaStreamNonBlocking, hi), "cudaStreamCreate");
     ST_CUDA(cudaStreamCreateWithPriority(&stream2, cudaStreamNonBlocking, lo), "cudaStreamCreate");
     ST_CUDA(cudaStreamCreateWithPriority(&stream3, cudaStreamNonBlocking, lo), "cudaStreamCreate");
+    ST_CUDA(cudaStreamCreateWithFlags(&copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");  // saved rows (CopyOut)
   }
   ST_CUDA(cudaEventCreateWithFlags(&ev_prop, cudaEventDisableTiming), "cudaEventCreate");
   ST_CUDA(cudaEventCreateWithFlags(&ev_zfree, cudaEventDisableTiming), "cudaEventCreate");
@@ -739,6 +735,8 @@ int Model::upload(std::string& e) {
     const bool pg = part && !global_rows.empty();
     for (int64_t i = 0; i < n_all; i++) key[i] = pg ? (long long)global_rows[perm[i]] : (long long)perm[i];
     ST_CUDA(dev_upload(key, d_rowkey, owned), "upload rowkey");
+    std::vector<long long> ip(iperm.begin(), iperm.end());
+    ST_CUDA(dev_upload(ip, d_iperm, owned), "upload iperm");  // (un-permutes the saved rows)
   }
   ST_CUDA(dev_zeros(d_red_scratch, 2 * kReduceScratch, owned), "alloc reduce scratch");  // one set per stream
   ST_CUDA(dev_zeros(d_vrow, n_all, owned), "alloc vrow");
@@ -1258,60 +1256,76 @@ int Model::get_w(double* out) {
 }
 int Model::set_w(const double* in) { stats_valid_mode_ = -1; return upload_rows(in, d_w); }
 
-int Model::save_begin(double* host_base, size_t bytes) {
-  if (!stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
-  save_registered = nullptr;
-  save_pending = false;
-  if (!copy_stream) {
-    ST_CUDA(cudaStreamCreateWithFlags(&copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
-    ST_CUDA(cudaEventCreateWithFlags(&ev_wready, cudaEventDisableTiming), "cudaEventCreate");
-    ST_CUDA(cudaEventCreateWithFlags(&ev_wcopied, cudaEventDisableTiming), "cudaEventCreate");
-    ST_CUDA(dev_zeros(d_wsave, n_all, owned), "alloc wsave");
-    std::vector<long long> ip(iperm.begin(), iperm.end());
-    ST_CUDA(dev_upload(ip, d_iperm, owned), "upload iperm");
-  }
-  if (!host_base || bytes == 0) return 0;
-  // page-lock the caller's output range for the duration of the run; if that is refused the save stays synchronous
-  if (cudaHostRegister(host_base, bytes, cudaHostRegisterPortable) == cudaSuccess) save_registered = host_base;
-  else (void)cudaGetLastError();
-  return 0;
-}
-
-int Model::save_w_async(double* host_dst, double* dev_dst) {
-  if (!dev_dst && !save_registered) return get_w(host_dst);
-  // (a slot of the device store is written once: only the shared staging buffer waits for the copy before it)
-  if (!dev_dst && save_pending) ST_CUDA(cudaStreamWaitEvent(stream, ev_wcopied, 0), "wait for the previous save");  // d_wsave is reused
-  double* buf = dev_dst ? dev_dst : d_wsave;
-  ST_CUDA(launch_permute(d_w, buf, d_iperm, n_all, stream), "permute_kernel");
+int Model::save_rows(CopyOut& co, int k, double* dev, double* host) {
+  // (a slot of the device store is written once: only a staging slot waits for the copy that read it)
+  double* buf = dev ? dev : co.buffer(k);
+  if (!buf) return 2;
+  if (k == 0) ST_CUDA(launch_permute(d_w, buf, d_iperm, n_all, stream), "permute_kernel");
+  else ST_CUDA(launch_yhat(dt, d_w, d_xb, d_tausq_inv, d_iperm, d_rowkey, n_all, d_mc, buf, stream), "yhat_kernel");
   n_launches++;
-  if (!host_dst) return 0;
-  if (!save_registered) {
-    ST_CUDA(cudaMemcpyAsync(host_dst, buf, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H w");
-    ST_CUDA(cudaStreamSynchronize(stream), "sync");
-    return 0;
+  const double* src = buf;
+  return co.send(k, &host, &src, 1, n_all);
+}
+
+int CopyOut::chk(cudaError_t e, const char* what) {
+  if (e == cudaSuccess) return 0;
+  err_ = std::string("CUDA error in ") + what + ": " + cudaGetErrorString(e);
+  return 2;  // ST_ERR_CUDA
+}
+
+int CopyOut::open(std::initializer_list<double*> hosts, size_t bytes_each, int nslots, size_t n) {
+  n_ = n;
+  copied_.assign(nslots, nullptr);
+  pending_.assign(nslots, 0);
+  if (int rc = chk(cudaMalloc((void**)&staging_, std::max<size_t>(nslots * n, 1) * sizeof(double)), "alloc staging")) {
+    staging_ = nullptr;
+    return rc;
   }
-  ST_CUDA(cudaEventRecord(ev_wready, stream), "event");
-  ST_CUDA(cudaStreamWaitEvent(copy_stream, ev_wready, 0), "wait");
-  ST_CUDA(cudaMemcpyAsync(host_dst, buf, n_all * sizeof(double), cudaMemcpyDeviceToHost, copy_stream), "D2H w (async)");
-  ST_CUDA(cudaEventRecord(ev_wcopied, copy_stream), "event");
-  save_pending = true;
+  if (int rc = chk(cudaEventCreateWithFlags(&ready_, cudaEventDisableTiming), "cudaEventCreate")) return rc;
+  for (cudaEvent_t& e : copied_)
+    if (int rc = chk(cudaEventCreateWithFlags(&e, cudaEventDisableTiming), "cudaEventCreate")) return rc;
+  for (double* h : hosts) {
+    if (!h || bytes_each == 0) continue;
+    if (cudaHostRegister(h, bytes_each, cudaHostRegisterPortable) == cudaSuccess) locked_.push_back(h);
+    else (void)cudaGetLastError();  // (the copies still go there, see the class comment)
+  }
   return 0;
 }
 
-int Model::save_sync() {
-  int rc = 0;
-  if (copy_stream && save_pending) {
-    if (cudaStreamSynchronize(copy_stream) != cudaSuccess) { err = "asynchronous save of w failed"; rc = 2; }
-    save_pending = false;
-  }
-  return rc;
+double* CopyOut::buffer(int slot) {
+  if (pending_[slot] && chk(cudaStreamWaitEvent(st_, copied_[slot], 0), "wait for the copy of an earlier row")) return nullptr;
+  return staging_ + (size_t)slot * n_;
 }
 
-int Model::save_end() {
-  const int rc = save_sync();
-  if (save_registered) { cudaHostUnregister(save_registered); save_registered = nullptr; }
-  return rc;
+int CopyOut::send(int slot, double* const* dst, const double* const* src, int count, size_t n) {
+  if (std::none_of(dst, dst + count, [](double* d) { return d != nullptr; })) return 0;
+  if (int rc = chk(cudaEventRecord(ready_, st_), "event")) return rc;
+  if (int rc = chk(cudaStreamWaitEvent(cs_, ready_, 0), "wait")) return rc;
+  for (int c = 0; c < count; c++)
+    if (dst[c])
+      if (int rc = chk(cudaMemcpyAsync(dst[c], src[c], n * sizeof(double), cudaMemcpyDeviceToHost, cs_), "D2H rows")) return rc;
+  if (int rc = chk(cudaEventRecord(copied_[slot], cs_), "event")) return rc;
+  pending_[slot] = 1;
+  return 0;
 }
+
+int CopyOut::finish() {
+  if (!staging_) return 0;
+  std::fill(pending_.begin(), pending_.end(), 0);
+  return chk(cudaStreamSynchronize(cs_), "sync of the copies");
+}
+
+CopyOut::~CopyOut() {
+  if (staging_) {  // (an early exit may leave kernels that write the staging, or copies from it, in flight)
+    cudaStreamSynchronize(cs_);
+    cudaStreamSynchronize(st_);
+  }
+  for (void* p : locked_) cudaHostUnregister(p);
+  for (cudaEvent_t e : copied_) if (e) cudaEventDestroy(e);
+  if (ready_) cudaEventDestroy(ready_);
+  if (staging_) cudaFree(staging_);
+}
+
 int Model::get_xb(double* out) {
   if (!stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
   ST_CUDA(cudaMemcpyAsync(h_stage, d_xb, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H xb");
@@ -1829,17 +1843,6 @@ int Model::bench_iteration(const double* theta_prop, int do_swap, uint64_t seed,
   return 0;
 }
 
-// src (n_all doubles, boundary order, written by the kernel just enqueued on `stream`: S.dbuf or a slot of the device store)
-// -> host_dst on the copy stream
-int Model::save_rows_async(AsyncSave& S, double* host_dst, const double* src) {
-  ST_CUDA(cudaEventRecord(S.ready, stream), "event");
-  ST_CUDA(cudaStreamWaitEvent(copy_stream, S.ready, 0), "wait");
-  ST_CUDA(cudaMemcpyAsync(host_dst, src, n_all * sizeof(double), cudaMemcpyDeviceToHost, copy_stream), "D2H rows (async)");
-  ST_CUDA(cudaEventRecord(S.copied, copy_stream), "event");
-  S.pending = true;
-  return 0;
-}
-
 // The loop of spamtree_mv_mcmc (spamtree_fit.cpp:167-391) with the chain state in device memory: the host only enqueues
 // (one CUDA-graph launch per iteration on a single-GPU handle), saved iterations leave through asynchronous copies, and
 // the one synchronisation is at the end of the run.  Random numbers: Philox streams keyed by (seed, row or parameter,
@@ -1853,23 +1856,10 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   }
   // the device sample store (st_keep_samples_on_device): sized and checked before anything is allocated or launched, so that a
   // refused run leaves the handle as it was; a run replaces the last run's store
-  const bool store_w = (keep_mask & ST_KEEP_W) != 0, store_y = (keep_mask & ST_KEEP_YHAT) != 0;
   if (keep_mask) {
     if (part) { err = "st_mcmc_run: the device sample store is not supported on partitioned handles"; return 4; }
-    const size_t per = (size_t)n_all * (size_t)std::max(o.keep, 0) * sizeof(double);
-    int rc = check_store_fits((store_w ? per : 0) + (store_y ? per : 0), store_[0].cap + store_[1].cap, "st_mcmc_run");
+    const int rc = store.reserve(keep_mask, (size_t)n_all * (size_t)std::max(o.keep, 0) * sizeof(double), "st_mcmc_run", err);
     if (rc) return rc;
-    store_samp_.clear();
-    for (int k = 0; k < 2; k++) {
-      SampleStore& s = store_[k];
-      if (!(keep_mask & (1 << k))) { s.release(); continue; }
-      if (s.reserve(std::max<size_t>(per, 8)) != cudaSuccess) {
-        (void)cudaGetLastError();
-        s.release();
-        err = "st_mcmc_run: allocating " + std::to_string(per) + " bytes for the device sample store failed";
-        return 4;
-      }
-    }
   }
   double o3[3];
   int rc = get_loglik_comps_w(0, o3);  // spamtree_fit.cpp:110-111
@@ -1893,30 +1883,13 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   d_theta_mcmc = dsamp; d_beta_mcmc = dsamp + n_th; d_tausq_mcmc = dsamp + n_th + n_be;
   rc = push_chain_state(&o, o.seed);
   if (rc) return rc;
-  // saved rows: w through the existing staging (un-permute kernel), yhat through its own
-  const bool save_w = out.w_mcmc != nullptr, save_y = out.yhat_mcmc != nullptr;
-  if (save_w || save_y || store_w || store_y) {
-    rc = save_begin(save_w ? out.w_mcmc : nullptr, (size_t)keep * n_all * sizeof(double));
+  // saved rows: w (k = 0) and yhat (k = 1) into the device store and / or the caller's arrays
+  double* const host_rows[2] = {out.w_mcmc, out.yhat_mcmc};
+  CopyOut co(stream, copy_stream, err);
+  if (host_rows[0] || host_rows[1]) {
+    rc = co.open({host_rows[0], host_rows[1]}, (size_t)keep * n_all * sizeof(double), 2, n_all);
     if (rc) return rc;
   }
-  if (save_y) {
-    if (!save_y_.dbuf) {
-      ST_CUDA(dev_zeros(save_y_.dbuf, n_all, owned), "alloc yhat");
-      ST_CUDA(cudaEventCreateWithFlags(&save_y_.ready, cudaEventDisableTiming), "cudaEventCreate");
-      ST_CUDA(cudaEventCreateWithFlags(&save_y_.copied, cudaEventDisableTiming), "cudaEventCreate");
-    }
-    save_y_.pending = false;
-    save_y_.registered = (cudaHostRegister(out.yhat_mcmc, (size_t)keep * n_all * sizeof(double), cudaHostRegisterPortable) == cudaSuccess) ? out.yhat_mcmc : nullptr;
-    if (!save_y_.registered) (void)cudaGetLastError();
-  }
-  struct SaveGuard {
-    Model& M; bool on;
-    ~SaveGuard() {
-      if (!on) return;
-      M.save_end();
-      if (M.save_y_.registered) { cudaHostUnregister(M.save_y_.registered); M.save_y_.registered = nullptr; }
-    }
-  } guard{*this, save_w || save_y};
   // one CUDA graph per kind of iteration (with / without prediction); partitioned handles enqueue directly (their
   // collectives are library calls on the stream)
   static const bool no_graph = getenv("ST_GRAPH") && atoi(getenv("ST_GRAPH")) == 0;
@@ -1962,20 +1935,12 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
     }
     if (!launched) { rc = enqueue_iteration(o, predicting, 0, first, !last, saved ? keep : 0); if (rc) return rc; }
     if (saved) {  // :376-389
-      if (save_w || store_w) {
-        rc = save_w_async(save_w ? out.w_mcmc + (size_t)msaved * n_all : nullptr, store_w ? store_[0].d + (size_t)msaved * n_all : nullptr);
+      const size_t off = (size_t)msaved * n_all;
+      for (int k = 0; k < 2; k++) {
+        const bool kept = (keep_mask & (1 << k)) != 0;
+        if (!host_rows[k] && !kept) continue;
+        rc = save_rows(co, k, kept ? store.get(k).d + off : nullptr, host_rows[k] ? host_rows[k] + off : nullptr);
         if (rc) return rc;
-      }
-      if (save_y || store_y) {
-        double* ybuf = store_y ? store_[1].d + (size_t)msaved * n_all : save_y_.dbuf;
-        if (!store_y && save_y_.pending) ST_CUDA(cudaStreamWaitEvent(stream, save_y_.copied, 0), "wait for the previous save");
-        ST_CUDA(launch_yhat(dt, d_w, d_xb, d_tausq_inv, d_iperm, d_rowkey, n_all, d_mc, ybuf, stream), "yhat_kernel");
-        n_launches++;
-        if (save_y && save_y_.registered) { rc = save_rows_async(save_y_, out.yhat_mcmc + (size_t)msaved * n_all, ybuf); if (rc) return rc; }
-        else if (save_y) {
-          ST_CUDA(cudaMemcpyAsync(out.yhat_mcmc + (size_t)msaved * n_all, ybuf, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H yhat");
-          ST_CUDA(cudaStreamSynchronize(stream), "sync");
-        }
       }
       msaved++;
     }
@@ -1983,9 +1948,8 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   // the one synchronisation of the run: chain state, samples, the saves in flight
   rc = pull_chain_state();
   if (rc) return rc;
-  if (copy_stream) ST_CUDA(cudaStreamSynchronize(copy_stream), "sync saves");
-  save_pending = false;
-  save_y_.pending = false;
+  rc = co.finish();
+  if (rc) return rc;
   dvec hs(std::max<size_t>(n_th + n_be + n_ta, 1));
   ST_CUDA(cudaMemcpy(hs.data(), dsamp, (n_th + n_be + n_ta) * sizeof(double), cudaMemcpyDeviceToHost), "D2H samples");
   out.mcmc_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
@@ -1998,22 +1962,68 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   if (h_mc->gibbs_fail) { err = "Error at gibbs_sample_w: conditional precision not positive definite"; return 3; }
   if (h_mc->nan_loglik) { err = "At nan loglik: error."; return 5; }
   if (keep_mask && keep > 0) {  // the run completed: its store and the samples st_predict_new_stored predicts from
-    for (int k = 0; k < 2; k++)
-      if (keep_mask & (1 << k)) { store_[k].n = n_all; store_[k].S = keep; }
-    store_samp_.assign(hs.begin(), hs.begin() + (n_th + n_be + n_ta));
+    store.commit(keep_mask, n_all, keep);
+    store.samples.assign(hs.begin(), hs.begin() + (n_th + n_be + n_ta));
   }
   return 0;
 }
 
-int Model::check_store_fits(size_t need, size_t reusable, const char* what) {
+// ---- the device draw store
+int DrawStore::reserve(int mask, size_t bytes_each, const char* what, std::string& err) {
+  const int group = ((mask & kRun) ? kRun : 0) | ((mask & kPrediction) ? kPrediction : 0);
+  size_t need = 0, reusable = 0;
+  for (int k = 0; k < 4; k++) {
+    if (mask & (1 << k)) need += bytes_each;
+    if (group & (1 << k)) reusable += s_[k].cap;
+  }
   size_t fr = 0, tot = 0;
-  ST_CUDA(cudaMemGetInfo(&fr, &tot), "cudaMemGetInfo");
+  if (const cudaError_t e = cudaMemGetInfo(&fr, &tot)) { err = std::string("CUDA error in cudaMemGetInfo: ") + cudaGetErrorString(e); return 2; }
   if (need > fr + reusable) {
     err = std::string(what) + ": the device sample store needs " + std::to_string(need) + " bytes and " + std::to_string(fr + reusable) +
           " bytes of device memory are free";
     return 4;
   }
+  if (group & kRun) samples.clear();
+  const size_t bytes = std::max<size_t>(bytes_each, 8);
+  for (int k = 0; k < 4; k++) {
+    if (!(group & (1 << k))) continue;
+    Store& s = s_[k];
+    s.S = 0;
+    if (!(mask & (1 << k))) { if (s.d) cudaFree(s.d); s = Store(); continue; }
+    if (bytes <= s.cap) continue;
+    if (s.d) cudaFree(s.d);
+    s = Store();
+    if (cudaMalloc((void**)&s.d, bytes) != cudaSuccess) {
+      (void)cudaGetLastError();
+      s.d = nullptr;
+      err = std::string(what) + ": allocating " + std::to_string(bytes_each) + " bytes for the device sample store failed";
+      return 4;
+    }
+    s.cap = bytes;
+  }
   return 0;
+}
+
+void DrawStore::commit(int mask, int64_t n, int S) {
+  for (int k = 0; k < 4; k++)
+    if (mask & (1 << k)) { s_[k].n = n; s_[k].S = S; }
+}
+
+const DrawStore::Store* DrawStore::find(int which, const std::string& who, std::string& err) const {
+  static const char* names[4] = {"w", "yhat", "w_new", "y_new"};
+  const Store& s = s_[which];
+  if (s.d && s.S >= 1) return &s;
+  err = who + "no stored draws of " + names[which] +
+        (which < 2 ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)" : " (st_predict_new_stored with keep_draws)");
+  return nullptr;
+}
+
+void DrawStore::release() {
+  for (Store& s : s_) {
+    if (s.d) cudaFree(s.d);
+    s = Store();
+  }
+  samples.clear();
 }
 
 int Model::keep_samples_on_device(int what) {
@@ -2023,26 +2033,19 @@ int Model::keep_samples_on_device(int what) {
   keep_mask = what;
   if (what == 0) {
     if (stream) cudaStreamSynchronize(stream);
-    for (SampleStore& s : store_) s.release();
-    store_samp_.clear();
+    store.release();
   }
   return 0;
 }
 
 int Model::summarize(int which, const double* probs, int n_probs, st_summary_out& out) {
-  static const char* names[4] = {"w", "yhat", "w_new", "y_new"};
   if (which < 0 || which > 3) { err = "st_summarize: which must be 0 (w), 1 (yhat), 2 (w_new) or 3 (y_new)"; return 1; }
-  const SampleStore& s = store_[which];
   out.n_rows = 0;
   out.n_samples = 0;
-  if (!s.d || s.S < 1) {
-    err = std::string("st_summarize: no stored draws of ") + names[which] +
-          (which < 2 ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)" : " (st_predict_new_stored with keep_draws)");
-    return 1;
-  }
-  if (n_probs < 0 || (n_probs > 0 && !probs)) { err = "st_summarize: n_probs < 0, or probs missing"; return 1; }
-  for (int j = 0; j < n_probs; j++)
-    if (!(probs[j] >= 0.0 && probs[j] <= 1.0)) { err = "st_summarize: every prob must lie in [0, 1] (NaN is refused)"; return 1; }
+  const DrawStore::Store* sp = store.find(which, "st_summarize: ", err);
+  if (!sp) return 1;
+  const DrawStore::Store& s = *sp;
+  if (const int rc = probs_check("st_summarize", probs, n_probs, err)) return rc;
   const size_t cap = 227 * 1024;
   const int R = summary_rows_per_cta(s.S, cap);
   if (R < 1) {
@@ -2077,11 +2080,16 @@ int Model::summarize(int which, const double* probs, int n_probs, st_summary_out
 // ---- several chains (st_summarize_chains, st_summarize_draws; DESIGN.md §5d)
 static const size_t kChainsSmemCap = 227 * 1024;
 
-int chains_check(const char* what, int K, int S, const double* probs, int n_probs, std::string& err) {
-  if (K < 1 || S < 1) { err = std::string(what) + ": n_chains and n_samples must be at least 1"; return 1; }
+int probs_check(const char* what, const double* probs, int n_probs, std::string& err) {
   if (n_probs < 0 || (n_probs > 0 && !probs)) { err = std::string(what) + ": n_probs < 0, or probs missing"; return 1; }
   for (int j = 0; j < n_probs; j++)
     if (!(probs[j] >= 0.0 && probs[j] <= 1.0)) { err = std::string(what) + ": every prob must lie in [0, 1] (NaN is refused)"; return 1; }
+  return 0;
+}
+
+int chains_check(const char* what, int K, int S, const double* probs, int n_probs, std::string& err) {
+  if (K < 1 || S < 1) { err = std::string(what) + ": n_chains and n_samples must be at least 1"; return 1; }
+  if (const int rc = probs_check(what, probs, n_probs, err)) return rc;
   if (chains_rows_per_cta(K, S, kChainsSmemCap) < 1) {
     err = std::string(what) + ": " + std::to_string(K) + " chains of " + std::to_string(S) + " draws exceed what one CTA stages in "
           "shared memory (n_chains x (n_samples + 1) = " + std::to_string((long long)K * (S + 1)) + ", at most " +
@@ -2140,17 +2148,15 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
   out.n_builds = 0;
   const int npar = (int)theta[0].size();
   st_pred_samples PS = PS_in;
-  if (from_store) {
-    const int Ss = store_[0].S;
-    if (!store_[0].d || Ss < 1 || store_samp_.empty()) {
-      err = "st_predict_new_stored: the last device-resident run kept no w on the device (st_keep_samples_on_device with ST_KEEP_W)";
-      return 1;
-    }
+  if (from_store) {  // (a stored w comes with the run's samples: DrawStore::commit)
+    const DrawStore::Store* sw = store.find(0, "st_predict_new_stored: ", err);
+    if (!sw) return 1;
+    const int Ss = sw->S;
     PS.n_samples = Ss;
-    PS.theta = store_samp_.data();
+    PS.theta = store.samples.data();
     PS.beta = PS.theta + (size_t)npar * Ss;
     PS.tausq = PS.beta + (size_t)p * Ss * q;
-    PS.w = store_[0].d;  // (a device pointer: read by gather_sample_kernel only)
+    PS.w = sw->d;  // (a device pointer: read by gather_sample_kernel only)
     PS.w_row_stride = 1;
     PS.w_sample_stride = n_all;
     PS.z = PS.eps = nullptr;
@@ -2159,16 +2165,8 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
   const int S = PS.n_samples;
   if (nn < 0 || S < 0) { err = "predict_new: negative n_new or n_samples"; return 1; }
   if (keep_draws) {  // checked before anything is allocated; the previous prediction's store is replaced
-    const size_t per = (size_t)std::max<int64_t>(nn, 0) * S * sizeof(double);
-    const int rc = check_store_fits(2 * per, store_[2].cap + store_[3].cap, "st_predict_new_stored");
+    const int rc = store.reserve(DrawStore::kPrediction, (size_t)std::max<int64_t>(nn, 0) * S * sizeof(double), "st_predict_new_stored", err);
     if (rc) return rc;
-    for (int k = 2; k < 4; k++)
-      if (store_[k].reserve(std::max<size_t>(per, 8)) != cudaSuccess) {
-        (void)cudaGetLastError();
-        store_[k].release();
-        err = "st_predict_new_stored: allocating " + std::to_string(per) + " bytes for the device draw store failed";
-        return 4;
-      }
   }
   if (nn == 0 || S == 0) return 0;
   if (!R.coords || !R.mv_id || !R.group || !R.parents_ptr || R.n_groups < 1 || !PS.theta || !PS.beta || !PS.tausq || !PS.w) {
@@ -2260,16 +2258,7 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
   // ---- temporary device state (freed on every exit)
   struct Scratch {
     std::vector<void*> dev;
-    std::vector<void*> reg;
-    std::vector<cudaEvent_t> evs;
-    cudaStream_t cs = nullptr;
-    ~Scratch() {
-      if (cs) cudaStreamSynchronize(cs);
-      for (void* p : reg) cudaHostUnregister(p);
-      for (cudaEvent_t e : evs) cudaEventDestroy(e);
-      if (cs) cudaStreamDestroy(cs);
-      for (void* p : dev) cudaFree(p);
-    }
+    ~Scratch() { for (void* p : dev) cudaFree(p); }
   } X;
   auto dalloc = [&](void** p, size_t bytes) -> cudaError_t {
     cudaError_t e = cudaMalloc(p, std::max<size_t>(bytes, 8));
@@ -2337,8 +2326,9 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
     ST_CUDA(dalloc((void**)&d_Xn, (size_t)nn * p * sizeof(double)), "alloc");
     ST_CUDA(cudaMemcpyAsync(d_Xn, R.X, (size_t)nn * p * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D X_new");
   }
-  // samples of w staged in blocks of B (one 2D copy each), the node-ordered w_s, mean / sd, normals, two output slots
-  // (from the store: every sample is already on the device, one block of S)
+  // samples of w staged in blocks of B (one 2D copy each), the node-ordered w_s, mean / sd, normals (from the store: every
+  // sample is already on the device, one block of S); the draws of a sample go out from one of two staging slots of
+  // 4 n_new doubles (w_new | y_new | mean | sd) while the next sample runs
   const int B = from_store ? S : (int)std::max<int64_t>(1, std::min<int64_t>(S, (256LL << 20) / (8 * n_all)));
   double *d_wblk = nullptr, *d_wnode, *d_mean, *d_sd, *d_acc, *d_zn = nullptr, *d_en = nullptr;
   if (!from_store) ST_CUDA(dalloc((void**)&d_wblk, (size_t)B * n_all * sizeof(double)), "alloc");
@@ -2348,23 +2338,10 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
   ST_CUDA(dalloc((void**)&d_acc, 4 * nn * sizeof(double)), "alloc");
   if (PS.z) ST_CUDA(dalloc((void**)&d_zn, nn * sizeof(double)), "alloc");
   if (PS.eps) ST_CUDA(dalloc((void**)&d_en, nn * sizeof(double)), "alloc");
-  double* d_out[2][4];
-  for (int r = 0; r < 2; r++)
-    for (int c = 0; c < 4; c++) ST_CUDA(dalloc((void**)&d_out[r][c], nn * sizeof(double)), "alloc");
-  double* hout[4] = {out.w_new, out.y_new, out.mean, out.sd};
-  const bool any_draw_out = hout[0] || hout[1] || hout[2] || hout[3];
-  ST_CUDA(cudaStreamCreateWithFlags(&X.cs, cudaStreamNonBlocking), "cudaStreamCreate");
-  cudaEvent_t ready[2], copied[2];
-  for (int r = 0; r < 2; r++) {
-    ST_CUDA(cudaEventCreateWithFlags(&ready[r], cudaEventDisableTiming), "cudaEventCreate"); X.evs.push_back(ready[r]);
-    ST_CUDA(cudaEventCreateWithFlags(&copied[r], cudaEventDisableTiming), "cudaEventCreate"); X.evs.push_back(copied[r]);
-  }
-  bool pending[2] = {false, false};
-  for (double* hp : hout)  // page-locked for the duration of the call, so that the copies overlap the next sample
-    if (hp) {
-      if (cudaHostRegister(hp, (size_t)nn * S * sizeof(double), cudaHostRegisterPortable) == cudaSuccess) X.reg.push_back(hp);
-      else (void)cudaGetLastError();
-    }
+  double* const hout[4] = {out.w_new, out.y_new, out.mean, out.sd};
+  CopyOut co(stream, copy_stream, err);
+  int rc = co.open({hout[0], hout[1], hout[2], hout[3]}, (size_t)nn * S * sizeof(double), 2, 4 * (size_t)nn);
+  if (rc) return rc;
 
   int last_ref = 0;
   while (last_ref < (int)levels.size() && levels[last_ref].is_ref) last_ref++;
@@ -2374,7 +2351,7 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
   ST_CUDA(dalloc((void**)&d_bfail, (size_t)S * sizeof(int)), "alloc");
   const int alt = phys(1);
   int si = 1, sb = (int)n_all;
-  const double* wsrc = from_store ? store_[0].d : d_wblk;
+  const double* wsrc = from_store ? PS.w : d_wblk;
   for (int j = 0; j < S; j++) {
     if (!from_store && j % B == 0) {
       const int nb = std::min(B, S - j);
@@ -2398,7 +2375,7 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
       ST_CUDA(launch_chain_set_theta(d_mc, 1, pkk, stream), "chain_set_theta_kernel");
       deferred_[alt] = false;  // (from here on the slot holds the reference levels of this theta only)
       alter_scratch = true;
-      const int rc = launch_build_levels(1, 0, last_ref, true, stream);
+      rc = launch_build_levels(1, 0, last_ref, true, stream);
       if (rc) return rc;
       // the BUILD's failure count, kept per BUILD; the counter is the chain's and starts from zero again
       ST_CUDA(cudaMemcpyAsync(d_bfail + out.n_builds, d_fail, sizeof(int), cudaMemcpyDeviceToDevice, stream), "D2D fail");
@@ -2415,26 +2392,23 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
     if (d_zn) ST_CUDA(cudaMemcpyAsync(d_zn, PS.z + (size_t)j * nn, nn * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D z");
     if (d_en) ST_CUDA(cudaMemcpyAsync(d_en, PS.eps + (size_t)j * nn, nn * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D eps");
     const int r = j & 1;
-    if (pending[r]) ST_CUDA(cudaStreamWaitEvent(stream, copied[r], 0), "wait for the copy of an earlier sample");
+    double* stage = co.buffer(r);
+    if (!stage) return 2;
     PredDrawPack pack{};
     for (int jq = 0; jq < q; jq++) {
       for (int a = 0; a < p; a++) pack.beta[a + jq * p] = PS.beta[a + (size_t)j * p + (size_t)jq * p * S];
       pack.sdtau[jq] = std::sqrt(PS.tausq[jq + (size_t)j * q]);
     }
-    double* dsrc[4] = {keep_draws ? store_[2].d + (size_t)j * nn : d_out[r][0], keep_draws ? store_[3].d + (size_t)j * nn : d_out[r][1],
-                       d_out[r][2], d_out[r][3]};
+    double* dsrc[4] = {keep_draws ? store.get(2).d + (size_t)j * nn : stage, keep_draws ? store.get(3).d + (size_t)j * nn : stage + nn,
+                       stage + 2 * nn, stage + 3 * nn};
     ST_CUDA(launch_predict_draw(nn, d_lay2row, d_cmvq, d_Xn, p, d_mean, d_sd, pack, PS.seed, j, d_zn, d_en, dsrc[0], dsrc[1],
                                 dsrc[2], dsrc[3], d_acc, stream),
             "predict_draw_kernel");
     n_launches += 2 + (double)launches.size();
-    if (any_draw_out) {
-      ST_CUDA(cudaEventRecord(ready[r], stream), "event");
-      ST_CUDA(cudaStreamWaitEvent(X.cs, ready[r], 0), "wait");
-      for (int c = 0; c < 4; c++)
-        if (hout[c]) ST_CUDA(cudaMemcpyAsync(hout[c] + (size_t)j * nn, dsrc[c], nn * sizeof(double), cudaMemcpyDeviceToHost, X.cs), "D2H draws");
-      ST_CUDA(cudaEventRecord(copied[r], X.cs), "event");
-      pending[r] = true;
-    }
+    double* hdst[4];
+    for (int c = 0; c < 4; c++) hdst[c] = hout[c] ? hout[c] + (size_t)j * nn : nullptr;
+    rc = co.send(r, hdst, dsrc, 4, nn);
+    if (rc) return rc;
   }
   double* hm[4] = {out.w_mean, out.w_sd, out.y_mean, out.y_sd};
   if (hm[0] || hm[1] || hm[2] || hm[3]) {
@@ -2448,7 +2422,8 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
   ST_CUDA(cudaMemcpyAsync(bfail.data(), d_bfail, bfail.size() * sizeof(int), cudaMemcpyDeviceToHost, stream), "D2H fail");
   // the one synchronisation
   ST_CUDA(cudaStreamSynchronize(stream), "sync");
-  ST_CUDA(cudaStreamSynchronize(X.cs), "sync copies");
+  rc = co.finish();
+  if (rc) return rc;
   // a theta whose covariance is not positive definite on some reference block: the chain would have rejected it, and its
   // draws are not draws of the model (the factor rows of that block are zeroed)
   for (int j = 0; j < S; j++)
@@ -2456,8 +2431,7 @@ int Model::predict_new(const st_new_rows& R, const st_pred_samples& PS_in, st_pr
       err = "predict_new: theta of sample " + std::to_string(j) + ": a reference-level Cholesky factorisation failed (covariance not positive definite)";
       return 3;
     }
-  if (keep_draws)
-    for (int k = 2; k < 4; k++) { store_[k].n = nn; store_[k].S = S; }
+  if (keep_draws) store.commit(DrawStore::kPrediction, nn, S);
   return 0;
 }
 

@@ -11,7 +11,9 @@
 #include <cuda_runtime.h>
 
 #include <functional>
+#include <initializer_list>
 #include <string>
+#include <vector>
 
 #include "../../include/spamtree_b200.h"
 #include "st_chain.hpp"
@@ -93,6 +95,71 @@ struct LevelInfo {
 };
 
 struct GroupSpec { int s, nn, NT; };  // a BUILD work group: nn sibling blocks from slot s, NT tiles of 8 columns
+
+// Rows a kernel writes on `stream` go to slices of the caller's host arrays on the copy stream, while the work enqueued
+// after them runs (DESIGN.md §5).  One per run or call: open() page-locks the caller's ranges where it can and allocates
+// the staging slots, buffer() hands out a slot once the last copy that read it is done (a wait of the stream, not of the
+// host), send() issues the copies, finish() waits for all of them.  A range that cannot be page-locked (pageable memory
+// the driver refuses, or memory that is page-locked already) takes the same copies: into pageable memory a device-to-host
+// copy returns only once it is complete, so only when a copy runs can change, never what arrives.  Status: 0, or
+// ST_ERR_CUDA with `err` set.
+class CopyOut {
+ public:
+  CopyOut(cudaStream_t stream, cudaStream_t copy_stream, std::string& err) : st_(stream), cs_(copy_stream), err_(err) {}
+  ~CopyOut();  // waits for both streams, unlocks the ranges, frees the staging
+  CopyOut(const CopyOut&) = delete;
+  CopyOut& operator=(const CopyOut&) = delete;
+  // hosts: the caller's arrays (NULL skipped), bytes_each bytes from each; nslots staging slots of n doubles
+  int open(std::initializer_list<double*> hosts, size_t bytes_each, int nslots, size_t n);
+  double* buffer(int slot);  // NULL on a CUDA error
+  // dst[c] <- src[c], n doubles each (NULL dst skipped), once what `stream` holds so far has run; `slot`: the staging slot
+  // the sources are in, whose next buffer() waits for these copies
+  int send(int slot, double* const* dst, const double* const* src, int count, size_t n);
+  int finish();
+
+ private:
+  int chk(cudaError_t e, const char* what);
+  cudaStream_t st_, cs_;
+  std::string& err_;
+  std::vector<void*> locked_;
+  double* staging_ = nullptr;
+  size_t n_ = 0;
+  cudaEvent_t ready_ = nullptr;
+  std::vector<cudaEvent_t> copied_;  // per slot
+  std::vector<char> pending_;
+};
+
+// Draws kept on the device (st_keep_samples_on_device, st_predict_new_stored, st_summarize; DESIGN.md §5c), the only code
+// that knows the stores' layout.  Store k holds [sample][row] draws, n rows x S samples: w (0) and yhat (1) of the last
+// device-resident run, w_new (2) and y_new (3) of the last stored prediction.  A mask selects store k by bit k (ST_KEEP_W,
+// ST_KEEP_YHAT for the first two).
+class DrawStore {
+ public:
+  static constexpr int kRun = 3, kPrediction = 12;  // what a run, a stored prediction replaces
+  struct Store {
+    double* d = nullptr;
+    size_t cap = 0;  // bytes allocated (reused by the next run when large enough)
+    int64_t n = 0;
+    int S = 0;       // 0: holds nothing
+  };
+  DrawStore() = default;
+  DrawStore(const DrawStore&) = delete;
+  DrawStore& operator=(const DrawStore&) = delete;
+  ~DrawStore() { release(); }
+  // empties the stores of the groups (kRun, kPrediction) that `mask` touches, makes room for bytes_each bytes in each
+  // store of `mask` and frees the group's others.  Refused (ST_ERR_UNSUPPORTED) when that does not fit the free device
+  // memory plus what those stores hold already: then every store is as it was
+  int reserve(int mask, size_t bytes_each, const char* what, std::string& err);
+  void commit(int mask, int64_t n, int S);  // a completed run or prediction wrote S draws of n rows into each store of mask
+  const Store& get(int which) const { return s_[which]; }
+  // the store, or NULL and err = who + "no stored draws of <name> (<how to keep them>)"
+  const Store* find(int which, const std::string& who, std::string& err) const;
+  void release();
+  dvec samples;  // theta (npar x S), beta (p x S x q), tausq (q x S) of the last stored run
+
+ private:
+  Store s_[4];
+};
 
 class Model {
  public:
@@ -204,11 +271,7 @@ class Model {
   bool llw_overlap = false;
   bool overlap = true;              // ST_OVERLAP=0 disables
   int n_early_levels_ = 0;          // leading tree levels whose BUILD runs underneath the sweep (ST_EARLY_LEVELS overrides)
-  cudaEvent_t ev_wready = nullptr, ev_wcopied = nullptr;
-  double* d_wsave = nullptr;        // w in boundary order (staging of the asynchronous save)
   long long* d_iperm = nullptr;     // boundary row -> node-major row
-  void* save_registered = nullptr;  // host range page-locked by save_begin
-  bool save_pending = false;
   cudaEvent_t ev[14]{};
   std::vector<void*> owned;  // device allocations to free
   // counters
@@ -227,12 +290,10 @@ class Model {
   int gibbs_sample_beta(const double* zb, bool faithful_index);  // :1364-1391
   int gibbs_sample_tausq(const double* fixed);         // :1393-1417
   int get_w(double* out);
-  // saved iterations: un-permute w on the device and copy it to `host_dst` (page-locked by save_begin) on a second
-  // stream, so that the copy overlaps the next iteration; save_end waits for the copies in flight
-  int save_begin(double* host_base, size_t bytes);
-  int save_sync();  // waits for the copies in flight (every saved w is on the host); save_end also releases the page lock
-  int save_w_async(double* host_dst, double* dev_dst = nullptr);  // dev_dst: a slot of the device store (then host_dst may be NULL)
-  int save_end();
+  // a saved iteration's w (k = 0, un-permuted) or yhat (k = 1, device-resident chain only), in boundary order: written on
+  // `stream` into `dev` (a slot of the device store) or, when dev is NULL, into co's staging slot k, then copied to `host`
+  // (NULL: none) on the copy stream
+  int save_rows(CopyOut& co, int k, double* dev, double* host);
   int set_w(const double* in);
   int get_xb(double* out);
   int set_tausq_inv(const double* t);
@@ -251,24 +312,7 @@ class Model {
   int keep_samples_on_device(int what);
   int summarize(int which, const double* probs, int n_probs, st_summary_out& out);
   int keep_mask = 0;                   // ST_KEEP_W | ST_KEEP_YHAT for the following device-resident runs
-  struct SampleStore {                 // [sample][row] draws of one quantity, n rows x S samples
-    double* d = nullptr;
-    size_t cap = 0;                    // bytes allocated (reused by the next run when large enough)
-    int64_t n = 0;
-    int S = 0;                         // 0: holds nothing
-    void release() { if (d) cudaFree(d); d = nullptr; cap = 0; n = 0; S = 0; }
-    cudaError_t reserve(size_t bytes) {
-      S = 0;
-      if (bytes <= cap) return cudaSuccess;
-      release();
-      const cudaError_t e = cudaMalloc((void**)&d, bytes);
-      if (e == cudaSuccess) cap = bytes; else d = nullptr;
-      return e;
-    }
-  };
-  SampleStore store_[4];               // w, yhat of the last run; w_new, y_new of the last stored prediction
-  dvec store_samp_;                    // theta (npar x S), beta (p x S x q), tausq (q x S) of the last stored run
-  int check_store_fits(size_t need, size_t reusable, const char* what);
+  DrawStore store;
 
  private:
   int phys(int slot) const { return slot ? 1 - cur : cur; }
@@ -287,16 +331,6 @@ class Model {
   int push_chain_state(const st_mcmc_opts* o, uint64_t seed);
   int pull_chain_state();
   cudaEvent_t* timing_events_ = nullptr;
-  // asynchronous saves of a device-resident run: a row vector in boundary order goes from its device staging buffer to
-  // the caller's (page-locked) array on the copy stream while the next iteration runs
-  struct AsyncSave {
-    double* dbuf = nullptr;
-    cudaEvent_t ready = nullptr, copied = nullptr;
-    void* registered = nullptr;
-    bool pending = false;
-  };
-  AsyncSave save_y_;
-  int save_rows_async(AsyncSave& S, double* host_dst, const double* src);
   bool deferred_[2] = {false, false};
   int refresh_grams(const int* run_flag = nullptr, cudaStream_t st = nullptr);
   int gibbs_launch_only(int* fail_ptr);
@@ -317,7 +351,8 @@ class Model {
 // ---- several chains (st_summarize_chains, st_summarize_draws; DESIGN.md §5d).  chains_check: K, S and probs as both
 // entry points refuse them (1), or K chains of S draws beyond one CTA's shared memory (4).  summarize_chains: src = K device
 // pointers (a host array), chain c's draw (s, i) at src[c][s * n + i]; runs on st and synchronises it; outputs as
-// st_chains_summary_out (NULL skipped, all NULL: the sizes only)
+// st_chains_summary_out (NULL skipped, all NULL: the sizes only).  probs_check: n_probs >= 0 probabilities in [0, 1] (1)
+int probs_check(const char* what, const double* probs, int n_probs, std::string& err);
 int chains_check(const char* what, int K, int S, const double* probs, int n_probs, std::string& err);
 int summarize_chains(const double* const* src, int64_t n, int K, int S, const double* probs, int n_probs, st_chains_summary_out& out,
                      cudaStream_t st, std::string& err);

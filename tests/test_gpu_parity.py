@@ -279,7 +279,7 @@ def test_deferred_backward_half_of_childless_levels():
 
 def test_asynchronous_save_of_w_equals_the_synchronous_one():
     """saved iterations without yhat copy w to the caller's buffer on a second stream while the next iteration runs
-    (st_model.cu: save_w_async); the saved draws must be the very same numbers as with the synchronous path"""
+    (st_model.cu: Model::save_rows, CopyOut); the saved draws must be the very same numbers as with the synchronous path"""
     from spamtree_b200 import synth
     pb = common.make_problem(3, 4000)
     npar = pb["theta"].size
