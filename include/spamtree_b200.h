@@ -289,6 +289,52 @@ int st_summarize_chains(st_handle* const* hs, int32_t n_chains, int32_t which, c
 int st_summarize_draws(int32_t device, const double* draws, int64_t n_rows, int32_t n_chains, int32_t n_samples,
                        const double* probs, int32_t n_probs, st_chains_summary_out* out);
 
+/* ---- model criteria: PSIS-LOO with Pareto k-hat, WAIC and DIC per observation (no reference counterpart; DESIGN.md §5e) ----
+ * K chains x S saved iterations, N = K S pooled draws g = c S + s.  For an observed row i (finite y_i; rows in boundary order,
+ * as w_mcmc) with outcome j = mv_id_i, the log-likelihood conditional on w:
+ *   ll[i,g] = -0.5 log(2 pi tausq[j,g]) - (y_i - x_i' beta[:,j,g] - w[i,g])^2 / (2 tausq[j,g])
+ * (beta p x S x q and tausq q x S as st_mcmc_out holds them; tausq is tau^2).  Rows with a missing y are NaN in every per-row
+ * output and are left out of every total; n_obs counts the observed rows.  Per row, LSE = log-sum-exp:
+ *   lpd = LSE_g(ll) - log N;  p_waic = var_g(ll) (ddof 1, NaN for N = 1);  elpd_waic = lpd - p_waic   (R loo::waic)
+ *   PSIS-LOO (R loo 2.x psis(), gpdfit with wip = TRUE, min_grid_pts = 30, prior 3): lw = r - max(r) with r = -ll;
+ *   L = tail_len = min(ceil(0.2 N), ceil(3 sqrt(N / r_eff))), k-hat = +Inf; if L >= 5 the largest L sorted lw form the tail
+ *   and the sorted value before them the cutoff; unless the tail is constant (max - min < DBL_EPSILON / 100), a generalised
+ *   Pareto distribution is fitted to x = exp(tail) - exp(cutoff) (Zhang and Stephens 2009, M = 30 + floor(sqrt(L)) grid
+ *   points, k-hat = (L k + 5) / (L + 10), NaN becomes +Inf), and for finite k-hat the tail is replaced by
+ *   log(sigma expm1(-k-hat log1p(-p_m)) / k-hat + exp(cutoff)), p_m = (m - 0.5) / L; lw is truncated at 0 and normalised;
+ *   elpd_loo = LSE_g(lw + ll), p_loo = lpd - elpd_loo.
+ *   DIC (Spiegelhalter et al. 2002, plug-in at the pooled posterior means as spBayes' spDiag): dbar = sum_i -2 mean_g ll,
+ *   dhat = sum_i -2 log N(y_i; x_i' mean(beta[:,j]) + mean(w_i), mean(tausq_j)), p_dic = dbar - dhat, dic = dbar + p_dic.
+ * Totals over the observed rows: elpd_loo_total = sum, se_elpd_loo = sqrt(n_obs var(elpd_loo_i, ddof 1)), looic = -2
+ * elpd_loo_total, se_looic = 2 se_elpd_loo; the same for WAIC; lpd_total; k_threshold = min(1 - 1 / log10(N), 0.7);
+ * n_k_high = rows with k-hat > k_threshold (+Inf included); n_p_waic_high = rows with p_waic > 0.4.
+ * The criteria condition on w, one latent value per observation, so w_i is informed mostly by y_i itself and PSIS-LOO of such
+ * a model often shows k-hat > 0.7 on many rows (Vehtari, Mononen, Tolvanen, Sivula and Winther 2016): n_k_high says how far
+ * elpd_loo can be trusted.  Every reduction runs in a fixed order: repeated calls are bit-identical.
+ * Refused: r_eff <= 0 or not finite, n_chains < 1, n_samples < 1 (ST_ERR_INVALID); N above what one CTA stages in shared
+ * memory (ST_ERR_UNSUPPORTED, the limit in the message). */
+typedef struct {                 /* caller-allocated; NULL pointers skipped; all NULL: only the sizes (n_rows, n_obs, n_chains,
+                                    n_samples, k_threshold) are returned and the other totals are NaN */
+  double *lpd, *elpd_loo, *p_loo, *pareto_k, *elpd_waic, *p_waic;   /* n_rows each, NaN at unobserved rows */
+  double elpd_loo_total, se_elpd_loo, p_loo_total, looic, se_looic;  /* out */
+  double elpd_waic_total, se_elpd_waic, p_waic_total, waic, se_waic, lpd_total;
+  double dbar, dhat, p_dic, dic, k_threshold;
+  int64_t n_rows, n_obs, n_k_high, n_p_waic_high;                    /* out */
+  int32_t n_chains, n_samples;                                      /* out */
+} st_fit_criteria_out;
+/* The w stores of n_chains handles read in place, with the beta / tausq samples of the same stored runs and the handles' y,
+ * X and mv_id.  Every handle must be on the same device, store the same n_rows and S, and have the same p, q, y, X and mv_id,
+ * else ST_ERR_INVALID naming the first handle that differs; a handle without a w store gives ST_ERR_INVALID.  Waits for every
+ * handle's stream, runs on that of hs[0] and returns when done; changes no handle's state.  Errors: st_last_error(hs[0]);
+ * st_last_error(NULL) when there is no handle to report to. */
+int st_fit_criteria(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit_criteria_out* out);
+/* The PSIS / WAIC part on a host log-likelihood [chain][sample][row] (n_chains x n_samples x n_rows), copied to `device` for
+ * the call: a row of NaN is an unobserved row; any other non-finite value is refused (ST_ERR_INVALID).  The DIC fields are NaN
+ * (no parameters are given).  ST_ERR_UNSUPPORTED when the copy does not fit in the free device memory.  Errors:
+ * st_last_error(NULL). */
+int st_fit_criteria_loglik(int32_t device, const double* loglik, int64_t n_rows, int32_t n_chains, int32_t n_samples,
+                           double r_eff, st_fit_criteria_out* out);
+
 /* ---- the Metropolis-Hastings glue (mh_adapt.h / mh_adapt.cpp), as st_mcmc_run uses it; host-only, no handle ---- */
 /* par_huvtransf_fwd / par_huvtransf_back (Rcpp exports), mh_adapt.cpp:3-15: logit / logistic on (bounds[j], bounds[j + npar]).
  * bounds: npar x 2. */

@@ -112,6 +112,19 @@ class StChainsSummaryOut(C.Structure):
     ]
 
 
+class StFitCriteriaOut(C.Structure):
+    _fields_ = [
+        ("lpd", c_double_p), ("elpd_loo", c_double_p), ("p_loo", c_double_p), ("pareto_k", c_double_p),
+        ("elpd_waic", c_double_p), ("p_waic", c_double_p),
+        ("elpd_loo_total", C.c_double), ("se_elpd_loo", C.c_double), ("p_loo_total", C.c_double), ("looic", C.c_double),
+        ("se_looic", C.c_double), ("elpd_waic_total", C.c_double), ("se_elpd_waic", C.c_double), ("p_waic_total", C.c_double),
+        ("waic", C.c_double), ("se_waic", C.c_double), ("lpd_total", C.c_double),
+        ("dbar", C.c_double), ("dhat", C.c_double), ("p_dic", C.c_double), ("dic", C.c_double), ("k_threshold", C.c_double),
+        ("n_rows", C.c_int64), ("n_obs", C.c_int64), ("n_k_high", C.c_int64), ("n_p_waic_high", C.c_int64),
+        ("n_chains", C.c_int32), ("n_samples", C.c_int32),
+    ]
+
+
 ST_KEEP_W, ST_KEEP_YHAT = 1, 2
 
 
@@ -145,6 +158,9 @@ SIGNATURES = {
                                       C.POINTER(StChainsSummaryOut)]),
     "st_summarize_draws": (C.c_int, [C.c_int32, c_double_p, C.c_int64, C.c_int32, C.c_int32, c_double_p, C.c_int32,
                                      C.POINTER(StChainsSummaryOut)]),
+    "st_fit_criteria": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_double, C.POINTER(StFitCriteriaOut)]),
+    "st_fit_criteria_loglik": (C.c_int, [C.c_int32, c_double_p, C.c_int64, C.c_int32, C.c_int32, C.c_double,
+                                         C.POINTER(StFitCriteriaOut)]),
     "st_bench_iteration": (C.c_int, [C.c_void_p, c_double_p, C.c_int, C.c_uint64, c_double_p, c_float_p]),
     "st_set_beta_index": (C.c_int, [C.c_void_p, C.c_int]),
     "st_get_counters": (C.c_int, [C.c_void_p, c_double_p]),

@@ -516,6 +516,17 @@ class SpamTreeMV:
         res["probs"] = pr.copy()
         return res
 
+    def fit_criteria(self, r_eff=1.0):
+        """PSIS-LOO (with Pareto k-hat), WAIC and DIC per observation of the last run with device_samples including "w"
+        (st_fit_criteria), from the draws of w kept on the device and that run's beta / tausq samples.  The log-likelihood is
+        conditional on w: ll[i, s] = log N(y_i; x_i' beta_s[:, j] + w[i, s], tausq_s[j]), j the row's outcome.  Returns the
+        per-row arrays "lpd", "elpd_loo", "p_loo", "pareto_k", "elpd_waic", "p_waic" (rows in boundary order, NaN where y is
+        missing) and the totals of fit_criteria_loglik.
+
+        With one latent w_i per observation, w_i is informed mostly by y_i itself, so PSIS-LOO of this model often shows
+        k-hat > 0.7 on many rows (Vehtari et al. 2016): check "n_k_high" before relying on "elpd_loo"."""
+        return _criteria([self], r_eff)
+
     def bench_iteration(self, theta_prop, do_swap=False, seed=0):
         t, o, ms = _f64(theta_prop), np.zeros(3), np.zeros(6, dtype=np.float32)
         self._chk(lib.st_bench_iteration(self._h, _dp(t), int(bool(do_swap)), int(seed), _dp(o), ms.ctypes.data_as(_lib.c_float_p)))
@@ -637,6 +648,90 @@ def summarize_draws(draws, probs=(0.025, 0.5, 0.975), device=0):
     return _chains_result(call, probs)
 
 
+# --------------------------------------------------------------------------------------------- model criteria (§5e)
+_CRIT_ROWS = ("lpd", "elpd_loo", "p_loo", "pareto_k", "elpd_waic", "p_waic")
+_CRIT_TOTALS = ("elpd_loo_total", "se_elpd_loo", "p_loo_total", "looic", "se_looic", "elpd_waic_total", "se_elpd_waic",
+                "p_waic_total", "waic", "se_waic", "lpd_total", "dbar", "dhat", "p_dic", "dic", "k_threshold")
+_CRIT_COUNTS = ("n_rows", "n_obs", "n_k_high", "n_p_waic_high", "n_chains", "n_samples")
+
+
+def _criteria_result(call):
+    """call(StFitCriteriaOut) -> None (raising on a refusal), made twice: for the sizes, then for the outputs"""
+    o = _lib.StFitCriteriaOut()
+    call(o)
+    n = int(o.n_rows)
+    res = {k: np.zeros(n) for k in _CRIT_ROWS}
+    for k in _CRIT_ROWS:
+        setattr(o, k, _dp(res[k]))
+    call(o)
+    res.update({k: float(getattr(o, k)) for k in _CRIT_TOTALS})
+    res.update({k: int(getattr(o, k)) for k in _CRIT_COUNTS})
+    return res
+
+
+def fit_criteria(models, r_eff=1.0):
+    """PSIS-LOO, WAIC and DIC of the draws several chains of the same model keep on the device (st_fit_criteria): the w
+    store of each model's last run with device_samples including "w", with that run's beta / tausq samples, pooled over
+    the chains.  The models must be fits of the same data (y, X and mv_id are compared) with the same number of draws.
+
+    Per row (rows in boundary order; NaN where y is missing): "lpd", "elpd_loo", "p_loo", "pareto_k" (the Pareto k-hat of
+    PSIS, +inf when the tail is too short or constant), "elpd_waic", "p_waic" (ddof 1).  Totals over the observed rows:
+    "elpd_loo_total", "se_elpd_loo", "p_loo_total", "looic", "se_looic", the same for WAIC, "lpd_total", DIC at the
+    posterior means ("dbar", "dhat", "p_dic", "dic"), "k_threshold" (min(1 - 1 / log10(N), 0.7)), "n_k_high" (rows with
+    k-hat above it), "n_p_waic_high" (rows with p_waic > 0.4), and "n_rows", "n_obs", "n_chains", "n_samples".  As R's loo
+    package with one scalar r_eff (default 1) and gpdfit's weakly informative prior; DESIGN.md §5e has the definitions.
+
+    The log-likelihood is conditional on w, one latent value per observation, so w_i is informed mostly by y_i itself and
+    PSIS-LOO often shows k-hat > 0.7 on many rows (Vehtari, Mononen, Tolvanen, Sivula and Winther 2016): "n_k_high" says
+    how far "elpd_loo" can be trusted.  Compare two fits of the same data with loo_compare."""
+    return _criteria(models, r_eff)
+
+
+def _criteria(models, r_eff):
+    models = list(models)
+    if not models:
+        raise SpamTreeError(1, "fit_criteria: no models")
+    hs = (C.c_void_p * len(models))(*[m._h for m in models])
+
+    def call(o):
+        models[0]._chk(lib.st_fit_criteria(hs, len(models), float(r_eff), C.byref(o)))
+    return _criteria_result(call)
+
+
+def fit_criteria_loglik(loglik, r_eff=1.0, device=0):
+    """The PSIS-LOO and WAIC part of fit_criteria on a log-likelihood the caller brings (st_fit_criteria_loglik): loglik
+    (n_chains, n_samples, n_rows) or (n_samples, n_rows), copied to the GPU for the call.  A row of NaN is an unobserved
+    row; any other NaN or infinite value is refused (SpamTreeError code 1).  The DIC totals are NaN."""
+    d = np.asarray(loglik, dtype=np.float64)
+    if d.ndim == 2:
+        d = d[None]
+    if d.ndim != 3:
+        raise SpamTreeError(1, "fit_criteria_loglik: loglik must be (n_chains, n_samples, n_rows) or (n_samples, n_rows)")
+    d = _f64(d)
+    K, S, n = d.shape
+
+    def call(o):
+        rc = lib.st_fit_criteria_loglik(int(device), _dp(d), n, K, S, float(r_eff), C.byref(o))
+        if rc:
+            raise SpamTreeError(rc, lib.st_last_error(None).decode())
+    return _criteria_result(call)
+
+
+def loo_compare(a, b, criterion="elpd_loo"):
+    """Difference of two fits of the same rows (results of fit_criteria / fit_criteria_loglik, or SpamTreeMV.fit_criteria):
+    "elpd_diff" = sum_i (a_i - b_i) of the per-row criterion ("elpd_loo" or "elpd_waic") over the rows observed in both,
+    "se_diff" = sqrt(n var(a_i - b_i, ddof 1)) and "n".  Positive: a predicts better.  spamtree() orders rows by their
+    coordinates alone, so two of its fits of the same data share the row order."""
+    if criterion not in ("elpd_loo", "elpd_waic"):
+        raise SpamTreeError(1, "loo_compare: criterion must be 'elpd_loo' or 'elpd_waic'")
+    x, z = np.asarray(a[criterion], dtype=np.float64), np.asarray(b[criterion], dtype=np.float64)
+    if x.shape != z.shape:
+        raise SpamTreeError(1, "loo_compare: the two results have different numbers of rows")
+    dlt = (x - z)[~(np.isnan(x) | np.isnan(z))]
+    n = dlt.size
+    return {"elpd_diff": float(dlt.sum()), "se_diff": float(np.sqrt(n * np.var(dlt, ddof=1))) if n > 1 else float("nan"), "n": n}
+
+
 def spamtree_mv_mcmc(y, X, Z, coords, mv_id, blocking, gix_block, res_is_ref, parents, children, limited_tree,
                      layer_names, layer_gibbs_group, indexing, set_unif_bounds_in, start_w, theta, beta, tausq, mcmcsd,
                      mcmc_keep=100, mcmc_burn=100, mcmc_thin=1, num_threads=1, use_alg='S', adapting=False,
@@ -672,7 +767,7 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
              limited_tree=False, cherrypick_same_margin=True, cherrypick_group_locations=True, mvbias=0,
              mcmc=None, num_threads=4, verbose=False, settings=None, prior=None, starting=None, debug=None, *,
              device=0, seed=1, rng_mode=1, tree_seed=0, coords_new=None, x_new=None, mv_id_new=None, summary_probs=None,
-             n_chains=1):
+             n_chains=1, fit_criteria=False):
     """Mirror of the R entry point spamtree() (R/spamtree_fit.R:1-371): same arguments and defaults, same returned
     names (`coords`, `coordsinfo`, `mv_id` + everything spamtree_mv_mcmc returns).  The tree is built by the
     deterministic stand-in for make_tree() (mvbias other than 0 is not supported).
@@ -698,7 +793,11 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
     (default (0.025, 0.5, 0.975)): "w_summary" and "yhat_summary" (with coords_new also "w_new_summary" and
     "yhat_new_summary"), and "theta_summary", "beta_summary" (rows in beta_mcmc's p x q order, column-major) and
     "tausq_summary" over the chains' samples.  R-hat can only detect what the starting points expose: identical starts are
-    the default only because the reference has a single start, so pass dispersed beta / tausq starts to test convergence."""
+    the default only because the reference has a single start, so pass dispersed beta / tausq starts to test convergence.
+
+    fit_criteria=True (rng_mode = 1): the result gains "fit_criteria", PSIS-LOO, WAIC and DIC per observation and in total
+    (the dict of SpamTreeMV.fit_criteria; with n_chains > 1 pooled over the chains), formed on the device from the draws of
+    w.  Every other key is what the call without it returns.  Compare two fits of the same data with loo_compare."""
     y = np.asarray(y, dtype=np.float64).reshape(-1)
     x = np.asarray(x, dtype=np.float64).reshape(y.size, -1)
     coords = np.asarray(coords, dtype=np.float64)
@@ -712,6 +811,9 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
         raise SpamTreeError(1, "n_chains must be at least 1")
     if n_chains > 1 and rng_mode != 1:
         raise SpamTreeError(1, "n_chains > 1 needs rng_mode = 1: the pooled summaries read every chain's draws on the device")
+    if fit_criteria and rng_mode != 1:
+        raise SpamTreeError(1, "fit_criteria needs rng_mode = 1: the criteria read the draws of w kept on the device")
+    crit = bool(fit_criteria)
     if isinstance(starting, (list, tuple)):
         if len(starting) != n_chains:
             raise SpamTreeError(1, "starting: one dict per chain")
@@ -780,7 +882,7 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
         results = _mv_mcmc_on(model, None, bounds, mcmc_mh_sd, mcmc["keep"], mcmc["burn"], mcmc["thin"], settings["adapting"],
                               debug["sample_beta"], debug["sample_tausq"], debug["sample_theta"], debug["sample_w"],
                               debug["sample_predicts"], rng_mode, seed_k, not summ, not summ,
-                              device_samples=("w", "yhat") if summ or on_device else ())
+                              device_samples=("w", "yhat") if summ or on_device else ("w",) if crit else ())
         if summ:
             results["w_summary"] = model.summarize("w", summary_probs)
             results["yhat_summary"] = model.summarize("yhat", summary_probs)
@@ -803,6 +905,8 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
         model = open_chain(starting)
         try:
             results = run_chain(model, seed, False)
+            if crit:
+                results["fit_criteria"] = model.fit_criteria()
         finally:
             model.close()
         return {"coords": cs, "coordsinfo": coordsinfo, "mv_id": mv_id, **results}
@@ -815,6 +919,8 @@ def spamtree(y, x, coords, mv_id=None, cell_size=25, K=None, start_level=0, tree
             chains.append(run_chain(models[-1], seed + k, True))
         for which in ("w", "yhat") + (("w_new", "yhat_new") if coords_new is not None else ()):
             out[which + "_summary"] = summarize_chains(models, which, probs)
+        if crit:
+            out["fit_criteria"] = _criteria(models, 1.0)
     finally:
         for m in models:
             m.close()

@@ -341,6 +341,125 @@ int st_summarize_draws(int32_t device, const double* draws, int64_t n_rows, int3
   } catch (const std::exception& ex) { g_create_error = ex.what(); } catch (...) { g_create_error = "unknown exception"; }
   return ST_ERR_INVALID;
 }
+int st_fit_criteria(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit_criteria_out* out) {
+  if (!hs || n_chains < 1 || !hs[0]) {  // (no handle to report to)
+    g_create_error = n_chains < 1 ? "st_fit_criteria: n_chains must be at least 1" : "st_fit_criteria: hs or hs[0] is NULL";
+    return ST_ERR_INVALID;
+  }
+  st_handle* h0 = hs[0];
+  st::Model& M0 = h0->model;
+  if (!out) { M0.err = "st_fit_criteria: out is NULL"; return ST_ERR_INVALID; }
+  activate(h0);
+  ST_GUARD_BEGIN
+  const int64_t n = M0.store.get(0).n;
+  const int S = M0.store.get(0).S, p = M0.p, q = M0.q;
+  int rc = st::criteria_check("st_fit_criteria", n_chains, std::max(S, 1), r_eff, M0.err);
+  if (rc) return rc;
+  const size_t nb = (size_t)p * S * q, nt = (size_t)q * S, N = (size_t)n_chains * S;
+  std::vector<const double*> src(n_chains);
+  st::dvec beta(N * p * q), tausq(N * q);  // pooled draw g = k S + s: p x q, then q
+  for (int k = 0; k < n_chains; k++) {
+    const std::string hk = "st_fit_criteria: handle " + std::to_string(k);
+    if (!hs[k]) { M0.err = hk + " is NULL"; return ST_ERR_INVALID; }
+    const st::Model& Mk = hs[k]->model;
+    if (Mk.device != M0.device) {
+      M0.err = hk + " is on device " + std::to_string(Mk.device) + ", handle 0 on device " + std::to_string(M0.device);
+      return ST_ERR_INVALID;
+    }
+    const st::DrawStore::Store* s = Mk.store.find(0, hk + " has ", M0.err);
+    if (!s) return ST_ERR_INVALID;
+    if (s->n != n || s->S != S) {
+      M0.err = hk + " stores " + std::to_string(s->S) + " draws of " + std::to_string(s->n) + " rows, handle 0 " + std::to_string(S) +
+               " draws of " + std::to_string(n) + " rows";
+      return ST_ERR_INVALID;
+    }
+    if (Mk.p != p || Mk.q != q) {
+      M0.err = hk + " has p = " + std::to_string(Mk.p) + ", q = " + std::to_string(Mk.q) + "; handle 0 p = " + std::to_string(p) +
+               ", q = " + std::to_string(q);
+      return ST_ERR_INVALID;
+    }
+    if (Mk.n_all != M0.n_all || std::memcmp(Mk.y.data(), M0.y.data(), M0.y.size() * sizeof(double)) ||
+        std::memcmp(Mk.X.data(), M0.X.data(), M0.X.size() * sizeof(double)) ||
+        std::memcmp(Mk.mv_id.data(), M0.mv_id.data(), M0.mv_id.size() * sizeof(int64_t))) {
+      M0.err = hk + " has a different y, X or mv_id from handle 0 (the criteria compare fits of the same data)";
+      return ST_ERR_INVALID;
+    }
+    const st::dvec& sm = Mk.store.samples;  // theta (npar x S) | beta (p x S x q) | tausq (q x S)
+    if (sm.size() < nb + nt) { M0.err = hk + ": the stored run's beta / tausq samples are missing"; return ST_ERR_INVALID; }
+    const double* be = sm.data() + (sm.size() - nb - nt);
+    const double* ta = be + nb;
+    for (int s2 = 0; s2 < S; s2++) {
+      const size_t g = (size_t)k * S + s2;
+      for (int j = 0; j < q; j++) {
+        for (int a = 0; a < p; a++) beta[(g * q + j) * p + a] = be[a + (size_t)s2 * p + (size_t)j * p * S];
+        tausq[g * q + j] = ta[j + (size_t)s2 * q];
+      }
+    }
+    src[k] = s->d;
+  }
+  for (int k = 1; k < n_chains; k++)  // every store is complete before the kernel reads it on hs[0]'s stream
+    if (const cudaError_t e = cudaStreamSynchronize(hs[k]->model.stream)) {
+      M0.err = std::string("st_fit_criteria: CUDA error in sync of handle ") + std::to_string(k) + ": " + cudaGetErrorString(e);
+      return ST_ERR_CUDA;
+    }
+  std::vector<char> obs(n);
+  for (int64_t i = 0; i < n; i++) obs[i] = std::isfinite(M0.y[i]);
+  const st::CritInputs in{M0.y.data(), M0.X.data(), M0.mv_id.data(), beta.data(), tausq.data(), p, q};
+  return st::fit_criteria(src.data(), n, n_chains, S, r_eff, obs, &in, *out, M0.stream, M0.err);
+  ST_GUARD_END(h0)
+}
+int st_fit_criteria_loglik(int32_t device, const double* loglik, int64_t n_rows, int32_t n_chains, int32_t n_samples, double r_eff,
+                           st_fit_criteria_out* out) {
+  if (!out || n_rows < 0 || (n_rows > 0 && !loglik)) {
+    g_create_error = "st_fit_criteria_loglik: out or loglik missing, or n_rows < 0";
+    return ST_ERR_INVALID;
+  }
+  try {
+    int rc = st::criteria_check("st_fit_criteria_loglik", n_chains, n_samples, r_eff, g_create_error);
+    if (rc) return rc;
+    // a row is unobserved when all its values are NaN; an observed row must be finite throughout
+    const size_t per = (size_t)n_rows * n_samples, all = per * n_chains;
+    std::vector<char> obs(n_rows);
+    for (int64_t i = 0; i < n_rows; i++) obs[i] = !std::isnan(loglik[i]);
+    for (size_t j = 0; j < all; j++) {
+      const int64_t i = (int64_t)(j % n_rows);
+      if (obs[i] ? !std::isfinite(loglik[j]) : !std::isnan(loglik[j])) {
+        g_create_error = "st_fit_criteria_loglik: row " + std::to_string(i) + " is observed (not all NaN) but value " + std::to_string(j) +
+                         " ([chain][sample][row] order) is not finite";
+        return ST_ERR_INVALID;
+      }
+    }
+    const bool any = out->lpd || out->elpd_loo || out->p_loo || out->pareto_k || out->elpd_waic || out->p_waic;
+    if (!any || n_rows == 0) return st::fit_criteria(nullptr, n_rows, n_chains, n_samples, r_eff, obs, nullptr, *out, 0, g_create_error);
+    if (cudaSetDevice(device) != cudaSuccess) { (void)cudaGetLastError(); g_create_error = "st_fit_criteria_loglik: cudaSetDevice failed"; return ST_ERR_CUDA; }
+    const size_t bytes = all * sizeof(double);
+    size_t fr = 0, tot = 0;
+    if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { (void)cudaGetLastError(); g_create_error = "st_fit_criteria_loglik: cudaMemGetInfo failed"; return ST_ERR_CUDA; }
+    // (the copy, plus the outputs' buffer and some headroom)
+    const size_t need = bytes + (size_t)n_rows * 8 * sizeof(double) + (64u << 20);
+    if (need > fr) {
+      g_create_error = "st_fit_criteria_loglik: the log-likelihood needs " + std::to_string(need) + " bytes of device memory and " +
+                       std::to_string(fr) + " bytes are free";
+      return ST_ERR_UNSUPPORTED;
+    }
+    double* d = nullptr;
+    cudaError_t e = cudaMalloc((void**)&d, bytes);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); g_create_error = std::string("st_fit_criteria_loglik: ") + cudaGetErrorString(e); return ST_ERR_UNSUPPORTED; }
+    e = cudaMemcpyAsync(d, loglik, bytes, cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess) {
+      std::vector<const double*> src(n_chains);
+      for (int c = 0; c < n_chains; c++) src[c] = d + (size_t)c * per;
+      rc = st::fit_criteria(src.data(), n_rows, n_chains, n_samples, r_eff, obs, nullptr, *out, 0, g_create_error);
+    } else {
+      g_create_error = std::string("CUDA error in H2D log-likelihood: ") + cudaGetErrorString(e);
+      rc = ST_ERR_CUDA;
+    }
+    cudaStreamSynchronize(0);
+    cudaFree(d);
+    return rc;
+  } catch (const std::exception& ex) { g_create_error = ex.what(); } catch (...) { g_create_error = "unknown exception"; }
+  return ST_ERR_INVALID;
+}
 int st_bench_iteration(st_handle* h, const double* theta_prop, int do_swap, uint64_t seed, double* out3, float* ms_out) {
   if (!h || !theta_prop || !out3) return ST_ERR_INVALID;
   activate(h);

@@ -1587,4 +1587,185 @@ cudaError_t launch_chains_summary(const double* const* src, long long n, int K, 
   return cudaGetLastError();
 }
 
+// ------------------------------------------------------------------ model criteria: PSIS-LOO, WAIC and DIC per observation
+// (st_fit_criteria / st_fit_criteria_loglik; DESIGN.md §5e)
+// the maximum over the G threads of each row group (as summary_group_sum, pairwise in a fixed order; NaN only if all are)
+__device__ __forceinline__ double summary_group_max(double v, double* red, int G) {
+  const int t = threadIdx.x, lane = t % G;
+  red[t] = v;
+  __syncthreads();
+  for (int s = G >> 1; s > 0; s >>= 1) {
+    if (lane < s) red[t] = fmax(red[t], red[t + s]);
+    __syncthreads();
+  }
+  const double total = red[t - lane];
+  __syncthreads();
+  return total;
+}
+
+constexpr int kGpdSlots = 7;  // grid points of the GPD fit per thread: 30 + floor(sqrt(ceil(0.2 N))) <= 105 <= 7 G (G >= 16)
+
+// One CTA per tile of R rows.  Draw g = c S + s of row i: src[c][s n + i], the log-likelihood itself (P.y == NULL) or w, from
+// which ll is formed with y, X, beta_g and tausq_g (every row of the tile reads the same beta_g / tausq_g: read-only path).
+// The tile is staged once with coalesced loads (consecutive threads, consecutive rows; T is a multiple of R, so thread t
+// stages row t % R throughout and sums its w there for the posterior mean), as order-preserving keys of ll, row-major
+// (key[r N + g]), then sorted per row (summary_sort_rows): ascending ll is descending lw = min(ll) - ll, so the PSIS tail is
+// sorted positions [0, L) and its cutoff position L.  Per row, over G = T / R threads, every reduction in a fixed order:
+// lpd, mean and variance of ll; the GPD fit (each thread takes grid points lane + 1 + u G and sums its point's log1p over the
+// tail sequentially; x_m and the smoothed weights are formed on the fly from the keys); the truncated, normalised weights and
+// elpd_loo.  out: 8 n doubles, [lpd | elpd_loo | p_loo | pareto_k | elpd_waic | p_waic | -2 mean ll | -2 log N(y; plug-in)],
+// NaN at unobserved rows.
+__global__ void __launch_bounds__(kSummaryThreads, 1)  // (min. one CTA per SM: ptxas otherwise caps it at 64 registers and spills)
+fit_criteria_kernel(const double* const* __restrict__ src, long long n, int K, int S, int R, int L, CritParams P, double* __restrict__ out) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double* red = reinterpret_cast<double*>(smem_raw);  // T
+  u64* key = reinterpret_cast<u64*>(red + blockDim.x);  // R x N
+  const int T = blockDim.x, t = threadIdx.x, G = T / R, r = t / G, lane = t % G;
+  const int N = K * S;
+  const double kNaN = __longlong_as_double(0x7ff8000000000000LL), kInf = __longlong_as_double(0x7ff0000000000000LL);
+  const double k2pi = 6.283185307179586;  // 2 pi
+  const bool par = P.y != nullptr;
+  const long long row0 = (long long)blockIdx.x * R;
+  const int nr = (int)min((long long)R, n - row0);
+  auto observed = [&](int rr) { return rr < nr && (par ? isfinite(P.y[row0 + rr]) : !isnan(src[0][row0 + rr])); };
+  // ---- stage: element e of the tile is (draw e / R, row e % R); unobserved rows and rows past n hold zeros
+  {
+    const int rs = t % R;
+    const long long is = row0 + rs;
+    const bool live = observed(rs);
+    const int js = live && par ? P.mvq[is] : 0;
+    const double yv = live && par ? P.y[is] : 0.0;
+    double wsum = 0.0;
+    for (int g = t / R; g < N; g += G) {
+      double ll = 0.0;
+      if (live) {
+        const int c = g / S, s = g - c * S;
+        const double v = src[c][(long long)s * n + is];
+        if (par) {
+          const double* b = P.beta + ((size_t)g * P.q + js) * P.p;
+          double xb = 0.0;
+          for (int a = 0; a < P.p; a++) xb += P.X[is + (long long)a * n] * __ldg(b + a);
+          const double tau = __ldg(P.tausq + (size_t)g * P.q + js);
+          const double res = yv - xb - v;
+          ll = -0.5 * log(k2pi * tau) - res * res / (2.0 * tau);
+          wsum += v;
+        } else {
+          ll = v;
+        }
+      }
+      key[(size_t)rs * N + g] = summary_key(ll);
+    }
+    red[t] = wsum;  // thread t's part of row t % R: draws g = t / R (mod G)
+  }
+  __syncthreads();
+  const double wpart = red[r + R * lane];
+  __syncthreads();
+  const double wbar = summary_group_sum(wpart, red, G) / N;
+  summary_sort_rows(key, R, N);
+  const u64* kr = key + (size_t)r * N;
+  auto llv = [&](int s) { return summary_val(kr[s]); };
+  const double lmin = llv(0), lmax = llv(N - 1);
+  // ---- lpd, mean and variance of ll
+  double acc = 0.0;
+  for (int s = lane; s < N; s += G) acc += exp(llv(s) - lmax);
+  const double lpd = lmax + log(summary_group_sum(acc, red, G)) - log((double)N);
+  acc = 0.0;
+  for (int s = lane; s < N; s += G) acc += llv(s);
+  const double mean = summary_group_sum(acc, red, G) / N;
+  acc = 0.0;
+  for (int s = lane; s < N; s += G) { const double d = llv(s) - mean; acc += d * d; }
+  const double ss = summary_group_sum(acc, red, G);
+  const double p_waic = N > 1 ? ss / (N - 1) : kNaN;
+  // ---- PSIS: the GPD fit of the tail (L is the same for every row: the branch and its barriers are uniform)
+  double khat = kInf, sig = 0.0, ec = 0.0;
+  if (L >= 5) {
+    ec = exp(lmin - llv(L));  // exp(cutoff)
+    const bool flat = fabs((lmin - llv(0)) - (lmin - llv(L - 1))) < 2.220446049250313e-16 / 100.0;
+    auto xt = [&](int m) { return exp(lmin - llv(L - 1 - m)) - ec; };  // x_m, ascending in m
+    const int Mg = 30 + (int)floor(sqrt((double)L));
+    const double xstar = xt((int)floor(L / 4.0 + 0.5) - 1), xmax = xt(L - 1);
+    double lj[kGpdSlots], thj[kGpdSlots], lm = -kInf;
+#pragma unroll
+    for (int u = 0; u < kGpdSlots; u++) {
+      const int j = lane + 1 + u * G;
+      lj[u] = -kInf;
+      thj[u] = 0.0;
+      if (j <= Mg) {
+        const double th = 1.0 / xmax + (1.0 - sqrt((double)Mg / (j - 0.5))) / 3.0 / xstar;
+        const double a = -th;
+        double ks = 0.0;
+        for (int m = 0; m < L; m++) ks += log1p(a * xt(m));
+        const double k = ks / L;
+        lj[u] = L * (log(a / k) - k - 1.0);
+        thj[u] = th;
+        lm = fmax(lm, lj[u]);
+      }
+    }
+    const double gm = summary_group_max(lm, red, G);
+    double se = 0.0, st = 0.0;
+#pragma unroll
+    for (int u = 0; u < kGpdSlots; u++)
+      if (lane + 1 + u * G <= Mg) { const double e = exp(lj[u] - gm); se += e; st += thj[u] * e; }
+    const double sum_e = summary_group_sum(se, red, G);
+    const double that = summary_group_sum(st, red, G) / sum_e;
+    acc = 0.0;
+    for (int m = lane; m < L; m += G) acc += log1p(-that * xt(m));
+    const double k = summary_group_sum(acc, red, G) / L;
+    sig = -k / that;
+    const double kw = (L * k + 5.0) / (L + 10.0);
+    khat = flat || isnan(kw) ? kInf : kw;
+  }
+  const bool smooth = isfinite(khat);
+  // ---- the smoothed (tail of a finite k-hat), truncated log weights by sorted position, then their normalisation and elpd_loo
+  auto lwv = [&](int s) {
+    double v = lmin - llv(s);
+    if (smooth && s < L) {
+      const double pm = ((L - 1 - s) + 0.5) / L;
+      v = log(sig * expm1(-khat * log1p(-pm)) / khat + ec);
+    }
+    return v > 0.0 ? 0.0 : v;
+  };
+  double mx = -kInf;
+  for (int s = lane; s < N; s += G) mx = fmax(mx, lwv(s));
+  mx = summary_group_max(mx, red, G);
+  acc = 0.0;
+  for (int s = lane; s < N; s += G) acc += exp(lwv(s) - mx);
+  const double lsw = mx + log(summary_group_sum(acc, red, G));
+  mx = -kInf;
+  for (int s = lane; s < N; s += G) mx = fmax(mx, (lwv(s) - lsw) + llv(s));
+  mx = summary_group_max(mx, red, G);
+  acc = 0.0;
+  for (int s = lane; s < N; s += G) acc += exp((lwv(s) - lsw) + llv(s) - mx);
+  const double elpd = mx + log(summary_group_sum(acc, red, G));
+  if (lane == 0 && r < nr) {
+    const long long i = row0 + r;
+    const bool live = observed(r);
+    double dhat = kNaN;
+    if (live && par) {
+      const int j = P.mvq[i];
+      double mu = 0.0;
+      for (int a = 0; a < P.p; a++) mu += P.X[i + (long long)a * n] * P.bbar[j * P.p + a];
+      mu += wbar;
+      const double tb = P.tbar[j], res = P.y[i] - mu;
+      dhat = -2.0 * (-0.5 * log(k2pi * tb) - res * res / (2.0 * tb));
+    }
+    const double v[8] = {lpd, elpd, lpd - elpd, khat, lpd - p_waic, p_waic, -2.0 * mean, dhat};
+#pragma unroll
+    for (int c = 0; c < 8; c++) out[(long long)c * n + i] = live ? v[c] : kNaN;
+  }
+}
+int criteria_tail_len(int N, double r_eff) { return (int)ceil(fmin(0.2 * N, 3.0 * sqrt(N / r_eff))); }
+cudaError_t launch_fit_criteria(const double* const* src, long long n, int K, int S, int R, double r_eff, const CritParams& P, double* out,
+                                cudaStream_t st) {
+  if (n <= 0 || K <= 0 || S <= 0) return cudaSuccess;
+  const int N = K * S, L = criteria_tail_len(N, r_eff);
+  if (L >= 5 && 30 + (int)floor(sqrt((double)L)) > kGpdSlots * (kSummaryThreads / R)) return cudaErrorInvalidValue;
+  static SmemOptIn opt;
+  const size_t smem = summary_smem_bytes(N, R);
+  cudaError_t e = ensure_dynamic_smem(fit_criteria_kernel, smem, opt);
+  if (e != cudaSuccess) return e;
+  fit_criteria_kernel<<<(unsigned)((n + R - 1) / R), kSummaryThreads, smem, st>>>(src, n, K, S, R, L, P, out);
+  return cudaGetLastError();
+}
+
 }  // namespace st

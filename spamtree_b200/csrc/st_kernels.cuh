@@ -142,5 +142,21 @@ size_t chains_smem_bytes(int K, int S, int R);
 int chains_rows_per_cta(int K, int S, size_t smem_cap);  // as summary_rows_per_cta; 0 when not even one row fits
 cudaError_t launch_chains_summary(const double* const* src, long long n, int K, int S, int R, const double* probs, int np, double* mean,
                                   double* sd, double* quant, double* rhat, double* ess_bulk, double* ess_tail, cudaStream_t st);
+// ---- model criteria over K chains of S draws of n rows (st_fit_criteria, st_fit_criteria_loglik; DESIGN.md §5e).  Shared
+// memory as summary_kernel's with N = K S draws per row: R = summary_rows_per_cta(K S, cap) rows per CTA.
+struct CritParams {
+  const double* y;      // n, NaN: unobserved row.  NULL: the draws are the log-likelihood itself (NaN in draw 0: unobserved)
+  const double* X;      // n x p, column-major
+  const int* mvq;       // n, 0-based outcome
+  const double* beta;   // draw g's p x q coefficients at beta[g p q ..), column-major
+  const double* tausq;  // draw g's q variances at tausq[g q ..)
+  const double* bbar;   // p x q pooled posterior means
+  const double* tbar;   // q
+  int p, q;
+};
+int criteria_tail_len(int N, double r_eff);  // min(ceil(0.2 N), ceil(3 sqrt(N / r_eff))), as R loo's n_pareto_draws
+// out: 8 n doubles, [lpd | elpd_loo | p_loo | pareto_k | elpd_waic | p_waic | -2 mean ll | -2 log N(y; plug-in means)]
+cudaError_t launch_fit_criteria(const double* const* src, long long n, int K, int S, int R, double r_eff, const CritParams& P, double* out,
+                                cudaStream_t st);
 
 }  // namespace st

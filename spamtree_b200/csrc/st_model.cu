@@ -6,6 +6,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <numeric>
 
 #include "../../include/spamtree_b200.h"
@@ -2131,6 +2132,126 @@ int summarize_chains(const double* const* src, int64_t n, int K, int S, const do
   }
   chk(cudaStreamSynchronize(st), "sync");  // (before the buffer is freed, whatever failed)
   return e == cudaSuccess ? 0 : 2;
+}
+
+// ---- model criteria (st_fit_criteria, st_fit_criteria_loglik; DESIGN.md §5e)
+int criteria_check(const char* what, int K, int S, double r_eff, std::string& err) {
+  if (K < 1 || S < 1) { err = std::string(what) + ": n_chains and n_samples must be at least 1"; return 1; }
+  if (!(r_eff > 0.0) || !std::isfinite(r_eff)) { err = std::string(what) + ": r_eff must be positive and finite"; return 1; }
+  const size_t lim = (kChainsSmemCap - (size_t)kSummaryThreads * sizeof(double)) / sizeof(unsigned long long);
+  if ((long long)K * S > (long long)lim || summary_rows_per_cta(K * S, kChainsSmemCap) < 1) {
+    err = std::string(what) + ": " + std::to_string(K) + " chains of " + std::to_string(S) + " draws exceed what one CTA stages in "
+          "shared memory (n_chains x n_samples = " + std::to_string((long long)K * S) + ", at most " + std::to_string(lim) + ")";
+    return 4;
+  }
+  return 0;
+}
+
+int fit_criteria(const double* const* src, int64_t n, int K, int S, double r_eff, const std::vector<char>& obs, const CritInputs* in,
+                 st_fit_criteria_out& out, cudaStream_t st, std::string& err) {
+  const double nan = std::numeric_limits<double>::quiet_NaN();
+  const int N = K * S;
+  out.n_rows = n;
+  out.n_chains = K;
+  out.n_samples = S;
+  out.n_obs = 0;
+  for (int64_t i = 0; i < n; i++) out.n_obs += obs[i] != 0;
+  out.k_threshold = std::min(1.0 - 1.0 / std::log10((double)N), 0.7);
+  out.n_k_high = out.n_p_waic_high = 0;
+  double* tot[16] = {&out.elpd_loo_total, &out.se_elpd_loo, &out.p_loo_total, &out.looic, &out.se_looic, &out.elpd_waic_total,
+                     &out.se_elpd_waic, &out.p_waic_total, &out.waic, &out.se_waic, &out.lpd_total, &out.dbar, &out.dhat,
+                     &out.p_dic, &out.dic, nullptr};
+  for (int c = 0; tot[c]; c++) *tot[c] = nan;
+  double* hdst[6] = {out.lpd, out.elpd_loo, out.p_loo, out.pareto_k, out.elpd_waic, out.p_waic};
+  if (!(hdst[0] || hdst[1] || hdst[2] || hdst[3] || hdst[4] || hdst[5]) || n == 0) return 0;
+  // one device buffer: the 8 per-row outputs | K chain pointers | with parameters: y | X | bbar | tbar | beta | tausq | mvq
+  const size_t nn = (size_t)n, p = in ? in->p : 0, q = in ? in->q : 0;
+  const size_t n_par = in ? nn + nn * p + p * q + q + (size_t)N * p * q + (size_t)N * q + (nn + 1) / 2 : 0;
+  const size_t nd = 8 * nn + (size_t)K + n_par;
+  double* d = nullptr;
+  cudaError_t e = cudaMalloc((void**)&d, nd * sizeof(double));
+  if (e != cudaSuccess) { (void)cudaGetLastError(); err = std::string("CUDA error in alloc criteria: ") + cudaGetErrorString(e); return 2; }
+  struct Free { double* p; ~Free() { cudaFree(p); } } fr{d};
+  auto chk = [&](cudaError_t c, const char* what) {
+    if (c != cudaSuccess && e == cudaSuccess) { e = c; err = std::string("CUDA error in ") + what + ": " + cudaGetErrorString(c); }
+  };
+  const double** dsrc = reinterpret_cast<const double**>(d + 8 * nn);
+  chk(cudaMemcpyAsync(dsrc, src, K * sizeof(double*), cudaMemcpyHostToDevice, st), "H2D chain pointers");
+  CritParams P{};
+  dvec bbar, tbar;
+  std::vector<int> mvq;
+  if (in) {  // (host vectors the copies read stay alive until the synchronisation at the end)
+    bbar.assign(p * q, 0.0);
+    tbar.assign(q, 0.0);
+    for (int g = 0; g < N; g++) {  // pooled means over the N draws, in draw order
+      for (size_t c = 0; c < p * q; c++) bbar[c] += in->beta[(size_t)g * p * q + c];
+      for (size_t j = 0; j < q; j++) tbar[j] += in->tausq[(size_t)g * q + j];
+    }
+    for (double& v : bbar) v /= N;
+    for (double& v : tbar) v /= N;
+    mvq.resize(nn);
+    for (size_t i = 0; i < nn; i++) mvq[i] = (int)in->mv_id[i] - 1;
+    double* a = d + 8 * nn + K;
+    double* dy = a; a += nn;
+    double* dX = a; a += nn * p;
+    double* dbb = a; a += p * q;
+    double* dtb = a; a += q;
+    double* dbe = a; a += (size_t)N * p * q;
+    double* dta = a; a += (size_t)N * q;
+    int* dmv = reinterpret_cast<int*>(a);
+    chk(cudaMemcpyAsync(dy, in->y, nn * sizeof(double), cudaMemcpyHostToDevice, st), "H2D y");
+    if (p) chk(cudaMemcpyAsync(dX, in->X, nn * p * sizeof(double), cudaMemcpyHostToDevice, st), "H2D X");
+    if (p) chk(cudaMemcpyAsync(dbb, bbar.data(), p * q * sizeof(double), cudaMemcpyHostToDevice, st), "H2D beta means");
+    chk(cudaMemcpyAsync(dtb, tbar.data(), q * sizeof(double), cudaMemcpyHostToDevice, st), "H2D tausq means");
+    if (p) chk(cudaMemcpyAsync(dbe, in->beta, (size_t)N * p * q * sizeof(double), cudaMemcpyHostToDevice, st), "H2D beta samples");
+    chk(cudaMemcpyAsync(dta, in->tausq, (size_t)N * q * sizeof(double), cudaMemcpyHostToDevice, st), "H2D tausq samples");
+    chk(cudaMemcpyAsync(dmv, mvq.data(), nn * sizeof(int), cudaMemcpyHostToDevice, st), "H2D mv_id");
+    P = CritParams{dy, dX, dmv, dbe, dta, dbb, dtb, (int)p, (int)q};
+  }
+  if (e == cudaSuccess)
+    chk(launch_fit_criteria(dsrc, n, K, S, summary_rows_per_cta(N, kChainsSmemCap), r_eff, P, d, st), "fit_criteria_kernel");
+  dvec h(8 * nn);
+  if (e == cudaSuccess) chk(cudaMemcpyAsync(h.data(), d, 8 * nn * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H criteria");
+  chk(cudaStreamSynchronize(st), "sync");  // (before the buffer is freed, whatever failed)
+  if (e != cudaSuccess) return 2;
+  for (int c = 0; c < 6; c++)
+    if (hdst[c]) std::copy(h.begin() + c * nn, h.begin() + (c + 1) * nn, hdst[c]);
+  // ---- totals over the observed rows, in row order
+  const double* lpd = h.data();
+  const double *el = lpd + nn, *pl = el + nn, *kh = pl + nn, *ew = kh + nn, *pw = ew + nn, *db = pw + nn, *dh = db + nn;
+  double s[7] = {0, 0, 0, 0, 0, 0, 0};  // elpd_loo, p_loo, elpd_waic, p_waic, lpd, dbar, dhat
+  for (size_t i = 0; i < nn; i++) {
+    if (!obs[i]) continue;
+    s[0] += el[i]; s[1] += pl[i]; s[2] += ew[i]; s[3] += pw[i]; s[4] += lpd[i]; s[5] += db[i]; s[6] += dh[i];
+    out.n_k_high += kh[i] > out.k_threshold;
+    out.n_p_waic_high += pw[i] > 0.4;
+  }
+  const double no = (double)out.n_obs;
+  auto se = [&](const double* v, double total) {  // sqrt(n_obs var(v_i, ddof 1))
+    const double m = total / no;
+    double ss = 0.0;
+    for (size_t i = 0; i < nn; i++)
+      if (obs[i]) ss += (v[i] - m) * (v[i] - m);
+    return out.n_obs > 1 ? std::sqrt(no * ss / (no - 1)) : nan;
+  };
+  out.elpd_loo_total = s[0];
+  out.se_elpd_loo = se(el, s[0]);
+  out.p_loo_total = s[1];
+  out.looic = -2.0 * s[0];
+  out.se_looic = 2.0 * out.se_elpd_loo;
+  out.elpd_waic_total = s[2];
+  out.se_elpd_waic = se(ew, s[2]);
+  out.p_waic_total = s[3];
+  out.waic = -2.0 * s[2];
+  out.se_waic = 2.0 * out.se_elpd_waic;
+  out.lpd_total = s[4];
+  if (in) {
+    out.dbar = s[5];
+    out.dhat = s[6];
+    out.p_dic = s[5] - s[6];
+    out.dic = s[5] + out.p_dic;
+  }
+  return 0;
 }
 
 

@@ -357,4 +357,20 @@ int chains_check(const char* what, int K, int S, const double* probs, int n_prob
 int summarize_chains(const double* const* src, int64_t n, int K, int S, const double* probs, int n_probs, st_chains_summary_out& out,
                      cudaStream_t st, std::string& err);
 
+// ---- model criteria (st_fit_criteria, st_fit_criteria_loglik; DESIGN.md §5e).  criteria_check: K, S and r_eff as both entry
+// points refuse them (1), or K S draws beyond one CTA's shared memory (4).  fit_criteria: src = K device pointers (a host
+// array), chain c's draw (s, i) at src[c][s * n + i]: w when `in` is given, else the log-likelihood itself; obs: n flags of
+// the observed rows.  Runs on st and synchronises it; outputs and totals as st_fit_criteria_out (all NULL: the sizes only).
+struct CritInputs {          // host arrays, rows in boundary order
+  const double* y;           // n, NaN = missing
+  const double* X;           // n x p, column-major
+  const int64_t* mv_id;      // n, 1-based
+  const double* beta;        // pooled draw g's p x q coefficients at beta[g p q ..), column-major
+  const double* tausq;       // pooled draw g's q variances at tausq[g q ..)
+  int p, q;
+};
+int criteria_check(const char* what, int K, int S, double r_eff, std::string& err);
+int fit_criteria(const double* const* src, int64_t n, int K, int S, double r_eff, const std::vector<char>& obs, const CritInputs* in,
+                 st_fit_criteria_out& out, cudaStream_t st, std::string& err);
+
 }  // namespace st
