@@ -221,10 +221,24 @@ int st_predict_new(st_handle* h, const st_new_rows* rows, const st_pred_samples*
  * The store (n_all x keep x 8 bytes per quantity) is checked against the free device memory before a run allocates or
  * launches anything: ST_ERR_UNSUPPORTED, with the bytes needed and free, and the handle as it was.  It holds the last completed
  * run, is replaced by the next one, and is freed by what = 0 or st_destroy.  ST_ERR_UNSUPPORTED: a store with rng_mode = 0,
- * or on a partitioned handle. */
+ * or on a partitioned handle.
+ * ST_KEEP_LOGLIK_INT: the integrated log-likelihood of every row at every saved iteration (DESIGN.md §5f), [sample][row] in
+ * boundary order, NaN at the rows whose y is missing.  Row i of draw s is ll = log N(y_i - x_i' beta; m_i, v_i + tausq_j), where
+ * N(m_i, v_i) is the prior conditional of w_i given the rest of w at theta_s, as the Gibbs sweep has it when it draws the block
+ * of row i, and beta, tausq are those the sweep uses.  Only the saved iterations' sweeps form it (with the same draws: the chain
+ * is bit for bit the chain without it).  Refused with ST_ERR_INVALID by an st_mcmc_run that does not sample w, besides the
+ * refusals above; st_deal_with_w forms it too while the bit is set (st_get_loglik_int). */
 #define ST_KEEP_W 1
 #define ST_KEEP_YHAT 2
+#define ST_KEEP_LOGLIK_INT 4
 int st_keep_samples_on_device(st_handle* h, int32_t what);
+/* The integrated log-likelihood of the last sweep that formed it (st_deal_with_w with ST_KEEP_LOGLIK_INT set, or the last saved
+ * iteration of an st_mcmc_run with it), n_all values in boundary order, NaN where y is missing.  ST_ERR_INVALID: no sweep has
+ * formed it on this handle. */
+int st_get_loglik_int(st_handle* h, double* out);
+/* Copies the draws of a device store to the host: which as st_summarize, and 4 = the integrated log-likelihood of the last
+ * stored run.  out: n_rows x n_samples doubles, [sample][row] (out NULL: the sizes only).  ST_ERR_INVALID: nothing stored. */
+int st_copy_store(st_handle* h, int32_t which, double* out, int64_t* n_rows, int32_t* n_samples);
 /* Per-row summaries of stored draws.  which: 0 = w, 1 = yhat of the last stored run (rows in boundary order); 2 = w_new,
  * 3 = y_new of the last st_predict_new_stored with keep_draws (rows in the caller's order).  Over the S draws of a row:
  *   mean; sd (ddof = 1, 0 for S = 1); quantiles at probs[0..n_probs) exactly as numpy.quantile(method="linear") (R type 7);
@@ -328,6 +342,11 @@ typedef struct {                 /* caller-allocated; NULL pointers skipped; all
  * handle's stream, runs on that of hs[0] and returns when done; changes no handle's state.  Errors: st_last_error(hs[0]);
  * st_last_error(NULL) when there is no handle to report to. */
 int st_fit_criteria(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit_criteria_out* out);
+/* Integrated PSIS-LOO and WAIC (DESIGN.md §5f): the same outputs and handle checks as st_fit_criteria, from the stores of the
+ * integrated log-likelihood (ST_KEEP_LOGLIK_INT) read in place instead of the log-likelihood conditional on w.  w_i is
+ * integrated out of each row's term, so the importance ratios of PSIS-LOO have lighter tails.  The DIC fields are NaN.  A
+ * handle without that store gives ST_ERR_INVALID. */
+int st_fit_criteria_integrated(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit_criteria_out* out);
 /* The PSIS / WAIC part on a host log-likelihood [chain][sample][row] (n_chains x n_samples x n_rows), copied to `device` for
  * the call: a row of NaN is an unobserved row; any other non-finite value is refused (ST_ERR_INVALID).  The DIC fields are NaN
  * (no parameters are given).  ST_ERR_UNSUPPORTED when the copy does not fit in the free device memory.  Errors:

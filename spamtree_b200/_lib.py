@@ -125,7 +125,7 @@ class StFitCriteriaOut(C.Structure):
     ]
 
 
-ST_KEEP_W, ST_KEEP_YHAT = 1, 2
+ST_KEEP_W, ST_KEEP_YHAT, ST_KEEP_LOGLIK_INT = 1, 2, 4
 
 
 # every symbol include/spamtree_b200.h declares, with its signature
@@ -152,6 +152,8 @@ SIGNATURES = {
     "st_mcmc_run": (C.c_int, [C.c_void_p, C.POINTER(StMcmcOpts), C.POINTER(StMcmcOut)]),
     "st_predict_new": (C.c_int, [C.c_void_p, C.POINTER(StNewRows), C.POINTER(StPredSamples), C.POINTER(StPredOut)]),
     "st_keep_samples_on_device": (C.c_int, [C.c_void_p, C.c_int32]),
+    "st_get_loglik_int": (C.c_int, [C.c_void_p, c_double_p]),
+    "st_copy_store": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, c_int64_p, C.POINTER(C.c_int32)]),
     "st_summarize": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, C.c_int32, C.POINTER(StSummaryOut)]),
     "st_predict_new_stored": (C.c_int, [C.c_void_p, C.POINTER(StNewRows), C.c_uint64, C.c_int32, C.POINTER(StPredOut)]),
     "st_summarize_chains": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_int32, c_double_p, C.c_int32,
@@ -159,6 +161,7 @@ SIGNATURES = {
     "st_summarize_draws": (C.c_int, [C.c_int32, c_double_p, C.c_int64, C.c_int32, C.c_int32, c_double_p, C.c_int32,
                                      C.POINTER(StChainsSummaryOut)]),
     "st_fit_criteria": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_double, C.POINTER(StFitCriteriaOut)]),
+    "st_fit_criteria_integrated": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_double, C.POINTER(StFitCriteriaOut)]),
     "st_fit_criteria_loglik": (C.c_int, [C.c_int32, c_double_p, C.c_int64, C.c_int32, C.c_int32, C.c_double,
                                          C.POINTER(StFitCriteriaOut)]),
     "st_bench_iteration": (C.c_int, [C.c_void_p, c_double_p, C.c_int, C.c_uint64, c_double_p, c_float_p]),

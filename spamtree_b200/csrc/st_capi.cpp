@@ -241,6 +241,18 @@ int st_keep_samples_on_device(st_handle* h, int32_t what) {
   ST_GUARD_BEGIN return h->model.keep_samples_on_device(what);
   ST_GUARD_END(h)
 }
+int st_get_loglik_int(st_handle* h, double* out) {
+  if (!h || !out) return ST_ERR_INVALID;
+  activate(h);
+  ST_GUARD_BEGIN return h->model.get_loglik_int(out);
+  ST_GUARD_END(h)
+}
+int st_copy_store(st_handle* h, int32_t which, double* out, int64_t* n_rows, int32_t* n_samples) {
+  if (!h) return ST_ERR_INVALID;
+  activate(h);
+  ST_GUARD_BEGIN return h->model.copy_store(which, out, n_rows, n_samples);
+  ST_GUARD_END(h)
+}
 int st_summarize(st_handle* h, int32_t which, const double* probs, int32_t n_probs, st_summary_out* out) {
   if (!h || !out) return ST_ERR_INVALID;
   activate(h);
@@ -341,6 +353,45 @@ int st_summarize_draws(int32_t device, const double* draws, int64_t n_rows, int3
   } catch (const std::exception& ex) { g_create_error = ex.what(); } catch (...) { g_create_error = "unknown exception"; }
   return ST_ERR_INVALID;
 }
+// the checks st_fit_criteria and st_fit_criteria_integrated make of handle k (hk names it) against handle 0, whose store `which`
+// holds S draws of n rows; *s: handle k's store
+static int criteria_handle(const std::string& hk, st::Model& M0, const st_handle* hk_h, int which, int64_t n, int S,
+                           const st::DrawStore::Store** s) {
+  if (!hk_h) { M0.err = hk + " is NULL"; return ST_ERR_INVALID; }
+  const st::Model& Mk = hk_h->model;
+  if (Mk.device != M0.device) {
+    M0.err = hk + " is on device " + std::to_string(Mk.device) + ", handle 0 on device " + std::to_string(M0.device);
+    return ST_ERR_INVALID;
+  }
+  *s = Mk.store.find(which, hk + " has ", M0.err);
+  if (!*s) return ST_ERR_INVALID;
+  if ((*s)->n != n || (*s)->S != S) {
+    M0.err = hk + " stores " + std::to_string((*s)->S) + " draws of " + std::to_string((*s)->n) + " rows, handle 0 " + std::to_string(S) +
+             " draws of " + std::to_string(n) + " rows";
+    return ST_ERR_INVALID;
+  }
+  if (Mk.p != M0.p || Mk.q != M0.q) {
+    M0.err = hk + " has p = " + std::to_string(Mk.p) + ", q = " + std::to_string(Mk.q) + "; handle 0 p = " + std::to_string(M0.p) +
+             ", q = " + std::to_string(M0.q);
+    return ST_ERR_INVALID;
+  }
+  if (Mk.n_all != M0.n_all || std::memcmp(Mk.y.data(), M0.y.data(), M0.y.size() * sizeof(double)) ||
+      std::memcmp(Mk.X.data(), M0.X.data(), M0.X.size() * sizeof(double)) ||
+      std::memcmp(Mk.mv_id.data(), M0.mv_id.data(), M0.mv_id.size() * sizeof(int64_t))) {
+    M0.err = hk + " has a different y, X or mv_id from handle 0 (the criteria compare fits of the same data)";
+    return ST_ERR_INVALID;
+  }
+  return ST_OK;
+}
+// every store is complete before the kernel reads it on hs[0]'s stream
+static int criteria_sync(const char* who, st_handle* const* hs, int32_t n_chains) {
+  for (int k = 1; k < n_chains; k++)
+    if (const cudaError_t e = cudaStreamSynchronize(hs[k]->model.stream)) {
+      hs[0]->model.err = std::string(who) + ": CUDA error in sync of handle " + std::to_string(k) + ": " + cudaGetErrorString(e);
+      return ST_ERR_CUDA;
+    }
+  return ST_OK;
+}
 int st_fit_criteria(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit_criteria_out* out) {
   if (!hs || n_chains < 1 || !hs[0]) {  // (no handle to report to)
     g_create_error = n_chains < 1 ? "st_fit_criteria: n_chains must be at least 1" : "st_fit_criteria: hs or hs[0] is NULL";
@@ -360,30 +411,10 @@ int st_fit_criteria(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit
   st::dvec beta(N * p * q), tausq(N * q);  // pooled draw g = k S + s: p x q, then q
   for (int k = 0; k < n_chains; k++) {
     const std::string hk = "st_fit_criteria: handle " + std::to_string(k);
-    if (!hs[k]) { M0.err = hk + " is NULL"; return ST_ERR_INVALID; }
+    const st::DrawStore::Store* s = nullptr;
+    rc = criteria_handle(hk, M0, hs[k], 0, n, S, &s);
+    if (rc) return rc;
     const st::Model& Mk = hs[k]->model;
-    if (Mk.device != M0.device) {
-      M0.err = hk + " is on device " + std::to_string(Mk.device) + ", handle 0 on device " + std::to_string(M0.device);
-      return ST_ERR_INVALID;
-    }
-    const st::DrawStore::Store* s = Mk.store.find(0, hk + " has ", M0.err);
-    if (!s) return ST_ERR_INVALID;
-    if (s->n != n || s->S != S) {
-      M0.err = hk + " stores " + std::to_string(s->S) + " draws of " + std::to_string(s->n) + " rows, handle 0 " + std::to_string(S) +
-               " draws of " + std::to_string(n) + " rows";
-      return ST_ERR_INVALID;
-    }
-    if (Mk.p != p || Mk.q != q) {
-      M0.err = hk + " has p = " + std::to_string(Mk.p) + ", q = " + std::to_string(Mk.q) + "; handle 0 p = " + std::to_string(p) +
-               ", q = " + std::to_string(q);
-      return ST_ERR_INVALID;
-    }
-    if (Mk.n_all != M0.n_all || std::memcmp(Mk.y.data(), M0.y.data(), M0.y.size() * sizeof(double)) ||
-        std::memcmp(Mk.X.data(), M0.X.data(), M0.X.size() * sizeof(double)) ||
-        std::memcmp(Mk.mv_id.data(), M0.mv_id.data(), M0.mv_id.size() * sizeof(int64_t))) {
-      M0.err = hk + " has a different y, X or mv_id from handle 0 (the criteria compare fits of the same data)";
-      return ST_ERR_INVALID;
-    }
     const st::dvec& sm = Mk.store.samples;  // theta (npar x S) | beta (p x S x q) | tausq (q x S)
     if (sm.size() < nb + nt) { M0.err = hk + ": the stored run's beta / tausq samples are missing"; return ST_ERR_INVALID; }
     const double* be = sm.data() + (sm.size() - nb - nt);
@@ -397,15 +428,43 @@ int st_fit_criteria(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit
     }
     src[k] = s->d;
   }
-  for (int k = 1; k < n_chains; k++)  // every store is complete before the kernel reads it on hs[0]'s stream
-    if (const cudaError_t e = cudaStreamSynchronize(hs[k]->model.stream)) {
-      M0.err = std::string("st_fit_criteria: CUDA error in sync of handle ") + std::to_string(k) + ": " + cudaGetErrorString(e);
-      return ST_ERR_CUDA;
-    }
+  rc = criteria_sync("st_fit_criteria", hs, n_chains);
+  if (rc) return rc;
   std::vector<char> obs(n);
   for (int64_t i = 0; i < n; i++) obs[i] = std::isfinite(M0.y[i]);
   const st::CritInputs in{M0.y.data(), M0.X.data(), M0.mv_id.data(), beta.data(), tausq.data(), p, q};
   return st::fit_criteria(src.data(), n, n_chains, S, r_eff, obs, &in, *out, M0.stream, M0.err);
+  ST_GUARD_END(h0)
+}
+int st_fit_criteria_integrated(st_handle* const* hs, int32_t n_chains, double r_eff, st_fit_criteria_out* out) {
+  if (!hs || n_chains < 1 || !hs[0]) {  // (no handle to report to)
+    g_create_error = n_chains < 1 ? "st_fit_criteria_integrated: n_chains must be at least 1"
+                                  : "st_fit_criteria_integrated: hs or hs[0] is NULL";
+    return ST_ERR_INVALID;
+  }
+  st_handle* h0 = hs[0];
+  st::Model& M0 = h0->model;
+  if (!out) { M0.err = "st_fit_criteria_integrated: out is NULL"; return ST_ERR_INVALID; }
+  activate(h0);
+  ST_GUARD_BEGIN
+  const int which = st::DrawStore::kLoglikInt;
+  const int64_t n = M0.store.get(which).n;
+  const int S = M0.store.get(which).S;
+  int rc = st::criteria_check("st_fit_criteria_integrated", n_chains, std::max(S, 1), r_eff, M0.err);
+  if (rc) return rc;
+  std::vector<const double*> src(n_chains);
+  for (int k = 0; k < n_chains; k++) {
+    const st::DrawStore::Store* s = nullptr;
+    rc = criteria_handle("st_fit_criteria_integrated: handle " + std::to_string(k), M0, hs[k], which, n, S, &s);
+    if (rc) return rc;
+    src[k] = s->d;
+  }
+  rc = criteria_sync("st_fit_criteria_integrated", hs, n_chains);
+  if (rc) return rc;
+  // the log-likelihood mode of fit_criteria_kernel: the stores hold ll itself, NaN at the rows whose y is missing
+  std::vector<char> obs(n);
+  for (int64_t i = 0; i < n; i++) obs[i] = std::isfinite(M0.y[i]);
+  return st::fit_criteria(src.data(), n, n_chains, S, r_eff, obs, nullptr, *out, M0.stream, M0.err);
   ST_GUARD_END(h0)
 }
 int st_fit_criteria_loglik(int32_t device, const double* loglik, int64_t n_rows, int32_t n_chains, int32_t n_samples, double r_eff,

@@ -7,7 +7,8 @@
 //                       (H' = L^-T Z) — all without leaving shared memory (SURVEY App. F).  Also used for the
 //                       prediction blocks (predict_std, :1234-1358).
 //  gibbs_level_kernel   Gibbs update of w for one level (gibbs_sample_w_std, :1011-1226) including the messages to
-//                       every ancestor, accumulated by pulling from the direct children (deterministic, no atomics).
+//                       every ancestor, accumulated by pulling from the direct children (deterministic, no atomics);
+//                       its ILOO variant also forms each row's integrated log-likelihood (DESIGN.md §5f).
 //  gram_level_kernel    theta-only part of the messages (Sigi_children, :1190-1192), refreshed only after theta changes.
 //  llw_kernel           log-density at the current theta with the new w (get_loglik_w_std, :781-826).
 //  row kernels          beta / tausq sufficient statistics (:1364-1417), X*beta, device normals, predictive draws.
@@ -26,11 +27,20 @@ namespace st {
 // ------------------------------------------------------------------------------------------------ GIBBS
 // One block per tree block (node).  Shared memory: RiS m*m | Sig m*m | wpa P | gwj (k+1)*m | smu m | wn m | rr m
 // REF = 1: full m x m conditional (:1037-1089); REF = 0: row-wise scalars (:1091-1155)
-template <int REF>
+// ILOO: also the integrated log-likelihood of every observed row (DESIGN.md §5f), ll[i] = log N(y_i - xb_i; m_i, v_i + tausq_i)
+// with N(m_i, v_i) the prior conditional of w_i given the state the block is drawn from.  ll is node-major; yobs holds y
+// node-major with NaN at the rows that are not observed, whose slots of ll the kernel leaves alone.
+// Its log-density term; v: the prior conditional's variance, tq: tausq_inv of the row.
+__device__ __forceinline__ double iloo_term(double resid, double mean, double v, double tq) {
+  const double s2 = v + 1.0 / tq, d = resid - mean;
+  return -0.5 * (log(6.283185307179586 * s2) + d * d / s2);
+}
+template <int REF, bool ILOO>
 __global__ void __launch_bounds__(kGibbsThreads)
 gibbs_level_kernel(DevTree T, DevSlots D, int slot0, double* __restrict__ w, const double* __restrict__ xb,
                    const double* __restrict__ z, const double* __restrict__ tausq_inv, const double* __restrict__ SigS,
-                   double* __restrict__ V, double* probe_sig, double* probe_smu, int* __restrict__ fail) {
+                   double* __restrict__ V, double* probe_sig, double* probe_smu, int* __restrict__ fail,
+                   double* __restrict__ ll, const double* __restrict__ yobs) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // programmatic dependent launch: the next (shallower) level may start early; it waits below before it reads the
   // messages this level writes (everything before that point depends on ancestors only)
@@ -216,6 +226,32 @@ gibbs_level_kernel(DevTree T, DevSlots D, int slot0, double* __restrict__ w, con
       }
     }
     __syncthreads();
+    if (ILOO) {
+      // w = L^-T (L^-1 Smu + z), so Sigi_tot w - Smu = L z exactly.  Without row a's own observation the precision is
+      // Q'_aa = (Ri'Ri)_aa + (children's Gram)_aa (formed directly, not as Sigi_tot_aa - tausq_inv: no cancellation at small
+      // tausq) and the prior conditional of w_a given everything else is N(w_a - [(L z)_a + tausq_inv (resid_a - w_a)] / Q'_aa,
+      // 1 / Q'_aa).  rr still holds z here; the loop below overwrites it.
+      // Thread a walks row a of L: at step t the threads read a stride of m doubles apart (odd m) or, walking back from the
+      // diagonal, m + 1 (even m), so that the stride is odd and the shared-memory reads are free of bank conflicts.  The
+      // column of Ri is read at a stride of rsm + 1, odd as well (tile_rs).
+      const long long so0 = T.soff[sd];
+      const bool back = (m & 1) == 0;
+      for (int a = tid; a < m; a += nth) {
+        const int i = row0 + a;
+        const double yi = yobs[i];
+        if (isnan(yi)) continue;  // not observed
+        double lz = 0.0, qa = 0.0;
+        for (int t = 0; t <= a; t++) {
+          const int j = back ? a - t : t;
+          lz = fma(Sig[a * m + j], rr[j], lz);
+        }
+        for (int r = a; r < m; r++) qa = fma(RiS[r * rsm + a], RiS[r * rsm + a], qa);
+        if (so0 >= 0) qa += SigS[so0 + (long long)a * m + a];
+        const double tq = tausq_inv[T.mvq[i]], res = yi - xb[i], wa = wn[a];
+        ll[i] = iloo_term(res, wa - (lz + tq * (res - wa)) / qa, 1.0 / qa, tq);
+      }
+      __syncthreads();
+    }
     for (int r = tid; r < m; r += nth) {
       double s = -gw[r];
       for (int r2 = 0; r2 <= r; r2++) s = fma(RiS[r * rsm + r2], wn[r2], s);
@@ -239,6 +275,10 @@ gibbs_level_kernel(DevTree T, DevSlots D, int slot0, double* __restrict__ w, con
         wa = w[row0 + a];
       }
       rr[a] = ri * wa - gw[a];
+      // the prior conditional of w_a is N(gw_a / ri, 1 / ri^2): it does not involve w_a.  (ri^2 is formed apart from prec:
+      // a second use of prec would keep the compiler from fusing it into sig, and w would change in the last bits.)
+      if (ILOO && !isnan(yobs[row0 + a]))
+        ll[row0 + a] = iloo_term(yobs[row0 + a] - xb[row0 + a], gw[a] / ri, 1.0 / __dmul_rn(ri, ri), wn[a]);
     }
   }
   __syncthreads();
@@ -280,12 +320,15 @@ gibbs_level_kernel(DevTree T, DevSlots D, int slot0, double* __restrict__ w, con
 
 cudaError_t launch_gibbs(int is_ref, const DevTree& T, const DevSlots& D, int slot0, int nslots, double* w,
                          const double* xb, const double* z, const double* tausq_inv, const double* SigS, double* V,
-                         double* probe_sig, double* probe_smu, int* fail, size_t smem, cudaStream_t st, bool pdl) {
+                         double* probe_sig, double* probe_smu, int* fail, size_t smem, cudaStream_t st, bool pdl, double* ll,
+                         const double* yobs) {
   if (nslots <= 0) return cudaSuccess;
-  static SmemOptIn optin[2];
-  auto kern = is_ref ? gibbs_level_kernel<1> : gibbs_level_kernel<0>;
+  static SmemOptIn optin[4];
+  const bool iloo = ll != nullptr;
+  auto kern = is_ref ? (iloo ? gibbs_level_kernel<1, true> : gibbs_level_kernel<1, false>)
+                     : (iloo ? gibbs_level_kernel<0, true> : gibbs_level_kernel<0, false>);
   {
-    cudaError_t e = ensure_dynamic_smem(kern, smem, optin[is_ref ? 1 : 0]);
+    cudaError_t e = ensure_dynamic_smem(kern, smem, optin[(is_ref ? 1 : 0) + (iloo ? 2 : 0)]);
     if (e != cudaSuccess) return e;
   }
   cudaLaunchConfig_t cfg = {};
@@ -298,7 +341,7 @@ cudaError_t launch_gibbs(int is_ref, const DevTree& T, const DevSlots& D, int sl
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, T, D, slot0, w, xb, z, tausq_inv, SigS, V, probe_sig, probe_smu, fail);
+  return cudaLaunchKernelEx(&cfg, kern, T, D, slot0, w, xb, z, tausq_inv, SigS, V, probe_sig, probe_smu, fail, ll, yobs);
 }
 
 // ------------------------------------------------------------------------------------------------ message Grams

@@ -50,7 +50,9 @@ cudaError_t launch_build(int mode, const DevTree& T, const DevSlots& D, int rel,
                          const int* run_flag = nullptr);  // pdl: programmatic dependent launch on the previous kernel of the stream
 cudaError_t launch_gibbs(int is_ref, const DevTree& T, const DevSlots& D, int slot0, int nslots, double* w,
                          const double* xb, const double* z, const double* tausq_inv, const double* SigS, double* V,
-                         double* probe_sig, double* probe_smu, int* fail, size_t smem, cudaStream_t st, bool pdl = false);
+                         double* probe_sig, double* probe_smu, int* fail, size_t smem, cudaStream_t st, bool pdl = false,
+                         double* ll = nullptr,   // ll != NULL: the ILOO variant, integrated log-likelihood into ll (node-major) at
+                         const double* yobs = nullptr);  // the rows where yobs (y node-major, NaN: not observed) is not NaN
 cudaError_t launch_gram(const DevTree& T, const DevSlots& D, int slot0, int nslots, double* U, double* SigS, int rch,
                         int ldx, int tile_doubles, int stage_off, int threads, cudaStream_t st, const int* run_flag = nullptr,
                         bool pdl = false);  // pdl: only after another gram launch (the kernel waits before it reads the children's tiles only)

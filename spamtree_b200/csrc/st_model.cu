@@ -1070,8 +1070,9 @@ int Model::refresh_grams(const int* run_flag, cudaStream_t st) {
   return 0;
 }
 
-// the level launches of one Gibbs sweep, leaves to root; fail_ptr: device int that counts failed factorisations
-int Model::gibbs_launch_only(int* fail_ptr) {
+// the level launches of one Gibbs sweep, leaves to root; fail_ptr: device int that counts failed factorisations; iloo: the
+// sweep also forms the integrated log-likelihood into d_ll_int_
+int Model::gibbs_launch_only(int* fail_ptr, bool iloo) {
   NvtxRange nvtx("GIBBS");
   for (int g = (int)levels.size() - 1; g >= 0; g--) {
     const LevelInfo& L = levels[g];
@@ -1087,7 +1088,8 @@ int Model::gibbs_launch_only(int* fail_ptr) {
     if (profile) { cudaEventCreate(&pe0); cudaEventCreate(&pe1); cudaEventRecord(pe0, stream); }
     ST_CUDA(launch_gibbs(L.is_ref, dt, dslots, L.slot0, L.nslots, d_w, d_xb, d_z, d_tausq_inv, d_S, d_V,
                          probes ? d_probe_sig : nullptr, probes ? d_probe_smu : nullptr, fail_ptr, L.smem_gibbs, stream,
-                         use_pdl && !profile && g != (int)levels.size() - 1),
+                         use_pdl && !profile && g != (int)levels.size() - 1, iloo ? d_ll_int_ : nullptr,
+                         iloo ? d_ll_int_ + n_all : nullptr),
             "gibbs_level_kernel");
     n_launches++;
     if (profile) {
@@ -1110,8 +1112,10 @@ int Model::deal_with_w(const double* z, uint64_t seed) {
   stats_valid_mode_ = -1;  // w is about to change
   { int rc = complete_slot(cur); if (rc) return rc; }
   if (gram_stale) { int rc = refresh_grams(); if (rc) return rc; }
+  const bool iloo = (keep_mask & ST_KEEP_LOGLIK_INT) != 0;
+  if (iloo) { int rc = alloc_loglik_int(); if (rc) return rc; }
   ST_CUDA(cudaMemsetAsync(d_fail, 0, sizeof(int), stream), "memset");
-  int rc = gibbs_launch_only(d_fail);
+  int rc = gibbs_launch_only(d_fail, iloo);
   if (rc) return rc;
   // failed factorisations, agreed over the ranks of a partition (every rank must take the same exit): the count rides in an
   // 8-double reduction slot, all-reduced on the stream
@@ -1121,6 +1125,31 @@ int Model::deal_with_w(const double* z, uint64_t seed) {
   ST_CUDA(cudaMemcpyAsync(h_scalars + 48, slot8, 8 * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H fail");
   ST_CUDA(cudaStreamSynchronize(stream), "sync");
   if (h_scalars[48 + 6] != 0.0) { err = "Error at gibbs_sample_w: conditional precision not positive definite"; return 3; }
+  if (iloo) ll_int_valid_ = true;
+  return 0;
+}
+
+int Model::alloc_loglik_int() {
+  if (d_ll_int_) return 0;
+  ST_CUDA(dev_zeros(d_ll_int_, 2 * n_all, owned), "alloc integrated log-likelihood");
+  ST_CUDA(cudaMemsetAsync(d_ll_int_, 0xff, n_all * sizeof(double), stream), "memset");  // (all bits set: a NaN)
+  const double nan = std::numeric_limits<double>::quiet_NaN();
+  for (int64_t i = 0; i < n_all; i++) h_stage[i] = std::isfinite(y[perm[i]]) ? y[perm[i]] : nan;
+  ST_CUDA(cudaMemcpyAsync(d_ll_int_ + n_all, h_stage, n_all * sizeof(double), cudaMemcpyHostToDevice, stream), "H2D y");
+  ST_CUDA(cudaStreamSynchronize(stream), "sync");  // (h_stage is free again)
+  return 0;
+}
+
+int Model::get_loglik_int(double* out) {
+  if (!stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
+  if (!ll_int_valid_) {
+    err = "st_get_loglik_int: no sweep has formed the integrated log-likelihood (st_keep_samples_on_device with ST_KEEP_LOGLIK_INT "
+          "before st_deal_with_w or st_mcmc_run)";
+    return 1;
+  }
+  ST_CUDA(cudaMemcpyAsync(h_stage, d_ll_int_, n_all * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H integrated log-likelihood");
+  ST_CUDA(cudaStreamSynchronize(stream), "sync");
+  for (int64_t i = 0; i < n_all; i++) out[perm[i]] = h_stage[i];
   return 0;
 }
 
@@ -1542,13 +1571,13 @@ int Model::get_index(const std::string& which, int u, int c, int64_t* out, int64
 
 // ------------------------------------------------------------------------------------------------ device-resident iteration
 // One Gibbs sweep, enqueued only: normals keyed by (seed, row, iteration), Gram refresh and deferred half are the callers'
-int Model::enqueue_gibbs(uint64_t seed, bool device_chain, bool draw) {
+int Model::enqueue_gibbs(uint64_t seed, bool device_chain, bool draw, bool iloo) {
   if (draw) {  // (draw = false: the previous iteration of the device-resident chain already drew this sweep's normals)
     ST_CUDA(launch_normals(d_z, n_all, seed, device_chain ? 0 : sweep_counter++, d_rowkey, device_chain ? &d_mc->iter : nullptr, stream),
             "normals_kernel");
     n_launches++;
   }
-  return gibbs_launch_only(device_chain ? &d_mc->gibbs_fail : d_fail);
+  return gibbs_launch_only(device_chain ? &d_mc->gibbs_fail : d_fail, iloo);
 }
 
 // One iteration of spamtree_fit.cpp:167-330 enqueued on the stream without any host synchronisation; every decision is
@@ -1586,7 +1615,7 @@ int Model::enqueue_iteration(const st_mcmc_opts& o, bool predicting, int accept_
   // bandwidth), after the sweep has finished.  (Partitioned handles keep it on the main stream, with their collectives.)
   const bool llw2 = llw_overlap && !part && o.sample_w && o.sample_theta && stream2 != nullptr;
   if (o.sample_w) {  // :183-187
-    rc = enqueue_gibbs(o.seed, true, draws_here);
+    rc = enqueue_gibbs(o.seed, true, draws_here, record_keep > 0 && (keep_mask & ST_KEEP_LOGLIK_INT));  // (saved iterations only)
     if (rc) return rc;
     if (tev) ST_CUDA(cudaEventRecord(tev[1], stream), "event");
     if (llw2 || ovl) ST_CUDA(cudaEventRecord(ev_sweep, stream), "event");
@@ -1857,9 +1886,14 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   }
   // the device sample store (st_keep_samples_on_device): sized and checked before anything is allocated or launched, so that a
   // refused run leaves the handle as it was; a run replaces the last run's store
+  const bool iloo = (keep_mask & ST_KEEP_LOGLIK_INT) != 0;
+  if (iloo && !o.sample_w) {
+    err = "st_mcmc_run: the integrated log-likelihood (ST_KEEP_LOGLIK_INT) is formed by the Gibbs sweep over w: it needs sample_w";
+    return 1;
+  }
   if (keep_mask) {
     if (part) { err = "st_mcmc_run: the device sample store is not supported on partitioned handles"; return 4; }
-    const int rc = store.reserve(keep_mask, (size_t)n_all * (size_t)std::max(o.keep, 0) * sizeof(double), "st_mcmc_run", err);
+    const int rc = store.reserve(DrawStore::mask_of(keep_mask), (size_t)n_all * (size_t)std::max(o.keep, 0) * sizeof(double), "st_mcmc_run", err);
     if (rc) return rc;
   }
   double o3[3];
@@ -1872,6 +1906,11 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   if (gram_stale) { rc = refresh_grams(); if (rc) return rc; }
   rc = set_widx_mode(o.faithful_beta_index != 0);
   if (rc) return rc;
+  if (iloo) {
+    rc = alloc_loglik_int();
+    if (rc) return rc;
+    ll_int_valid_ = false;
+  }
   const int npar = (int)theta[0].size(), keep = o.keep, mcmc = o.thin * o.keep + o.burn;
   // sample arrays on the device, copied out once at the end
   const size_t n_th = (size_t)npar * keep, n_be = (size_t)p * keep * q, n_ta = (size_t)q * keep;
@@ -1899,9 +1938,11 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   // of tools/run_partition.py hung with it, so it is not the default
   static const bool part_graph = getenv("ST_PART_GRAPH") && atoi(getenv("ST_PART_GRAPH")) == 1;
   bool use_graph = !no_graph && (!part || (nccl_comm != nullptr && part_graph));
-  // (a graph holds the addresses and the layout of the sample arrays: keep and their base are part of its key)
-  const long long key_base = ((o.sample_beta ? 1 : 0) | (o.sample_tausq ? 2 : 0) | (o.sample_theta ? 4 : 0) | (o.sample_w ? 8 : 0) | (o.sample_predicts ? 16 : 0)) +
-                             32LL * keep + (long long)(reinterpret_cast<uintptr_t>(d_samp_) >> 4) * 1000003LL;
+  // (a graph holds the addresses and the layout of the sample arrays: keep and their base are part of its key; and whether
+  // its sweep forms the integrated log-likelihood)
+  const long long key_base = ((o.sample_beta ? 1 : 0) | (o.sample_tausq ? 2 : 0) | (o.sample_theta ? 4 : 0) | (o.sample_w ? 8 : 0) | (o.sample_predicts ? 16 : 0) |
+                              (iloo ? 32 : 0)) +
+                             64LL * keep + (long long)(reinterpret_cast<uintptr_t>(d_samp_) >> 4) * 1000003LL;
   int msaved = 0;
   const auto t0 = std::chrono::steady_clock::now();
   for (int m = 0; m < mcmc; m++) {
@@ -1943,6 +1984,10 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
         rc = save_rows(co, k, kept ? store.get(k).d + off : nullptr, host_rows[k] ? host_rows[k] + off : nullptr);
         if (rc) return rc;
       }
+      if (iloo) {  // this iteration's sweep formed it: into its slot of the store, in boundary order
+        ST_CUDA(launch_permute(d_ll_int_, store.get(DrawStore::kLoglikInt).d + off, d_iperm, n_all, stream), "permute_kernel");
+        n_launches++;
+      }
       msaved++;
     }
   }
@@ -1962,8 +2007,9 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
   out.n_chol_fail = h_mc->n_chol_fail;
   if (h_mc->gibbs_fail) { err = "Error at gibbs_sample_w: conditional precision not positive definite"; return 3; }
   if (h_mc->nan_loglik) { err = "At nan loglik: error."; return 5; }
+  if (iloo && keep > 0) ll_int_valid_ = true;
   if (keep_mask && keep > 0) {  // the run completed: its store and the samples st_predict_new_stored predicts from
-    store.commit(keep_mask, n_all, keep);
+    store.commit(DrawStore::mask_of(keep_mask), n_all, keep);
     store.samples.assign(hs.begin(), hs.begin() + (n_th + n_be + n_ta));
   }
   return 0;
@@ -1973,7 +2019,7 @@ int Model::chain_run(const st_mcmc_opts& o, st_mcmc_out& out) {
 int DrawStore::reserve(int mask, size_t bytes_each, const char* what, std::string& err) {
   const int group = ((mask & kRun) ? kRun : 0) | ((mask & kPrediction) ? kPrediction : 0);
   size_t need = 0, reusable = 0;
-  for (int k = 0; k < 4; k++) {
+  for (int k = 0; k < kStores; k++) {
     if (mask & (1 << k)) need += bytes_each;
     if (group & (1 << k)) reusable += s_[k].cap;
   }
@@ -1986,7 +2032,7 @@ int DrawStore::reserve(int mask, size_t bytes_each, const char* what, std::strin
   }
   if (group & kRun) samples.clear();
   const size_t bytes = std::max<size_t>(bytes_each, 8);
-  for (int k = 0; k < 4; k++) {
+  for (int k = 0; k < kStores; k++) {
     if (!(group & (1 << k))) continue;
     Store& s = s_[k];
     s.S = 0;
@@ -2006,16 +2052,18 @@ int DrawStore::reserve(int mask, size_t bytes_each, const char* what, std::strin
 }
 
 void DrawStore::commit(int mask, int64_t n, int S) {
-  for (int k = 0; k < 4; k++)
+  for (int k = 0; k < kStores; k++)
     if (mask & (1 << k)) { s_[k].n = n; s_[k].S = S; }
 }
 
 const DrawStore::Store* DrawStore::find(int which, const std::string& who, std::string& err) const {
-  static const char* names[4] = {"w", "yhat", "w_new", "y_new"};
+  static const char* names[kStores] = {"w", "yhat", "w_new", "y_new", "the integrated log-likelihood"};
   const Store& s = s_[which];
   if (s.d && s.S >= 1) return &s;
   err = who + "no stored draws of " + names[which] +
-        (which < 2 ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)" : " (st_predict_new_stored with keep_draws)");
+        (which == kLoglikInt ? " (st_keep_samples_on_device with ST_KEEP_LOGLIK_INT before a device-resident st_mcmc_run that samples w)"
+         : which < 2         ? " (st_keep_samples_on_device before a device-resident st_mcmc_run)"
+                             : " (st_predict_new_stored with keep_draws)");
   return nullptr;
 }
 
@@ -2028,7 +2076,10 @@ void DrawStore::release() {
 }
 
 int Model::keep_samples_on_device(int what) {
-  if (what < 0 || what > (ST_KEEP_W | ST_KEEP_YHAT)) { err = "st_keep_samples_on_device: what must be a mask of ST_KEEP_W | ST_KEEP_YHAT"; return 1; }
+  if (what < 0 || what > (ST_KEEP_W | ST_KEEP_YHAT | ST_KEEP_LOGLIK_INT)) {
+    err = "st_keep_samples_on_device: what must be a mask of ST_KEEP_W | ST_KEEP_YHAT | ST_KEEP_LOGLIK_INT";
+    return 1;
+  }
   if (what && !stream) { err = "this handle has no device state (created with device < 0)"; return 2; }
   if (what && part) { err = "st_keep_samples_on_device: partitioned handles are not supported"; return 4; }
   keep_mask = what;
@@ -2075,6 +2126,21 @@ int Model::summarize(int which, const double* probs, int n_probs, st_summary_out
     if (hdst[c] && cnt) ST_CUDA(cudaMemcpyAsync(hdst[c], dsrc[c], cnt * sizeof(double), cudaMemcpyDeviceToHost, stream), "D2H summaries");
   }
   ST_CUDA(cudaStreamSynchronize(stream), "sync");
+  return 0;
+}
+
+int Model::copy_store(int which, double* out, int64_t* n_rows, int32_t* n_samples) {
+  if (which < 0 || which >= DrawStore::kStores) {
+    err = "st_copy_store: which must be 0 (w), 1 (yhat), 2 (w_new), 3 (y_new) or 4 (the integrated log-likelihood)";
+    return 1;
+  }
+  const DrawStore::Store* sp = store.find(which, "st_copy_store: ", err);
+  if (!sp) return 1;
+  if (n_rows) *n_rows = sp->n;
+  if (n_samples) *n_samples = sp->S;
+  if (!out || sp->n == 0) return 0;
+  ST_CUDA(cudaStreamSynchronize(stream), "sync");  // (the run or prediction that wrote it)
+  ST_CUDA(cudaMemcpy(out, sp->d, (size_t)sp->n * sp->S * sizeof(double), cudaMemcpyDeviceToHost), "D2H store");
   return 0;
 }
 

@@ -130,12 +130,14 @@ class CopyOut {
 };
 
 // Draws kept on the device (st_keep_samples_on_device, st_predict_new_stored, st_summarize; DESIGN.md §5c), the only code
-// that knows the stores' layout.  Store k holds [sample][row] draws, n rows x S samples: w (0) and yhat (1) of the last
-// device-resident run, w_new (2) and y_new (3) of the last stored prediction.  A mask selects store k by bit k (ST_KEEP_W,
-// ST_KEEP_YHAT for the first two).
+// that knows the stores' layout.  Store k holds [sample][row] draws, n rows x S samples: w (0), yhat (1) and the integrated
+// log-likelihood (4) of the last device-resident run, w_new (2) and y_new (3) of the last stored prediction.  A mask selects
+// store k by bit k (mask_of turns an st_keep_samples_on_device mask into one).
 class DrawStore {
  public:
-  static constexpr int kRun = 3, kPrediction = 12;  // what a run, a stored prediction replaces
+  static constexpr int kStores = 5, kLoglikInt = 4;
+  static constexpr int kRun = 3 | (1 << kLoglikInt), kPrediction = 12;  // what a run, a stored prediction replaces
+  static int mask_of(int keep) { return (keep & (ST_KEEP_W | ST_KEEP_YHAT)) | ((keep & ST_KEEP_LOGLIK_INT) ? 1 << kLoglikInt : 0); }
   struct Store {
     double* d = nullptr;
     size_t cap = 0;  // bytes allocated (reused by the next run when large enough)
@@ -158,7 +160,7 @@ class DrawStore {
   dvec samples;  // theta (npar x S), beta (p x S x q), tausq (q x S) of the last stored run
 
  private:
-  Store s_[4];
+  Store s_[kStores];
 };
 
 class Model {
@@ -290,6 +292,8 @@ class Model {
   int gibbs_sample_beta(const double* zb, bool faithful_index);  // :1364-1391
   int gibbs_sample_tausq(const double* fixed);         // :1393-1417
   int get_w(double* out);
+  int get_loglik_int(double* out);  // st_get_loglik_int
+  int copy_store(int which, double* out, int64_t* n_rows, int32_t* n_samples);  // st_copy_store
   // a saved iteration's w (k = 0, un-permuted) or yhat (k = 1, device-resident chain only), in boundary order: written on
   // `stream` into `dev` (a slot of the device store) or, when dev is NULL, into co's staging slot k, then copied to `host`
   // (NULL: none) on the copy stream
@@ -311,7 +315,7 @@ class Model {
   // ---- device sample store (st_keep_samples_on_device, st_summarize; DESIGN.md §5c)
   int keep_samples_on_device(int what);
   int summarize(int which, const double* probs, int n_probs, st_summary_out& out);
-  int keep_mask = 0;                   // ST_KEEP_W | ST_KEEP_YHAT for the following device-resident runs
+  int keep_mask = 0;                   // ST_KEEP_W | ST_KEEP_YHAT | ST_KEEP_LOGLIK_INT for the following device-resident runs
   DrawStore store;
 
  private:
@@ -325,7 +329,7 @@ class Model {
   int complete_slot(int pslot);  // the deferred half of BUILD for the slot's childless levels, if pending
   int launch_deferred_half(int rel, const int* run_flag, cudaStream_t st);
   int push_slot_theta(int ps);   // host-driven path: theta[ps] and its covariance table into the device chain state
-  int enqueue_gibbs(uint64_t seed, bool device_chain, bool draw = true);
+  int enqueue_gibbs(uint64_t seed, bool device_chain, bool draw = true, bool iloo = false);
   int enqueue_stats();
   int enqueue_iteration(const st_mcmc_opts& o, bool predicting, int accept_mode, bool draws_here, bool draws_next, int record_keep = 0);
   int push_chain_state(const st_mcmc_opts* o, uint64_t seed);
@@ -333,7 +337,13 @@ class Model {
   cudaEvent_t* timing_events_ = nullptr;
   bool deferred_[2] = {false, false};
   int refresh_grams(const int* run_flag = nullptr, cudaStream_t st = nullptr);
-  int gibbs_launch_only(int* fail_ptr);
+  int gibbs_launch_only(int* fail_ptr, bool iloo = false);
+  // the integrated log-likelihood of the sweeps that form it (ST_KEEP_LOGLIK_INT; DESIGN.md §5f): node-major, n_all doubles,
+  // NaN until a sweep writes them (the rows that are not observed stay NaN), then n_all doubles of y node-major with NaN at
+  // the rows that are not observed, which tell the ILOO Gibbs kernel which rows to form.  Allocated and filled once.
+  double* d_ll_int_ = nullptr;
+  bool ll_int_valid_ = false;  // a sweep has formed it
+  int alloc_loglik_int();
   int rowstats(bool faithful_index);
   std::vector<int> isref_host_;
   long long sd_total_ = 0;
